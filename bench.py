@@ -4,6 +4,8 @@
     python bench.py --gpus 1 --steps K --warmup W              # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...    # the reference's CPU kd-tree on the host cores
     torchrun --nproc-per-node N ... bench.py --gpus N ...      # one rank per GPU, weak scaling
+    python bench.py ... --dump-outputs DIR                     # + the last timed step's radii as DIR/radius.npy
+                                                               #   (rank 0's only: other ranks' batches are not written)
 
 A step = one pass of the hot path over one batch: `pc_radius_batch` (safeRegionRrtStar::radiusSearch,
 Planner/src/corridor_finder.cpp:113-133) for a batch of RRT* sample points against the resident index of the
@@ -70,7 +72,24 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-sample", type=int, default=1_000_000)
     ap.add_argument("--ref-sample", type=int, default=200_000, help="queries per step of the reference arm")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the radii the last timed step returned to DIR/radius.npy; "
+                         "with several ranks only rank 0's radii are written, not the other ranks' batches")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+# --dump-outputs writes at most this many bytes; a larger output is thinned to every k-th value (k fixed by its size)
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, radius):
+    """Write the last timed step's radii as out_dir/radius.npy, so that two builds can be compared value for value."""
+    stride = -(-radius.nbytes // DUMP_MAX_BYTES)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "radius.npy"), np.ascontiguousarray(radius[::stride]))
 
 
 def workload_config(args):
@@ -181,8 +200,10 @@ def run_reference(args):
         cpu_radius(tree, kind, qs[s], start)
     t0 = time.perf_counter()
     for s in range(args.steps):
-        cpu_radius(tree, kind, qs[args.warmup + s], start)
+        r_last = cpu_radius(tree, kind, qs[args.warmup + s], start)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, r_last)
     val = m * args.steps / dt
     line = {"impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
             "warmup": args.warmup, "ms_per_step": dt / args.steps * 1e3, "higher_is_better": True, "scaling": "weak",
@@ -327,6 +348,8 @@ def run_b200(args):
     barrier()
     launches = ix.launches()
     elapsed_ms = e0.elapsed_time(e1)
+    # step k wrote t_rs[k % 3]; the loops below overwrite these buffers, so the last timed step's radii are copied out now
+    r_last = t_rs[(args.steps - 1) % 3].cpu().numpy() if args.dump_outputs and rank == 0 else None
     # kernel-level durations of the dominant kernel, measured with CUDA events around it (separate short loop so
     # that reading the events does not stall the timed region above)
     for _ in range(min(args.steps, 10)):
@@ -613,6 +636,8 @@ def run_b200(args):
             cb, r_cpu = cpu_baseline(pts, q_host, start, args.cpu_sample)
             cb["gpu_matches_cpu_sample"] = bool((r_cpu.astype(np.float32) == t_r[: len(r_cpu)].cpu().numpy()).all())
             line["cpu_baseline"] = cb
+        if r_last is not None:
+            dump_outputs(args.dump_outputs, r_last)
         emit(line)
     ix.close()
     if world > 1:

@@ -17,6 +17,8 @@ SIMULATION = dict(search_margin=0.0, max_radius=5.0, sample_range=30.0)       # 
 
 
 def _cpu_tree(pts, seed=0):
+    """The unmodified reference kd-tree when oracle/_ref holds it, else the oracle's C restatement (kd_oracle.c).  The
+    restatement is not the original: test_oracle.py pins it to the reference's stored answers in tests/golden."""
     order = np.random.default_rng(seed).permutation(len(pts))
     if oracle.have_reference():
         return oracle.KdReference().build(pts, order), True
@@ -29,7 +31,8 @@ def _cpu_radius(tree, is_ref, params, start, q):
 
 
 def test_c2_radius_parity_on_the_1m_point_map():
-    """The bench workload itself: 1M-point map, both parameter sets, bounded and full-NN, against the (reference) kd-tree."""
+    """The bench workload itself: 1M-point map, both parameter sets, bounded and full-NN, against the CPU kd-tree of
+    _cpu_tree (the reference's own when oracle/_ref is present, else the oracle's restatement)."""
     pts, half = synth.forest_cloud(1_000_000, seed=1, variant="J", return_half=True)
     q = synth.rrt_queries(250_000, half, seed=21)
     tree, is_ref = _cpu_tree(pts)

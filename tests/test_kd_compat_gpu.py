@@ -31,7 +31,7 @@ def _read(path, m, nr):
     return nn, pos, cnt, items
 
 
-@pytest.mark.skipif(not oracle.have_reference(), reason="oracle/_ref/libkdtree_ref.so not present")
+@pytest.mark.skipif(not oracle.have_reference(), reason="needs the upstream pointcloudTraj kd-tree compiled into oracle/_ref (make -C oracle REF=<pointcloudTraj checkout>)")
 def test_same_client_two_backends(tmp_path):
     tmp = str(tmp_path)
     pts, half = synth.forest_cloud(40_000, seed=8, variant="J", return_half=True)

@@ -46,7 +46,7 @@ def test_known_answers(golden_dir):
     assert empty.range(np.zeros((2, 3), np.float32), 1.0)[0].tolist() == [0, 0, 0]
 
 
-@pytest.mark.skipif(not oracle.have_reference(), reason="oracle/_ref/libkdtree_ref.so not built (needs /root/reference)")
+@pytest.mark.skipif(not oracle.have_reference(), reason="needs the upstream pointcloudTraj kd-tree compiled into oracle/_ref (make -C oracle REF=<pointcloudTraj checkout>)")
 @pytest.mark.parametrize("variant,n,m,lat", [("L", 30000, 6000, 0.5), ("J", 30000, 6000, 0.0)])
 def test_oracle_equals_reference_library(variant, n, m, lat):
     pts, half = synth.forest_cloud(n, seed=4, variant=variant, return_half=True)
@@ -65,7 +65,7 @@ def test_oracle_equals_reference_library(variant, n, m, lat):
     assert (d1[:1000] == db).all()
 
 
-@pytest.mark.skipif(not oracle.have_reference(), reason="oracle/_ref/libkdtree_ref.so not built")
+@pytest.mark.skipif(not oracle.have_reference(), reason="needs the upstream pointcloudTraj kd-tree compiled into oracle/_ref (make -C oracle REF=<pointcloudTraj checkout>)")
 def test_radius_restatement_matches_reference_harness():
     pts, half = synth.forest_cloud(20000, seed=2, variant="J", return_half=True)
     q = synth.rrt_queries(4000, half * 1.5, seed=3)

@@ -19,7 +19,7 @@ from rrt_common import GOAL, PRM, START, blocked_cloud, write_input
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
-pytestmark = pytest.mark.skipif(not oracle.have_planner_reference(), reason="oracle/_ref/libplanner_ref.so not built (needs /root/reference)")
+pytestmark = pytest.mark.skipif(not oracle.have_planner_reference(), reason="needs the upstream pointcloudTraj planner compiled into oracle/_ref (make -C oracle REF=<pointcloudTraj checkout>)")
 
 
 def build_ref_check(tmp):

@@ -13,7 +13,7 @@ from rrt_common import GOAL, PRM, START
 from test_planner_ref import build_ref_check, parse_phases, two_cloud_scenario
 
 pytestmark = [pytest.mark.gpu,
-              pytest.mark.skipif(not oracle.have_planner_reference(), reason="oracle/_ref/libplanner_ref.so not built")]
+              pytest.mark.skipif(not oracle.have_planner_reference(), reason="needs the upstream pointcloudTraj planner compiled into oracle/_ref (make -C oracle REF=<pointcloudTraj checkout>)")]
 
 
 def test_rrt_loops_driven_by_the_gpu_match_the_compiled_reference(tmp_path):

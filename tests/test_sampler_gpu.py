@@ -40,7 +40,7 @@ def test_sample_stream_vs_oracle(ix, goal, inlier, k):
     assert (got2 == want2).all() and ps.engine_state == os_.engine_state
 
 
-@pytest.mark.skipif(not oracle.have_planner_reference(), reason="oracle/_ref/libplanner_ref.so not built")
+@pytest.mark.skipif(not oracle.have_planner_reference(), reason="needs the upstream pointcloudTraj planner compiled into oracle/_ref (make -C oracle REF=<pointcloudTraj checkout>)")
 def test_sample_stream_vs_compiled_reference(ix):
     """Against k calls of the UNMODIFIED genSample (corridor_finder.cpp:333-383) on the planner's own engine (eng(0))."""
     ref = oracle.PlannerReference(**PRM)
