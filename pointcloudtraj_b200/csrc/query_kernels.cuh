@@ -124,6 +124,31 @@ __device__ __forceinline__ void pc_consider(const float4 p, float d, float qx, f
     }
 }
 
+// fp64 re-check of a scanned leaf for one query.  A point can be the exact minimiser only if its fp32 d2 is within the
+// fp32 error of the leaf's fp32 minimum dmin: any point with d2 > dmin (1 + 2^-20) + 2^-147 (relative error < 2^-22, and
+// the absolute 2^-147 covers fp32 underflow of tiny distances) has a larger fp64 distance than the minimum's point.  So
+// only the points inside that margin (and inside thr) -- almost always one -- are re-evaluated, in a loop with ONE fp64
+// site instead of one per point; the point is read again (an L1 hit) rather than held in registers.  The result is the
+// one every point's re-check would give: smallest (d2, original index).
+__device__ __forceinline__ void pc_exact_leaf(const float4 *__restrict__ pts, const float (&d)[PC_LEAF], float dmin,
+                                              float qx, float qy, float qz, pc_best &b)
+{
+    if (!(dmin <= b.thr)) return;          // one branch for the whole leaf: after the first leaves almost never taken
+    const float cut = fminf(b.thr, __fmaf_ru(dmin, PC_THR_SLACK, 4.0f * FLT_TRUE_MIN));
+    uint32_t cand = 0;
+#pragma unroll
+    for (int i = 0; i < PC_LEAF; i++) cand |= (d[i] <= cut ? 1u : 0u) << i;
+    const double dqx = qx, dqy = qy, dqz = qz;
+    while (cand) {
+        const float4 p = __ldg(pts + (__ffs(cand) - 1));
+        cand &= cand - 1u;
+        const double e = pc_exact_d2(p.x, p.y, p.z, dqx, dqy, dqz);
+        const int32_t id = __float_as_int(p.w);
+        if (e < b.d2 || (e == b.d2 && (uint32_t)id < (uint32_t)b.idx)) { b.d2 = e; b.idx = id; }
+    }
+    b.thr = fminf(b.thr, pc_thr_from(b.d2));
+}
+
 // Leaf scan for NQ queries of one lane: PC_LEAF consecutive points from an arbitrary start (128-bit loads).  The points
 // behind the leaf's own count are real points of the cloud too (or pad copies of the last one), so scanning them cannot
 // break exactness.
@@ -145,38 +170,26 @@ __device__ __forceinline__ void pc_scan_leaf(const float4 *__restrict__ pts, con
         }
     }
 #pragma unroll
-    for (int j = 0; j < NQ; j++) {
-        if (dmin[j] <= b[j].thr) {          // one branch for the whole leaf: after the first leaves almost never taken
-#pragma unroll
-            for (int i = 0; i < PC_LEAF; i++) pc_consider(p[i], d[j][i], q[j][0], q[j][1], q[j][2], b[j]);
-        }
-    }
+    for (int j = 0; j < NQ; j++) pc_exact_leaf(pts, d[j], dmin[j], q[j][0], q[j][1], q[j][2], b[j]);
 }
 
 // the same leaf scan for the two queries of a lane, distances two at a time (nq* = (-qa, -qb) per axis)
 __device__ __forceinline__ void pc_scan_leaf_x2(const float4 *__restrict__ pts, float2 nqx, float2 nqy, float2 nqz, pc_best (&b)[2])
 {
-    float4 p[PC_LEAF];
-    float2 d[PC_LEAF];
+    float da[PC_LEAF], db[PC_LEAF];
     const float2 zero = make_float2(0.f, 0.f);
-#pragma unroll
-    for (int i = 0; i < PC_LEAF; i++) p[i] = __ldg(pts + i);
     float mina = FLT_MAX, minb = FLT_MAX;
 #pragma unroll
     for (int i = 0; i < PC_LEAF; i++) {
-        const float2 ex = pc_add2(make_float2(p[i].x, p[i].x), nqx), ey = pc_add2(make_float2(p[i].y, p[i].y), nqy),
-                     ez = pc_add2(make_float2(p[i].z, p[i].z), nqz);
-        d[i] = pc_fma2(ez, ez, pc_fma2(ey, ey, pc_fma2(ex, ex, zero)));
-        mina = fminf(mina, d[i].x); minb = fminf(minb, d[i].y);
+        const float4 p = __ldg(pts + i);
+        const float2 ex = pc_add2(make_float2(p.x, p.x), nqx), ey = pc_add2(make_float2(p.y, p.y), nqy),
+                     ez = pc_add2(make_float2(p.z, p.z), nqz);
+        const float2 dd = pc_fma2(ez, ez, pc_fma2(ey, ey, pc_fma2(ex, ex, zero)));
+        da[i] = dd.x; db[i] = dd.y;
+        mina = fminf(mina, dd.x); minb = fminf(minb, dd.y);
     }
-    if (mina <= b[0].thr) {
-#pragma unroll
-        for (int i = 0; i < PC_LEAF; i++) pc_consider(p[i], d[i].x, -nqx.x, -nqy.x, -nqz.x, b[0]);
-    }
-    if (minb <= b[1].thr) {
-#pragma unroll
-        for (int i = 0; i < PC_LEAF; i++) pc_consider(p[i], d[i].y, -nqx.y, -nqy.y, -nqz.y, b[1]);
-    }
+    pc_exact_leaf(pts, da, mina, -nqx.x, -nqy.x, -nqz.x, b[0]);
+    pc_exact_leaf(pts, db, minb, -nqx.y, -nqy.y, -nqz.y, b[1]);
 }
 
 // Core traversal of one query by one thread.  On entry b holds the initial bound (d2 = +inf, idx = -1, thr = bound).
