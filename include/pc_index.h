@@ -10,6 +10,7 @@
  *   pc_index_build              kd_clear + n x kd_insert3(x,y,z,(void*)i)   kdtree.h:49,58  (kdtree.c:143-159,244-251)
  *                               == safeRegionRrtStar::setInput      Planner/src/corridor_finder.cpp:93-99
  *   pc_nearest_batch            kd_nearest3 + kd_res_item + kd_res_free     kdtree.h:67,113,97 (kdtree.c:493-500,641-650,613)
+ *   pc_knn_batch                pcl::search::KdTree nearestKSearch, radiusSearch with max_nn (no counterpart in Utils/kdtree)
  *   pc_range_batch              kd_nearest_range3 + kd_res_size/next/item   kdtree.h:92,100-113 (kdtree.c:595-602)
  *   pc_radius_batch             safeRegionRrtStar::radiusSearch     Planner/src/corridor_finder.cpp:113-133
  *                               (parameters of setParam :17-23, start point of setStartPt :43-50)
@@ -66,7 +67,7 @@ extern "C" {
 /* flags for pc_radius_batch / pc_clearance_batch */
 #define PC_RADIUS_BOUNDED   0  /* default: search only within max_radius + search_margin (exact for the radius) */
 #define PC_RADIUS_FULL_NN   1  /* unbounded search: out_idx is the true nearest point even where the radius clamps */
-/* flags for pc_nearest_batch / pc_radius_batch: reorder the batch along a space-filling (Hilbert) curve first (same results) */
+/* flags for pc_nearest_batch / pc_radius_batch / pc_knn_batch: reorder the batch along a space-filling (Hilbert) curve first (same results) */
 #define PC_QUERY_AUTO      0
 #define PC_QUERY_UNSORTED  2
 #define PC_QUERY_SORTED    4
@@ -137,6 +138,22 @@ int  pc_radius_batch(pc_index *ix, const float *q_xyz, int64_t m, int64_t q_stri
 int  pc_range_batch(pc_index *ix, const float *q_xyz, int64_t m, int64_t q_stride, int space,
                     const double *range, int range_is_scalar,
                     int64_t *out_offsets, int32_t *out_idx, int64_t cap);
+
+/* The k nearest points of every query (pcl::search::KdTree::nearestKSearch; with a bound, radiusSearch(q, r, ..., max_nn = k)).
+ * Row i is out_idx[i*k .. i*k+k) and out_d2[i*k .. i*k+k); either output may be NULL.  Entries are the k smallest points
+ * under the lexicographic order (fp64 d2, original index), d2 the reference's expression of the exactness contract above:
+ * among points tied at the k-th distance the lowest indices win, and at k = 1 this is the tie rule of pc_nearest_batch.
+ * out_d2 holds the fp64 value rounded once to float32.
+ *   max_range < 0    unbounded.
+ *   max_range >= 0   only points with d2 <= max_range^2 (the inclusion test of pc_range_batch, max_range^2 in fp64): a
+ *                    bounded row is the first k entries of pc_range_batch's list for the same range, re-sorted by (d2, index).
+ * Rows with fewer than k points (small cloud, empty index, the bound) are padded with idx -1 and d2 +inf.
+ * k in [1, PC_KNN_MAX], else PC_EINVAL; for more neighbours use pc_range_batch.  space: PC_HOST or PC_DEVICE (the ASYNC
+ * spaces return PC_EINVAL).  flags: PC_QUERY_AUTO / PC_QUERY_UNSORTED / PC_QUERY_SORTED as for pc_nearest_batch.  A handle
+ * in pc_batch_shard mode (n_ranks > 1) returns PC_EINVAL.  k = 1 unbounded runs pc_nearest_batch. */
+#define PC_KNN_MAX 32
+int  pc_knn_batch(pc_index *ix, const float *q_xyz, int64_t m, int64_t q_stride, int space, int flags,
+                  int k, double max_range, int32_t *out_idx, float *out_d2);
 
 /* Arithmetic of the radiusSearch epilogue (pc_radius_batch, pc_clearance_batch) on this handle:
  *   PC_ARITH_FP64 (default)  radius = sqrt(d2) - search_margin in double precision from the kd-tree's fp64 d2 -- the parity

@@ -17,6 +17,7 @@
 #include "build_kernels.cuh"
 #include "query_kernels.cuh"
 #include "range_kernels.cuh"
+#include "knn_kernels.cuh"
 #include "clearance_kernels.cuh"
 #include "grid_kernels.cuh"
 #include "sampler_kernels.cuh"
@@ -133,6 +134,7 @@ struct pc_index {
     int64_t tiny_batch = PC_TINY_BATCH;   // PC_HOST calls up to this many queries take the mapped-memory path (PC_TINY_BATCH_QUERIES, 0 = off)
     bool host_ramp = false;               // PC_HOST calls: smaller first chunks (PC_HOST_RAMP=1 switches it on)
     int64_t host_chunk = PC_HOST_CHUNK;   // PC_HOST calls: queries per pipelined chunk (PC_HOST_CHUNK_QUERIES)
+    int64_t knn_sort_min = 0;             // pc_knn_batch, PC_QUERY_AUTO: smallest batch that is ordered (PC_KNN_SORT_MIN_BATCH; 0 = by k, knn_host.inl)
     char err[256] = "";
 };
 
@@ -304,6 +306,7 @@ extern "C" int pc_index_create(pc_index **out, int device, int64_t max_points, v
         if (const char *v = getenv("PC_COOP_GROUP")) { int b_ = atoi(v); ix->coop_group = (b_ == 32 || b_ == 16 || b_ == 8 || b_ == 4) ? b_ : 0; }
         if (const char *v = getenv("PC_COOP_MAX_BATCH")) { long long b_ = atoll(v); ix->coop_max = ix->coop_max_unbounded = b_ < 0 ? 0 : b_; }
         if (const char *v = getenv("PC_SORT_MIN_BATCH")) { long long b_ = atoll(v); ix->sort_min_radius = ix->sort_min_nearest = b_ < 1 ? 1 : b_; }
+        if (const char *v = getenv("PC_KNN_SORT_MIN_BATCH")) { long long b_ = atoll(v); ix->knn_sort_min = b_ < 0 ? 0 : b_; }
         if (const char *v = getenv("PC_TINY_BATCH_QUERIES")) { long long b_ = atoll(v); ix->tiny_batch = b_ < 0 ? 0 : (b_ > PC_TINY_BATCH ? PC_TINY_BATCH : b_); }
         if (cuda_stream) { ix->stream = (cudaStream_t)cuda_stream; ix->own_stream = false; }
         else { TRY(cudaStreamCreateWithFlags(&ix->stream, cudaStreamNonBlocking)); ix->own_stream = true; }
@@ -1166,6 +1169,7 @@ extern "C" int pc_radius_batch(pc_index *ix, const float *q_xyz, int64_t m, int6
 }
 
 #include "range_host.inl"
+#include "knn_host.inl"
 #include "clearance_host.inl"
 #include "sampler_host.inl"
 #include "comm_host.inl"
