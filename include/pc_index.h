@@ -12,6 +12,7 @@
  *   pc_nearest_batch            kd_nearest3 + kd_res_item + kd_res_free     kdtree.h:67,113,97 (kdtree.c:493-500,641-650,613)
  *   pc_knn_batch                pcl::search::KdTree nearestKSearch, radiusSearch with max_nn (no counterpart in Utils/kdtree)
  *   pc_range_batch              kd_nearest_range3 + kd_res_size/next/item   kdtree.h:92,100-113 (kdtree.c:595-602)
+ *   pc_range_sorted_batch       pcl::search::KdTree radiusSearch(q, r, k_indices, k_sqr_distances, max_nn), any max_nn
  *   pc_radius_batch             safeRegionRrtStar::radiusSearch     Planner/src/corridor_finder.cpp:113-133
  *                               (parameters of setParam :17-23, start point of setStartPt :43-50)
  *   pc_clearance_batch          checkSafeTrajectory + getPosFromBezier + checkTrajPtCol
@@ -139,6 +140,20 @@ int  pc_range_batch(pc_index *ix, const float *q_xyz, int64_t m, int64_t q_strid
                     const double *range, int range_is_scalar,
                     int64_t *out_offsets, int32_t *out_idx, int64_t cap);
 
+/* pcl::search::KdTree::radiusSearch(q, r, k_indices, k_sqr_distances, max_nn) for a batch, exactly.  Row i holds the hit set
+ * of pc_range_batch for the same (q, range) -- d2 <= range^2 in fp64, inclusive -- ascending by (fp64 d2, original index):
+ * points at equal distance come lowest index first, the tie rule of pc_knn_batch.
+ *   max_nn == 0   every hit;  max_nn > 0   the first max_nn entries of that order;  max_nn < 0   PC_EINVAL.
+ * out_offsets[m+1] is the CSR row pointer over the row lengths min(hits, max_nn); out_idx[cap] the concatenated rows;
+ * out_d2[cap] (nullable) each entry's fp64 d2 rounded once to float32, the value pc_knn_batch writes.  Capacity as for
+ * pc_range_batch: a total above cap returns PC_ECAP with out_offsets complete; out_idx == NULL, out_d2 == NULL, cap == 0
+ * returns the offsets only (PC_OK).  space: PC_HOST or PC_DEVICE (the ASYNC spaces return PC_EINVAL).  A pc_batch_shard
+ * handle answers every query, as pc_range_batch does.  With a scalar range and max_nn <= PC_KNN_MAX a row equals the
+ * non-padding prefix of pc_knn_batch(k = max_nn, max_range = range). */
+int  pc_range_sorted_batch(pc_index *ix, const float *q_xyz, int64_t m, int64_t q_stride, int space,
+                           const double *range, int range_is_scalar, int64_t max_nn,
+                           int64_t *out_offsets, int32_t *out_idx, float *out_d2, int64_t cap);
+
 /* The k nearest points of every query (pcl::search::KdTree::nearestKSearch; with a bound, radiusSearch(q, r, ..., max_nn = k)).
  * Row i is out_idx[i*k .. i*k+k) and out_d2[i*k .. i*k+k); either output may be NULL.  Entries are the k smallest points
  * under the lexicographic order (fp64 d2, original index), d2 the reference's expression of the exactness contract above:
@@ -148,7 +163,7 @@ int  pc_range_batch(pc_index *ix, const float *q_xyz, int64_t m, int64_t q_strid
  *   max_range >= 0   only points with d2 <= max_range^2 (the inclusion test of pc_range_batch, max_range^2 in fp64): a
  *                    bounded row is the first k entries of pc_range_batch's list for the same range, re-sorted by (d2, index).
  * Rows with fewer than k points (small cloud, empty index, the bound) are padded with idx -1 and d2 +inf.
- * k in [1, PC_KNN_MAX], else PC_EINVAL; for more neighbours use pc_range_batch.  space: PC_HOST or PC_DEVICE (the ASYNC
+ * k in [1, PC_KNN_MAX], else PC_EINVAL; for more neighbours use pc_range_sorted_batch.  space: PC_HOST or PC_DEVICE (the ASYNC
  * spaces return PC_EINVAL).  flags: PC_QUERY_AUTO / PC_QUERY_UNSORTED / PC_QUERY_SORTED as for pc_nearest_batch.  A handle
  * in pc_batch_shard mode (n_ranks > 1) returns PC_EINVAL.  k = 1 unbounded runs pc_nearest_batch. */
 #define PC_KNN_MAX 32

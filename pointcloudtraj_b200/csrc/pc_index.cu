@@ -18,6 +18,7 @@
 #include "query_kernels.cuh"
 #include "range_kernels.cuh"
 #include "knn_kernels.cuh"
+#include "range_sorted_kernels.cuh"
 #include "clearance_kernels.cuh"
 #include "grid_kernels.cuh"
 #include "sampler_kernels.cuh"
@@ -87,6 +88,8 @@ struct pc_index {
 
     // generic device scratch for range / clearance / expansion batches
     void *scratch = nullptr; int64_t scratch_cap = 0;
+    // pc_range_sorted_batch: the lists too long for the capturing warp, untruncated (fp64 d2, then original index)
+    uint32_t *range_long = nullptr; int64_t range_long_cap = 0;
     // pc_expand_batch: running candidate totals per chunk (pinned) and the events the host waits on before copying a chunk back
     char *h_stage = nullptr;           // pc_clearance_batch: pinned staging block of small PC_HOST calls
     unsigned long long *h_totals = nullptr;
@@ -390,7 +393,7 @@ extern "C" void pc_index_destroy(pc_index *ix)
     if (ix->tiny_i) cudaFreeHost(ix->tiny_i);
     cudaFree(ix->d_xyz); cudaFree(ix->d_bbox); cudaFree(ix->keys_a); cudaFree(ix->keys_b);
     cudaFree(ix->vals_a); cudaFree(ix->vals_b); cudaFree(ix->tile_hist); cudaFree(ix->digit_total);
-    cudaFree(ix->tree); cudaFree(ix->scratch); cudaFree(ix->grid_cell_start); cudaFree(ix->grid_points); cudaFree(ix->hilbert_lut);
+    cudaFree(ix->tree); cudaFree(ix->scratch); cudaFree(ix->range_long); cudaFree(ix->grid_cell_start); cudaFree(ix->grid_points); cudaFree(ix->hilbert_lut);
     if (ix->ev_b0) cudaEventDestroy(ix->ev_b0);
     if (ix->ev_b1) cudaEventDestroy(ix->ev_b1);
     if (ix->ev_ready) cudaEventDestroy(ix->ev_ready);
@@ -1169,6 +1172,7 @@ extern "C" int pc_radius_batch(pc_index *ix, const float *q_xyz, int64_t m, int6
 }
 
 #include "range_host.inl"
+#include "range_sorted_host.inl"
 #include "knn_host.inl"
 #include "clearance_host.inl"
 #include "sampler_host.inl"

@@ -214,6 +214,44 @@ class PointCloudIndex:
             raise L.PcError(rc, f"range: {int(off[-1])} hits exceed cap {cap}")
         return off, out[: int(off[-1])]
 
+    def range_sorted(self, q, r, max_nn=0, cap=None):
+        """pcl radiusSearch(q, r, k_indices, k_sqr_distances, max_nn) for every row of q (pc_range_sorted_batch).  r: one
+        radius or one per query; max_nn = 0 keeps every hit.  Returns (offsets int64[m+1], idx int32[total], d2 float32[total]),
+        each row ascending by (d2, index) and cut to max_nn.  numpy queries give numpy arrays; torch CUDA tensors give tensors
+        (sized by an offsets-only call first)."""
+        p, m, stride, space, keep, tm = self._rows(q, "q")
+        max_nn = int(max_nn)
+        if tm:
+            import torch
+            rr = torch.as_tensor(r, dtype=torch.float64, device=keep.device).reshape(-1).contiguous()
+            n_r, pr = rr.shape[0], C.c_void_p(rr.data_ptr())
+            off = torch.zeros(m + 1, dtype=torch.int64, device=keep.device)
+            poff = C.c_void_p(off.data_ptr())
+        else:
+            rr = np.ascontiguousarray(np.atleast_1d(r), dtype=np.float64)
+            n_r, pr = rr.shape[0], C.c_void_p(rr.ctypes.data)
+            off = np.zeros(m + 1, dtype=np.int64)
+            poff = C.c_void_p(off.ctypes.data)
+        scalar = 1 if n_r == 1 else 0
+        if not scalar and n_r != m:
+            raise ValueError("range_sorted: need one radius or one per query")
+        call = lambda pi, pd, c: self._L.pc_range_sorted_batch(self._h, p, m, stride, space, pr, scalar, max_nn, poff, pi, pd, c)
+        self._torch_fence(tm)
+        if cap is None:
+            self._check(call(C.c_void_p(0), C.c_void_p(0), 0))
+            self._torch_fence(tm, after=True)
+            cap = int(off[-1])
+        cap = int(cap)
+        idx, pi = self._out(max(cap, 1), np.int32, tm, keep)
+        d2, pd = self._out(max(cap, 1), np.float32, tm, keep)
+        rc = call(pi, pd, cap)
+        self._torch_fence(tm, after=True)
+        self._check(rc, ok=(L.PC_OK, L.PC_ECAP))
+        total = int(off[-1])
+        if rc == L.PC_ECAP:
+            raise L.PcError(rc, f"range_sorted: {total} hits exceed cap {cap}")
+        return off, idx[:total], d2[:total]
+
     def sphere_gather(self, center, radius):
         """All points within `radius` of `center`, ascending original index (camera_sensor.cpp:133-145, LiDAR mode)."""
         c = (C.c_double * 3)(*[float(v) for v in center])
