@@ -11,6 +11,7 @@
  *                               == safeRegionRrtStar::setInput      Planner/src/corridor_finder.cpp:93-99
  *   pc_nearest_batch            kd_nearest3 + kd_res_item + kd_res_free     kdtree.h:67,113,97 (kdtree.c:493-500,641-650,613)
  *   pc_knn_batch                pcl::search::KdTree nearestKSearch, radiusSearch with max_nn (no counterpart in Utils/kdtree)
+ *   pc_knn_large_batch          pcl::search::KdTree nearestKSearch with 32 < k <= 1024
  *   pc_range_batch              kd_nearest_range3 + kd_res_size/next/item   kdtree.h:92,100-113 (kdtree.c:595-602)
  *   pc_range_sorted_batch       pcl::search::KdTree radiusSearch(q, r, k_indices, k_sqr_distances, max_nn), any max_nn
  *   pc_radius_batch             safeRegionRrtStar::radiusSearch     Planner/src/corridor_finder.cpp:113-133
@@ -68,7 +69,7 @@ extern "C" {
 /* flags for pc_radius_batch / pc_clearance_batch */
 #define PC_RADIUS_BOUNDED   0  /* default: search only within max_radius + search_margin (exact for the radius) */
 #define PC_RADIUS_FULL_NN   1  /* unbounded search: out_idx is the true nearest point even where the radius clamps */
-/* flags for pc_nearest_batch / pc_radius_batch / pc_knn_batch: reorder the batch along a space-filling (Hilbert) curve first (same results) */
+/* flags for pc_nearest_batch / pc_radius_batch / pc_knn_batch / pc_knn_large_batch: reorder the batch along a space-filling (Hilbert) curve first (same results) */
 #define PC_QUERY_AUTO      0
 #define PC_QUERY_UNSORTED  2
 #define PC_QUERY_SORTED    4
@@ -163,12 +164,25 @@ int  pc_range_sorted_batch(pc_index *ix, const float *q_xyz, int64_t m, int64_t 
  *   max_range >= 0   only points with d2 <= max_range^2 (the inclusion test of pc_range_batch, max_range^2 in fp64): a
  *                    bounded row is the first k entries of pc_range_batch's list for the same range, re-sorted by (d2, index).
  * Rows with fewer than k points (small cloud, empty index, the bound) are padded with idx -1 and d2 +inf.
- * k in [1, PC_KNN_MAX], else PC_EINVAL; for more neighbours use pc_range_sorted_batch.  space: PC_HOST or PC_DEVICE (the ASYNC
+ * k in [1, PC_KNN_MAX], else PC_EINVAL; for more neighbours use pc_knn_large_batch (k <= PC_KNN_LARGE_MAX, bounded or
+ * not) or pc_range_sorted_batch (bounded, any length).  space: PC_HOST or PC_DEVICE (the ASYNC
  * spaces return PC_EINVAL).  flags: PC_QUERY_AUTO / PC_QUERY_UNSORTED / PC_QUERY_SORTED as for pc_nearest_batch.  A handle
  * in pc_batch_shard mode (n_ranks > 1) returns PC_EINVAL.  k = 1 unbounded runs pc_nearest_batch. */
 #define PC_KNN_MAX 32
 int  pc_knn_batch(pc_index *ix, const float *q_xyz, int64_t m, int64_t q_stride, int space, int flags,
                   int k, double max_range, int32_t *out_idx, float *out_d2);
+
+/* pcl::search::KdTree nearestKSearch(q, k) for 1 <= k <= PC_KNN_LARGE_MAX: the arguments, rows, order, bound, padding,
+ * spaces and flags of pc_knn_batch, with longer rows.  Row i is out_idx[i*k .. i*k+k) / out_d2[i*k .. i*k+k) (either output
+ * may be NULL): the k smallest points under (fp64 d2, original index), ties at the k-th distance to the lowest index, d2
+ * rounded once to float32; max_range >= 0 keeps only points with d2 <= max_range^2 (pc_range_batch's test), max_range < 0
+ * is unbounded, a NaN max_range returns PC_EINVAL; short rows are padded with idx -1 and d2 +inf.
+ * k outside [1, PC_KNN_LARGE_MAX], the ASYNC spaces, unknown flags and a pc_batch_shard handle return PC_EINVAL; longer
+ * bounded lists come from pc_range_sorted_batch.  k <= PC_KNN_MAX runs pc_knn_batch.  The first PC_KNN_MAX columns of a row
+ * are pc_knn_batch's row for k = PC_KNN_MAX, and a bounded row is the row of pc_range_sorted_batch with max_nn = k. */
+#define PC_KNN_LARGE_MAX 1024
+int  pc_knn_large_batch(pc_index *ix, const float *q_xyz, int64_t m, int64_t q_stride, int space, int flags,
+                        int k, double max_range, int32_t *out_idx, float *out_d2);
 
 /* Arithmetic of the radiusSearch epilogue (pc_radius_batch, pc_clearance_batch) on this handle:
  *   PC_ARITH_FP64 (default)  radius = sqrt(d2) - search_margin in double precision from the kd-tree's fp64 d2 -- the parity

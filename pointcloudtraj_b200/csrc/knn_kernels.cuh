@@ -14,6 +14,7 @@
 //                         (lane j holds the j-th entry); also answers the queries of the packets the packet kernel puts aside
 //   pc_knn_packet_kernel  one warp walks the tree once for the 32 neighbouring queries of a curve-ordered batch (the walk of
 //                         pc_packet_traverse); every lane keeps its query's k-list in shared memory
+// The warp walk (pc_knn_warp_search) is a template over the list, shared with pc_knn_large_kernel (knn_large_kernels.cuh).
 #pragma once
 #include "query_kernels.cuh"
 
@@ -74,10 +75,12 @@ __device__ __forceinline__ void pc_knn_warp_insert(bool have, double e, uint32_t
     W.thr = fminf(K.bound_thr, pc_thr_from(W.kd));
 }
 
-// scan NL leaves per lane (ref with PC_REF_LEAF, cnt points each; cnt 0 = none) and offer the survivors to the list
-template <int NL>
+// scan NL leaves per lane (ref with PC_REF_LEAF, cnt points each; cnt 0 = none) and offer the survivors to the list.
+// LIST: pc_knn_wlist (this file) or pc_knn_qlist (knn_large_kernels.cuh); each has its pc_knn_warp_insert and a warp-uniform
+// filter W.thr.
+template <int NL, typename LIST>
 __device__ __forceinline__ void pc_knn_warp_scan(const pc_tree &T, const uint32_t (&ref)[NL], const uint32_t (&cnt)[NL],
-                                                 float qx, float qy, float qz, int lane, const pc_knn_dev &K, pc_knn_wlist &W)
+                                                 float qx, float qy, float qz, int lane, const pc_knn_dev &K, LIST &W)
 {
     float d[NL * PC_LEAF];
 #pragma unroll
@@ -108,8 +111,9 @@ __device__ __forceinline__ void pc_knn_warp_scan(const pc_tree &T, const uint32_
     }
 }
 
+template <typename LIST>
 __device__ __forceinline__ void pc_knn_warp_search(const pc_tree &T, const pc_knn_dev &K, float qx, float qy, float qz,
-                                                   uint2 *__restrict__ F, int lane, pc_knn_wlist &W)
+                                                   uint2 *__restrict__ F, int lane, LIST &W)
 {
     const uint32_t lt = (1u << lane) - 1u;
     // the seeds: leaves met while the top of the tree was expanded (one per lane, their own counts) and <= 32 inner nodes

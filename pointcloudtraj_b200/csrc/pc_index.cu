@@ -18,6 +18,7 @@
 #include "query_kernels.cuh"
 #include "range_kernels.cuh"
 #include "knn_kernels.cuh"
+#include "knn_large_kernels.cuh"
 #include "range_sorted_kernels.cuh"
 #include "clearance_kernels.cuh"
 #include "grid_kernels.cuh"
@@ -1174,6 +1175,7 @@ extern "C" int pc_radius_batch(pc_index *ix, const float *q_xyz, int64_t m, int6
 #include "range_host.inl"
 #include "range_sorted_host.inl"
 #include "knn_host.inl"
+#include "knn_large_host.inl"
 #include "clearance_host.inl"
 #include "sampler_host.inl"
 #include "comm_host.inl"

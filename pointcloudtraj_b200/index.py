@@ -168,6 +168,20 @@ class PointCloudIndex:
         self._torch_fence(tm, after=True)
         return idx.reshape(m, k), d2.reshape(m, k)
 
+    def knn_large(self, q, k, max_range=None, flags=L.PC_QUERY_AUTO):
+        """knn() for k up to PC_KNN_LARGE_MAX (pc_knn_large_batch; pcl nearestKSearch with any k a kd-tree user asks for).
+        Returns (idx int32 (m, k), d2 float32 (m, k)), each row ascending by (d2, index), padded with -1 / inf; numpy queries give
+        numpy arrays, torch CUDA tensors give tensors."""
+        p, m, stride, space, keep, tm = self._rows(q, "q")
+        k = int(k)
+        idx, pi = self._out(m * k, np.int32, tm, keep)
+        d2, pd = self._out(m * k, np.float32, tm, keep)
+        r = -1.0 if max_range is None else float(max_range)
+        self._torch_fence(tm)
+        self._check(self._L.pc_knn_large_batch(self._h, p, m, stride, space, int(flags), k, r, pi, pd))
+        self._torch_fence(tm, after=True)
+        return idx.reshape(m, k), d2.reshape(m, k)
+
     def radius(self, q, params: L.PcRadiusParams, flags=L.PC_RADIUS_BOUNDED, want_idx=False):
         """safeRegionRrtStar::radiusSearch for every row of q.  Returns radius float32 (and idx int32)."""
         p, m, stride, space, keep, tm = self._rows(q, "q")
