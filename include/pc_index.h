@@ -251,7 +251,7 @@ typedef struct pc_candidate {      /* one new node the expansion loop would go o
  * rebuilt here), radiusSearch answers the centres against `cloud`'s index, and only the candidates the loop would keep
  * (nearest vertex valid, centre z >= z_l, radius >= safety_margin, :726-731) come back, in sample order.  out: host memory,
  * cap entries; *out_count is always the number of candidates (PC_ECAP if it exceeds cap).  Both handles must live on the
- * same device.  Identical, candidate for candidate, with k x genSample + pc_nearest_batch + steering on the host +
+ * same device; a pc_batch_shard handle on either side (n_ranks > 1) returns PC_EINVAL.  Identical, candidate for candidate, with k x genSample + pc_nearest_batch + steering on the host +
  * pc_radius_batch (tests/test_sampler_gpu.py). */
 int  pc_expand_batch(pc_index *cloud, pc_index *nodes, const pc_node_set *set, const pc_sampler *sampler,
                      const pc_radius_params *params, double z_l, double safety_margin, int64_t k,

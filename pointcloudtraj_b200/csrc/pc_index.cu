@@ -886,6 +886,7 @@ static int pc_run_batch(pc_index *ix, pc_lane &L, const pc_qargs &A, const float
         RN.defer_list = L.keys_a;               // the ordering pass is done with its key buffer; one entry per packet at most
         if (!(RN.packet_split > 0.f) || !is_ordered) RN.packet_split = 0.f;
     }
+    bool packet_walk = false;           // pc_query_packet_kernel ran: it may have put packets aside for the deferred kernel
     if (ml == 0) {
         // pc_batch_shard: nothing of this batch belongs to this rank
     } else if (ix->grid_ready && is_ordered && A.kind == PC_Q_RADIUS && A.R.bounded) {
@@ -896,6 +897,7 @@ static int pc_run_batch(pc_index *ix, pc_lane &L, const pc_qargs &A, const float
         // curve-ordered batch: one warp walks the tree once for its 32 or 64 neighbouring queries
         const int per_cta = (ix->query_kernel == 5 ? 4 : (two_per_lane ? 2 : 1)) * PC_QUERY_THREADS;
         const int grid = (int)((ml + per_cta - 1) / per_cta);
+        packet_walk = true;
         if (ix->query_kernel == 5) {           // experiment: 128-query packets, four queries per lane
             if (A.kind == PC_Q_NEAREST)
                 pc_query_packet_kernel<PC_KIND_NEAREST, 4><<<grid, PC_QUERY_THREADS, 0, L.stream>>>(T, RN, d_q, m, qstride, perm, ordered, m_eff, d_idx, d_f);
@@ -921,7 +923,7 @@ static int pc_run_batch(pc_index *ix, pc_lane &L, const pc_qargs &A, const float
             pc_query_simple_kernel<PC_KIND_RADIUS><<<grid, PC_QUERY_THREADS, 0, L.stream>>>(T, A.R, d_q, m, qstride, perm, ordered, m_eff, d_idx, d_f);
     }
     if (ml > 0) ix->launches++;
-    if (ml > 0 && RN.packet_split > 0.f && ix->query_kernel >= 3 && is_ordered && !ix->grid_ready) {
+    if (packet_walk && RN.packet_split > 0.f) {
         // the packets the walk above put aside as incoherent (normally none or a handful: the kernel then costs its launch)
         const int dgrid = ix->sm_count * PC_DEFER_CTAS_PER_SM;
         const int per_packet = 32 * (ix->query_kernel == 5 ? 4 : (two_per_lane ? 2 : 1));
