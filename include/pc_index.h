@@ -12,6 +12,7 @@
  *   pc_nearest_batch            kd_nearest3 + kd_res_item + kd_res_free     kdtree.h:67,113,97 (kdtree.c:493-500,641-650,613)
  *   pc_knn_batch                pcl::search::KdTree nearestKSearch, radiusSearch with max_nn (no counterpart in Utils/kdtree)
  *   pc_knn_large_batch          pcl::search::KdTree nearestKSearch with 32 < k <= 1024
+ *   pc_segment_nearest_batch    (no counterpart: the reference samples points along an edge) nearest point to a segment
  *   pc_range_batch              kd_nearest_range3 + kd_res_size/next/item   kdtree.h:92,100-113 (kdtree.c:595-602)
  *   pc_range_sorted_batch       pcl::search::KdTree radiusSearch(q, r, k_indices, k_sqr_distances, max_nn), any max_nn
  *   pc_radius_batch             safeRegionRrtStar::radiusSearch     Planner/src/corridor_finder.cpp:113-133
@@ -69,7 +70,7 @@ extern "C" {
 /* flags for pc_radius_batch / pc_clearance_batch */
 #define PC_RADIUS_BOUNDED   0  /* default: search only within max_radius + search_margin (exact for the radius) */
 #define PC_RADIUS_FULL_NN   1  /* unbounded search: out_idx is the true nearest point even where the radius clamps */
-/* flags for pc_nearest_batch / pc_radius_batch / pc_knn_batch / pc_knn_large_batch: reorder the batch along a space-filling (Hilbert) curve first (same results) */
+/* flags for pc_nearest_batch / pc_radius_batch / pc_knn_batch / pc_knn_large_batch / pc_segment_nearest_batch: reorder the batch along a space-filling (Hilbert) curve first (same results) */
 #define PC_QUERY_AUTO      0
 #define PC_QUERY_UNSORTED  2
 #define PC_QUERY_SORTED    4
@@ -183,6 +184,25 @@ int  pc_knn_batch(pc_index *ix, const float *q_xyz, int64_t m, int64_t q_stride,
 #define PC_KNN_LARGE_MAX 1024
 int  pc_knn_large_batch(pc_index *ix, const float *q_xyz, int64_t m, int64_t q_stride, int space, int flags,
                         int k, double max_range, int32_t *out_idx, float *out_d2);
+
+/* Nearest cloud point to each line segment [a_i, b_i] (float32 endpoints, stride 3 or 4, a and b in the same space).
+ * Distance: A = a, B = b, P = p widened to double; D = B - A, W = P - A per axis; L2 = (Dx*Dx + Dy*Dy) + Dz*Dz,
+ * s = (Wx*Dx + Wy*Dy) + Wz*Dz, every operation rounded to nearest, never fused:
+ *   s <= 0 or L2 == 0   d2 = the reference's expression of P against A (the exactness contract above)
+ *   s >= L2             d2 = the same against B
+ *   otherwise           t = s / L2 (IEEE division), E = W - t*D per axis, d2 = (Ex*Ex + Ey*Ey) + Ez*Ez.
+ * out_idx[i] is the point with the smallest d2, the lowest original index among exact ties; out_d2[i] that fp64 value
+ * rounded once to float32.  A segment with a == b gives exactly pc_nearest_batch's (idx, d2) for the point a.
+ *   max_range < 0    unbounded.
+ *   max_range >= 0   only points with d2 <= max_range^2 (pc_range_batch's test); a row without one gets idx -1, d2 +inf.
+ * An empty index gives idx -1, d2 +inf.  A segment with a non-finite endpoint coordinate gives idx -1 and d2 NaN (empty
+ * index or not): a collision check `d2 < r*r` must treat NaN as "not checked", e.g. test !(d2 >= r*r).
+ * A polyline of n points is checked with b_xyz = a_xyz + stride and m = n - 1 (the two arrays may overlap).
+ * Either output may be NULL.  space: PC_HOST or PC_DEVICE.  flags: PC_QUERY_AUTO / PC_QUERY_UNSORTED / PC_QUERY_SORTED
+ * (SORTED orders the segments along the curve by their midpoints first; same results).  PC_EINVAL: a bad stride, a NULL
+ * a_xyz / b_xyz with m > 0, the ASYNC spaces, unknown flags, a NaN max_range, a pc_batch_shard handle (n_ranks > 1). */
+int  pc_segment_nearest_batch(pc_index *ix, const float *a_xyz, const float *b_xyz, int64_t m, int64_t stride,
+                              int space, int flags, double max_range, int32_t *out_idx, float *out_d2);
 
 /* Arithmetic of the radiusSearch epilogue (pc_radius_batch, pc_clearance_batch) on this handle:
  *   PC_ARITH_FP64 (default)  radius = sqrt(d2) - search_margin in double precision from the kd-tree's fp64 d2 -- the parity

@@ -20,6 +20,7 @@
 #include "knn_kernels.cuh"
 #include "knn_large_kernels.cuh"
 #include "range_sorted_kernels.cuh"
+#include "segment_kernels.cuh"
 #include "clearance_kernels.cuh"
 #include "grid_kernels.cuh"
 #include "sampler_kernels.cuh"
@@ -52,6 +53,7 @@ struct pc_lane {
     unsigned long long *counter = nullptr;                   // [1]: queries that still need a search after the ordering pass
     uint32_t *bins = nullptr; int64_t bins_cap = 0;          // cell-binning ordering: 2^bits counters / cursors + their tile sums
     float4 *ordered = nullptr; int64_t ordered_cap = 0;      // cell-binning ordering: the batch gathered into cell order
+    float4 *d_mid = nullptr; int64_t mid_cap = 0;            // pc_segment_nearest_batch: the segments' midpoints (ordering keys)
     double per_cell = 0.0;                                   // last ordered batch: estimated queries per 1/256-extent cell
     cudaEvent_t done = nullptr;
     cudaStream_t order_stream = nullptr;                     // high-priority stream for the ordering pass of pipelined batches
@@ -374,7 +376,7 @@ extern "C" void pc_index_destroy(pc_index *ix)
         if (L.stream && L.own_stream) { cudaStreamSynchronize(L.stream); cudaStreamDestroy(L.stream); }
         cudaFree(L.d_q); cudaFree(L.d_i32); cudaFree(L.d_f32);
         cudaFree(L.keys_a); cudaFree(L.keys_b); cudaFree(L.vals_a); cudaFree(L.vals_b);
-        cudaFree(L.tile_hist); cudaFree(L.digit_total); cudaFree(L.counter); cudaFree(L.bins); cudaFree(L.ordered);
+        cudaFree(L.tile_hist); cudaFree(L.digit_total); cudaFree(L.counter); cudaFree(L.bins); cudaFree(L.ordered); cudaFree(L.d_mid);
         if (L.done) cudaEventDestroy(L.done);
         if (L.ev_deps) cudaEventDestroy(L.ev_deps);
         if (L.ev_ordered) cudaEventDestroy(L.ev_ordered);
@@ -1178,6 +1180,7 @@ extern "C" int pc_radius_batch(pc_index *ix, const float *q_xyz, int64_t m, int6
 #include "range_sorted_host.inl"
 #include "knn_host.inl"
 #include "knn_large_host.inl"
+#include "segment_host.inl"
 #include "clearance_host.inl"
 #include "sampler_host.inl"
 #include "comm_host.inl"

@@ -182,6 +182,22 @@ class PointCloudIndex:
         self._torch_fence(tm, after=True)
         return idx.reshape(m, k), d2.reshape(m, k)
 
+    def segment_nearest(self, a, b, max_range=None, flags=L.PC_QUERY_AUTO):
+        """The nearest cloud point to every segment [a[i], b[i]] (pc_segment_nearest_batch); with max_range only points within
+        it.  Returns (idx int32, d2 float32): -1 / inf where no point counts, -1 / NaN for a non-finite endpoint.  a and b are
+        both numpy arrays or both torch CUDA tensors of the same shape."""
+        pa, m, stride, space, keep_a, tm = self._rows(a, "a")
+        pb, mb, stride_b, space_b, keep_b, _ = self._rows(b, "b")
+        if (mb, stride_b, space_b) != (m, stride, space):
+            raise ValueError("segment_nearest: a and b need the same shape and memory space")
+        idx, pi = self._out(m, np.int32, tm, keep_a)
+        d2, pd = self._out(m, np.float32, tm, keep_a)
+        r = -1.0 if max_range is None else float(max_range)
+        self._torch_fence(tm)
+        self._check(self._L.pc_segment_nearest_batch(self._h, pa, pb, m, stride, space, int(flags), r, pi, pd))
+        self._torch_fence(tm, after=True)
+        return idx, d2
+
     def radius(self, q, params: L.PcRadiusParams, flags=L.PC_RADIUS_BOUNDED, want_idx=False):
         """safeRegionRrtStar::radiusSearch for every row of q.  Returns radius float32 (and idx int32)."""
         p, m, stride, space, keep, tm = self._rows(q, "q")
