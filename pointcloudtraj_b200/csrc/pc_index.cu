@@ -22,7 +22,6 @@
 #include "range_sorted_kernels.cuh"
 #include "segment_kernels.cuh"
 #include "clearance_kernels.cuh"
-#include "grid_kernels.cuh"
 #include "sampler_kernels.cuh"
 
 #define PC_VERSION_STRING "pcindex 0.2 (sm_100a)"
@@ -35,7 +34,6 @@
 #define PC_SORT_MIN_NEAREST 360000      // query on the UNORDERED batch is faster on the prefix-split tree (profiles/r2_mid_batch_ab.txt)
 #define PC_COOP_MAX_BATCH 24576         // unordered batches up to this size: a group of lanes per query (profiles/r2_small_batch_ab.txt)
 #define PC_COOP_MAX_BATCH_UNBOUNDED 8192
-#define PC_SORT_MIN_BATCH (1 << 17)     // smallest chunk of a pipelined PC_HOST call
 #define PC_SHARD_EXACT_MIN (1 << 20)    // pc_batch_shard: batches at least this large read their share's size back (see pc_share_size)
 
 static thread_local char g_create_error[256] = "";
@@ -105,10 +103,9 @@ struct pc_index {
 
     int64_t launches = 0;
     bool profile = false, profiled = false;
-    // tuning knobs (environment: PC_QUERY_KERNEL, PC_SORT_BITS), see DESIGN.md "Query kernel variants"
-    int query_kernel = 3;     // 1 = thread per query, 3 = warp packets of 32 (ordered batches) / warp per query (small
-                              // unordered ones), 4 = packets of 64
-    bool query_kernel_auto = true;   // no PC_QUERY_KERNEL in the environment: 3, or 4 for dense batches
+    // tuning knobs (environment: PC_QUERY_KERNEL, PC_SORT_BITS), see DESIGN.md §4.6
+    int query_kernel = 3;     // packets of ordered batches: 3 = 32 queries, 4 = 64 queries (two per lane)
+    bool query_kernel_auto = true;   // PC_QUERY_KERNEL neither 3 nor 4: 3, or 4 for dense batches
     int sort_bits = 24;       // radix-sorted key width of the batch ordering pass (0 = never order)
     bool sort_bits_auto = true;   // no PC_SORT_BITS in the environment: pick 24 or 32 from the batch density
     int next_lane = 0;        // PC_HOST_ASYNC: lane of the next batch
@@ -118,19 +115,10 @@ struct pc_index {
     double trace_slow_ms = 0.0;        // PC_TRACE_SLOW_MS: pc_range_batch calls slower than this report their host-side phases
     bool shard_exact = true;           // pc_batch_shard: read the size of the share back (8 bytes, one stream sync) and size the sort / search launches by it
     int radius_arith = PC_ARITH_FP64;  // pc_index_set_radius_arith
-    // experiment (PC_GRID=1): the voxel grid of grid_kernels.cuh next to the tree, used by bounded radius batches
-    bool use_grid = false, grid_ready = false;
-    double grid_cell = 0.5;            // requested cell edge in metres (PC_GRID_CELL)
-    pc_grid grid;
-    uint32_t *grid_cell_start = nullptr; int64_t grid_cells_cap = 0;
-    float4 *grid_points = nullptr; int64_t grid_points_cap = 0;
     bool onesweep = true;              // PC_ONESWEEP=0: the three-kernel-per-pass radix sort (radix_sort.cuh)
     uint16_t *hilbert_lut = nullptr;   // 16^3 + 32^3 Hilbert indices for the cell binning (pc_hilbert_lut_kernel)
     int key_ctas_per_sm = 0, sortkey_ctas_per_sm = 0;   // occupancy of the bin-count / key kernels (queried once)
     int bin_bits = 0;                  // PC_BIN_BITS: log2 of the number of cells of the binning (0 = from the batch size)
-    bool order_bins_all = false;       // PC_ORDER_BINS=2: bin unbounded (nearest / full-NN) batches too
-    bool order_bins = true;            // PC_ORDER_BINS=0: always radix-sort the batch instead of binning it by cell
-    int sort_items = 16;               // keys per thread of the batch-ordering sort (PC_SORT_ITEMS = 8 | 16)
     int coop_group = 0;                     // lanes per query of the small-batch kernel: 0 = by batch size, else 32 / 16 / 8 (PC_COOP_GROUP)
     int64_t coop_g32_max = 6144, coop_g16_max = 12288;   // batch sizes up to which 32 / 16 lanes per query are used (8 above)
     int64_t coop_max = PC_COOP_MAX_BATCH;   // unordered batches up to this size run a group of lanes per query (PC_COOP_MAX_BATCH)
@@ -138,7 +126,6 @@ struct pc_index {
                                             // beyond 8 k queries one thread per query wins (profiles/r2_coop_group_ab.txt: 24 k nearest 0.17 -> 0.11 ms)
     int64_t sort_min_radius = PC_SORT_MIN_RADIUS, sort_min_nearest = PC_SORT_MIN_NEAREST;   // PC_SORT_MIN_BATCH sets both
     int64_t tiny_batch = PC_TINY_BATCH;   // PC_HOST calls up to this many queries take the mapped-memory path (PC_TINY_BATCH_QUERIES, 0 = off)
-    bool host_ramp = false;               // PC_HOST calls: smaller first chunks (PC_HOST_RAMP=1 switches it on)
     int64_t host_chunk = PC_HOST_CHUNK;   // PC_HOST calls: queries per pipelined chunk (PC_HOST_CHUNK_QUERIES)
     int64_t knn_sort_min = 0;             // pc_knn_batch, PC_QUERY_AUTO: smallest batch that is ordered (PC_KNN_SORT_MIN_BATCH; 0 = by k, knn_host.inl)
     char err[256] = "";
@@ -296,20 +283,16 @@ extern "C" int pc_index_create(pc_index **out, int device, int64_t max_points, v
         TRY(cudaGetDeviceProperties(&prop, device));
         if (prop.major < 10) { rc = pc_fail(nullptr, PC_ECUDA, "pc_index_create: device is sm_%d%d, this library is built for sm_100a only", prop.major, prop.minor); break; }
         ix->sm_count = prop.multiProcessorCount;
-        if (const char *v = getenv("PC_QUERY_KERNEL")) { ix->query_kernel_auto = false; int b_ = atoi(v); ix->query_kernel = (b_ == 1 || b_ == 4 || b_ == 5) ? b_ : 3; }
+        // PC_QUERY_KERNEL: 3 or 4 forces 32- or 64-query packets; any other value is ignored (the batch density decides)
+        if (const char *v = getenv("PC_QUERY_KERNEL")) { int b_ = atoi(v); if (b_ == 3 || b_ == 4) { ix->query_kernel_auto = false; ix->query_kernel = b_; } }
         if (const char *v = getenv("PC_SORT_BITS")) { ix->sort_bits_auto = false; int b_ = atoi(v); ix->sort_bits = b_ <= 0 ? 0 : (b_ <= 16 ? 16 : (b_ <= 24 ? 24 : 32)); }
-        if (const char *v = getenv("PC_HOST_RAMP")) ix->host_ramp = atoi(v) != 0;
         if (const char *v = getenv("PC_ONESWEEP")) ix->onesweep = atoi(v) != 0;
-        if (const char *v = getenv("PC_ORDER_BINS")) { ix->order_bins = atoi(v) != 0; ix->order_bins_all = atoi(v) == 2; }
         if (const char *v = getenv("PC_BIN_BITS")) { int b_ = atoi(v); ix->bin_bits = b_ < 12 ? 0 : (b_ > PC_BIN_MAX_BITS ? PC_BIN_MAX_BITS : b_); }
-        if (const char *v = getenv("PC_GRID")) ix->use_grid = atoi(v) != 0;
-        if (const char *v = getenv("PC_GRID_CELL")) { double c_ = atof(v); if (c_ > 0.0) ix->grid_cell = c_; }
-        if (const char *v = getenv("PC_SORT_ITEMS")) ix->sort_items = atoi(v) == 8 ? 8 : 16;
         if (const char *v = getenv("PC_SHARD_EXACT")) ix->shard_exact = atoi(v) != 0;
         if (const char *v = getenv("PC_TRACE_SLOW_MS")) ix->trace_slow_ms = atof(v);
         if (const char *v = getenv("PC_PACKET_SPLIT")) { double c_ = atof(v); ix->packet_split = c_ > 0.0 ? (float)c_ : 0.f; }
         if (const char *v = getenv("PC_HOST_CHUNK_QUERIES")) { long long b_ = atoll(v); if (b_ >= 1024) ix->host_chunk = b_; }
-        if (const char *v = getenv("PC_COOP_GROUP")) { int b_ = atoi(v); ix->coop_group = (b_ == 32 || b_ == 16 || b_ == 8 || b_ == 4) ? b_ : 0; }
+        if (const char *v = getenv("PC_COOP_GROUP")) { int b_ = atoi(v); ix->coop_group = (b_ == 32 || b_ == 16 || b_ == 8) ? b_ : 0; }
         if (const char *v = getenv("PC_COOP_MAX_BATCH")) { long long b_ = atoll(v); ix->coop_max = ix->coop_max_unbounded = b_ < 0 ? 0 : b_; }
         if (const char *v = getenv("PC_SORT_MIN_BATCH")) { long long b_ = atoll(v); ix->sort_min_radius = ix->sort_min_nearest = b_ < 1 ? 1 : b_; }
         if (const char *v = getenv("PC_KNN_SORT_MIN_BATCH")) { long long b_ = atoll(v); ix->knn_sort_min = b_ < 0 ? 0 : b_; }
@@ -396,7 +379,7 @@ extern "C" void pc_index_destroy(pc_index *ix)
     if (ix->tiny_i) cudaFreeHost(ix->tiny_i);
     cudaFree(ix->d_xyz); cudaFree(ix->d_bbox); cudaFree(ix->keys_a); cudaFree(ix->keys_b);
     cudaFree(ix->vals_a); cudaFree(ix->vals_b); cudaFree(ix->tile_hist); cudaFree(ix->digit_total);
-    cudaFree(ix->tree); cudaFree(ix->scratch); cudaFree(ix->range_long); cudaFree(ix->grid_cell_start); cudaFree(ix->grid_points); cudaFree(ix->hilbert_lut);
+    cudaFree(ix->tree); cudaFree(ix->scratch); cudaFree(ix->range_long); cudaFree(ix->hilbert_lut);
     if (ix->ev_b0) cudaEventDestroy(ix->ev_b0);
     if (ix->ev_b1) cudaEventDestroy(ix->ev_b1);
     if (ix->ev_ready) cudaEventDestroy(ix->ev_ready);
@@ -547,43 +530,6 @@ extern "C" int pc_index_build(pc_index *ix, const float *xyz, int64_t n, int64_t
     }
     PC_CUDA(ix, cudaMemcpyAsync(ix->h_bbox, ix->d_bbox, 6 * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
     PC_CUDA(ix, cudaEventRecord(ix->ev_b1, st));
-    ix->grid_ready = false;
-    if (ix->use_grid) {
-        // experiment: the voxel grid over the same cloud (its build is NOT part of the timed index build above; it needs the
-        // bounding box on the host, hence the sync)
-        PC_CUDA(ix, cudaStreamSynchronize(st));
-        pc_grid G;
-        double ext[3], vol = 1.0, emax = 0.0;
-        for (int a = 0; a < 3; a++) {
-            G.lo[a] = pc_ordered_to_float(ix->h_bbox[a]);
-            ext[a] = (double)pc_ordered_to_float(ix->h_bbox[3 + a]) - (double)G.lo[a];
-            emax = ext[a] > emax ? ext[a] : emax;
-        }
-        double h = ix->grid_cell;
-        for (;;) {                                   // at most 2^24 cells
-            vol = 1.0;
-            for (int a = 0; a < 3; a++) vol *= floor(ext[a] / h) + 1.0;
-            if (vol <= 16777216.0) break;
-            h *= 1.26;
-        }
-        G.h = (float)h; G.inv_h = 1.0f / G.h; G.eps = (float)(emax + h) * 9.6e-7f;        // 8 ulp of the largest coordinate offset
-        int64_t cells = 1;
-        for (int a = 0; a < 3; a++) { G.n[a] = (int)floor(ext[a] / h) + 1; cells *= G.n[a]; }
-        int rcg;
-        if ((rcg = pc_grow(ix, &ix->grid_cell_start, &ix->grid_cells_cap, cells + 2)) != PC_OK) return rcg;
-        if ((rcg = pc_grow(ix, &ix->grid_points, &ix->grid_points_cap, n)) != PC_OK) return rcg;
-        G.cell_start = ix->grid_cell_start; G.points = ix->grid_points;
-        if (ix->key_bytes != 4 || n >= OS_MAX_N) return pc_fail(ix, PC_ENOTIMPL, "PC_GRID: clouds up to 4 Mi points");
-        pc_grid_key_kernel<<<(int)((n + 255) / 256), 256, 0, st>>>(src, n, stride, G, (uint32_t *)ix->keys_a, ix->vals_a);
-        int kb = 8;
-        while (kb < 32 && (cells >> kb) != 0) kb += 8;
-        int w = pc_sort_pairs<uint32_t, 8>(ix, (uint32_t *)ix->keys_a, ix->vals_a, (uint32_t *)ix->keys_b, ix->vals_b, n, 0, kb, ix->tile_hist, ix->digit_total, st);
-        pc_grid_cells_kernel<<<(int)((cells + 1 + 255) / 256), 256, 0, st>>>((const uint32_t *)(w ? ix->keys_b : ix->keys_a), n, cells, ix->grid_cell_start);
-        pc_grid_gather_kernel<<<(int)((n + 255) / 256), 256, 0, st>>>(src, stride, w ? ix->vals_b : ix->vals_a, n, ix->grid_points);
-        PC_CHECK_LAUNCH(ix);
-        ix->grid = G;
-        ix->grid_ready = true;
-    }
     PC_CUDA(ix, cudaEventRecord(ix->ev_ready, st));
     ix->n = n; ix->n_nodes = n_nodes; ix->build_timed = true; ix->bbox_from_bcast = false;
     ix->root = n_nodes > 0 ? 0u : PC_REF_LEAF; ix->root_count = n_nodes > 0 ? 0u : (uint32_t)n;
@@ -702,7 +648,7 @@ static int pc_sort_queries(pc_index *ix, pc_lane &L, const pc_qargs &A, const fl
     const bool prof = ix->profile && &L == &ix->lane[0];
     // (bounded radius batches only: unbounded nearest batches measured 5 % slower end to end on the binned order -- their
     // search is 11 % slower on it, profiles/r2_order_bins_sweep.txt -- and keep the radix sort)
-    if (ix->order_bins && bits == 24 && m < ((int64_t)1 << 32) - 1 && (ix->order_bins_all || (A.kind == PC_Q_RADIUS && A.R.bounded))) {
+    if (bits == 24 && m < ((int64_t)1 << 32) - 1 && A.kind == PC_Q_RADIUS && A.R.bounded) {
         // cell binning (query_kernels.cuh): counting sort by the 21-bit Hilbert cell, the queries themselves gathered into
         // cell order.  Taken whenever the density test would have picked the 24-bit radix sort.
         // number of cells: about half the batch size (a handful of queries per occupied cell, like the 24-bit radix order),
@@ -714,14 +660,8 @@ static int pc_sort_queries(pc_index *ix, pc_lane &L, const pc_qargs &A, const fl
         if (rcb != PC_OK) return rcb;
         if ((rcb = pc_grow(ix, &L.ordered, &L.ordered_cap, m)) != PC_OK) return rcb;
         if (ix->key_ctas_per_sm == 0) {
-            int a = 0, b = 0;
-            int c = 0, d = 0;
-            PC_CUDA(ix, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&a, pc_bin_count_kernel<PC_KIND_RADIUS, false>, 256, 0));
-            PC_CUDA(ix, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, pc_bin_count_kernel<PC_KIND_NEAREST, false>, 256, 0));
-            PC_CUDA(ix, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&c, pc_bin_count_kernel<PC_KIND_RADIUS, true>, 256, 0));
-            PC_CUDA(ix, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&d, pc_bin_count_kernel<PC_KIND_NEAREST, true>, 256, 0));
-            ix->key_ctas_per_sm = a < b ? a : b;
-            ix->key_ctas_per_sm_shard = c < d ? c : d;
+            PC_CUDA(ix, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ix->key_ctas_per_sm, pc_bin_count_kernel<false>, 256, 0));
+            PC_CUDA(ix, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ix->key_ctas_per_sm_shard, pc_bin_count_kernel<true>, 256, 0));
             if (ix->key_ctas_per_sm_shard < 1) ix->key_ctas_per_sm_shard = 1;
             if (ix->key_ctas_per_sm < 1) ix->key_ctas_per_sm = 1;
         }
@@ -733,9 +673,8 @@ static int pc_sort_queries(pc_index *ix, pc_lane &L, const pc_qargs &A, const fl
         const int n_tiles = (int)(n_bins / PC_BIN_SCAN_TILE);
         PC_CUDA(ix, cudaMemsetAsync(L.bins, 0, (size_t)n_bins * sizeof(uint32_t), L.os));
         if (prof) PC_CUDA(ix, cudaEventRecord(L.ta, L.os));
-#define PC_BIN_COUNT(K, S) pc_bin_count_kernel<K, S><<<grid, 256, 0, L.os>>>(d_q, m, qstride, ix->d_bbox, A.R, d_idx, d_f, L.keys_a, L.bins, bin_bits, ix->shard_rank, ix->shard_n, ix->hilbert_lut)
-        if (A.kind == PC_Q_RADIUS) { if (sharded) PC_BIN_COUNT(PC_KIND_RADIUS, true); else PC_BIN_COUNT(PC_KIND_RADIUS, false); }
-        else { if (sharded) PC_BIN_COUNT(PC_KIND_NEAREST, true); else PC_BIN_COUNT(PC_KIND_NEAREST, false); }
+#define PC_BIN_COUNT(S) pc_bin_count_kernel<S><<<grid, 256, 0, L.os>>>(d_q, m, qstride, ix->d_bbox, A.R, d_idx, d_f, L.keys_a, L.bins, bin_bits, ix->shard_rank, ix->shard_n, ix->hilbert_lut)
+        if (sharded) PC_BIN_COUNT(true); else PC_BIN_COUNT(false);
 #undef PC_BIN_COUNT
         if (prof) PC_CUDA(ix, cudaEventRecord(L.tb, L.os));
         pc_bin_scan_tiles<<<n_tiles, 256, 0, L.os>>>(L.bins, tile_sum);
@@ -770,7 +709,7 @@ static int pc_sort_queries(pc_index *ix, pc_lane &L, const pc_qargs &A, const fl
     const int64_t key_ctas = (m + 256 * PC_KEY_ITEMS - 1) / (256 * PC_KEY_ITEMS);
     const int64_t key_wave = (int64_t)ix->sm_count * (sharded ? ix->sortkey_ctas_per_sm_shard : ix->sortkey_ctas_per_sm);
     const int grid = (int)(key_ctas < key_wave ? key_ctas : key_wave);
-    const int items = ix->sort_items;
+    constexpr int items = 16;          // keys per thread of the ordering sort
     const bool fused_hist = ix->onesweep && m < OS_MAX_N;
     uint32_t *gh = fused_hist ? os_ghist(L.tile_hist) : nullptr;
     if (fused_hist) {
@@ -798,8 +737,7 @@ static int pc_sort_queries(pc_index *ix, pc_lane &L, const pc_qargs &A, const fl
         }
     }
     // only the L.counter[1] compacted entries (device-side count <= m; n_sort bounds it on the host) are sorted
-    int which = items == 8 ? pc_sort_pairs<uint32_t, 8>(ix, L.keys_a, L.vals_a, L.keys_b, L.vals_b, n_sort, 0, bits, L.tile_hist, L.digit_total, L.os, L.counter + 1, fused_hist)
-                           : pc_sort_pairs<uint32_t, 16>(ix, L.keys_a, L.vals_a, L.keys_b, L.vals_b, n_sort, 0, bits, L.tile_hist, L.digit_total, L.os, L.counter + 1, fused_hist);
+    int which = pc_sort_pairs<uint32_t, items>(ix, L.keys_a, L.vals_a, L.keys_b, L.vals_b, n_sort, 0, bits, L.tile_hist, L.digit_total, L.os, L.counter + 1, fused_hist);
     PC_CHECK_LAUNCH(ix);
     *perm = which ? L.vals_b : L.vals_a;
     return PC_OK;
@@ -835,7 +773,6 @@ static void pc_launch_coop(const pc_index *ix, const pc_qargs &A, const pc_tree 
     if (g == 0) g = m <= ix->coop_g32_max ? 32 : (m <= ix->coop_g16_max ? 16 : 8);
     if (g == 32) pc_launch_coop_g<32>(A, T, d_q, m, qstride, d_idx, d_f, st);
     else if (g == 16) pc_launch_coop_g<16>(A, T, d_q, m, qstride, d_idx, d_f, st);
-    else if (g == 4) pc_launch_coop_g<4>(A, T, d_q, m, qstride, d_idx, d_f, st);
     else pc_launch_coop_g<8>(A, T, d_q, m, qstride, d_idx, d_f, st);
 }
 
@@ -874,7 +811,7 @@ static int pc_run_batch(pc_index *ix, pc_lane &L, const pc_qargs &A, const float
     pc_tree T = pc_tree_of(ix);
     // dense batches (>= 3 queries per cell of 1/256 of the cloud's extent): 64-query packets, two queries per lane
     // (profiles/r1_sweep5*: +10 % radius, +18 % nearest at 10 M queries; -3 % at 2 M, hence the threshold)
-    const bool two_per_lane = ix->query_kernel == 4 || (ix->query_kernel == 3 && ix->query_kernel_auto && L.per_cell >= 3.0);
+    const bool two_per_lane = ix->query_kernel == 4 || (ix->query_kernel_auto && L.per_cell >= 3.0);
     const bool is_ordered = perm || ordered;
     const int64_t ml = is_ordered ? m_launch : m;        // entries the search launch has to cover
     // unbounded packet walks are shared by queries within a few packet extents of each other only (pc_query_packet_kernel):
@@ -888,24 +825,13 @@ static int pc_run_batch(pc_index *ix, pc_lane &L, const pc_qargs &A, const float
         RN.defer_list = L.keys_a;               // the ordering pass is done with its key buffer; one entry per packet at most
         if (!(RN.packet_split > 0.f) || !is_ordered) RN.packet_split = 0.f;
     }
-    bool packet_walk = false;           // pc_query_packet_kernel ran: it may have put packets aside for the deferred kernel
     if (ml == 0) {
         // pc_batch_shard: nothing of this batch belongs to this rank
-    } else if (ix->grid_ready && is_ordered && A.kind == PC_Q_RADIUS && A.R.bounded) {
-        // experiment (PC_GRID=1): ring search over the voxel grid instead of the tree walk
-        const int grid = (int)((ml + PC_QUERY_THREADS - 1) / PC_QUERY_THREADS);
-        pc_radius_grid_kernel<<<grid, PC_QUERY_THREADS, 0, L.stream>>>(ix->grid, A.R, d_q, m, qstride, perm, ordered, m_eff, d_idx, d_f);
-    } else if (ix->query_kernel >= 3 && is_ordered) {
+    } else if (is_ordered) {
         // curve-ordered batch: one warp walks the tree once for its 32 or 64 neighbouring queries
-        const int per_cta = (ix->query_kernel == 5 ? 4 : (two_per_lane ? 2 : 1)) * PC_QUERY_THREADS;
+        const int per_cta = (two_per_lane ? 2 : 1) * PC_QUERY_THREADS;
         const int grid = (int)((ml + per_cta - 1) / per_cta);
-        packet_walk = true;
-        if (ix->query_kernel == 5) {           // experiment: 128-query packets, four queries per lane
-            if (A.kind == PC_Q_NEAREST)
-                pc_query_packet_kernel<PC_KIND_NEAREST, 4><<<grid, PC_QUERY_THREADS, 0, L.stream>>>(T, RN, d_q, m, qstride, perm, ordered, m_eff, d_idx, d_f);
-            else
-                pc_query_packet_kernel<PC_KIND_RADIUS, 4><<<grid, PC_QUERY_THREADS, 0, L.stream>>>(T, RN, d_q, m, qstride, perm, ordered, m_eff, d_idx, d_f);
-        } else if (two_per_lane) {
+        if (two_per_lane) {
             if (A.kind == PC_Q_NEAREST)
                 pc_query_packet_kernel<PC_KIND_NEAREST, 2><<<grid, PC_QUERY_THREADS, 0, L.stream>>>(T, RN, d_q, m, qstride, perm, ordered, m_eff, d_idx, d_f);
             else
@@ -914,21 +840,21 @@ static int pc_run_batch(pc_index *ix, pc_lane &L, const pc_qargs &A, const float
             pc_query_packet_kernel<PC_KIND_NEAREST, 1><<<grid, PC_QUERY_THREADS, 0, L.stream>>>(T, RN, d_q, m, qstride, perm, ordered, m_eff, d_idx, d_f);
         else
             pc_query_packet_kernel<PC_KIND_RADIUS, 1><<<grid, PC_QUERY_THREADS, 0, L.stream>>>(T, RN, d_q, m, qstride, perm, ordered, m_eff, d_idx, d_f);
-    } else if (ix->query_kernel >= 3 && !is_ordered && m <= ((A.kind == PC_Q_NEAREST || !A.R.bounded) ? ix->coop_max_unbounded : ix->coop_max)) {
+    } else if (m <= ((A.kind == PC_Q_NEAREST || !A.R.bounded) ? ix->coop_max_unbounded : ix->coop_max)) {
         // small unordered batch: one warp per query (a thread-per-query search is a chain of dependent loads)
         pc_launch_coop(ix, A, T, d_q, m, qstride, d_idx, d_f, L.stream);
     } else {
-        const int grid = (int)((ml + PC_QUERY_THREADS - 1) / PC_QUERY_THREADS);
+        const int grid = (int)((m + PC_QUERY_THREADS - 1) / PC_QUERY_THREADS);
         if (A.kind == PC_Q_NEAREST)
-            pc_query_simple_kernel<PC_KIND_NEAREST><<<grid, PC_QUERY_THREADS, 0, L.stream>>>(T, A.R, d_q, m, qstride, perm, ordered, m_eff, d_idx, d_f);
+            pc_query_simple_kernel<PC_KIND_NEAREST><<<grid, PC_QUERY_THREADS, 0, L.stream>>>(T, A.R, d_q, m, qstride, d_idx, d_f);
         else
-            pc_query_simple_kernel<PC_KIND_RADIUS><<<grid, PC_QUERY_THREADS, 0, L.stream>>>(T, A.R, d_q, m, qstride, perm, ordered, m_eff, d_idx, d_f);
+            pc_query_simple_kernel<PC_KIND_RADIUS><<<grid, PC_QUERY_THREADS, 0, L.stream>>>(T, A.R, d_q, m, qstride, d_idx, d_f);
     }
     if (ml > 0) ix->launches++;
-    if (packet_walk && RN.packet_split > 0.f) {
+    if (is_ordered && ml > 0 && RN.packet_split > 0.f) {
         // the packets the walk above put aside as incoherent (normally none or a handful: the kernel then costs its launch)
         const int dgrid = ix->sm_count * PC_DEFER_CTAS_PER_SM;
-        const int per_packet = 32 * (ix->query_kernel == 5 ? 4 : (two_per_lane ? 2 : 1));
+        const int per_packet = (two_per_lane ? 2 : 1) * 32;
         if (A.kind == PC_Q_NEAREST) pc_query_deferred_kernel<PC_KIND_NEAREST><<<dgrid, PC_QUERY_THREADS, 0, L.stream>>>(T, RN, d_q, m, qstride, per_packet, perm, ordered, m_eff, d_idx, d_f);
         else pc_query_deferred_kernel<PC_KIND_RADIUS><<<dgrid, PC_QUERY_THREADS, 0, L.stream>>>(T, RN, d_q, m, qstride, per_packet, perm, ordered, m_eff, d_idx, d_f);
         ix->launches++;
@@ -1019,16 +945,8 @@ static int pc_tiny_host_batch(pc_index *ix, const pc_qargs &A, const float *q, i
     pc_tree T = pc_tree_of(ix);
     int32_t *d_i = out_idx ? ix->tiny_i_dev : nullptr;
     float *d_f = out_f ? ix->tiny_f_dev : nullptr;
-    if (ix->query_kernel == 1) {             // PC_QUERY_KERNEL=1: one thread per query, for comparison
-        const int grid = (int)((m + PC_QUERY_THREADS - 1) / PC_QUERY_THREADS);
-        if (A.kind == PC_Q_NEAREST)
-            pc_query_simple_kernel<PC_KIND_NEAREST><<<grid, PC_QUERY_THREADS, 0, ix->stream>>>(T, A.R, ix->tiny_q_dev, m, qs, nullptr, nullptr, nullptr, d_i, d_f);
-        else
-            pc_query_simple_kernel<PC_KIND_RADIUS><<<grid, PC_QUERY_THREADS, 0, ix->stream>>>(T, A.R, ix->tiny_q_dev, m, qs, nullptr, nullptr, nullptr, d_i, d_f);
-    } else {
-        // one warp per query: the search of a single query is a chain of dependent loads, the warp shortens it
-        pc_launch_coop(ix, A, T, ix->tiny_q_dev, m, qs, d_i, d_f, ix->stream);
-    }
+    // one warp per query: the search of a single query is a chain of dependent loads, the warp shortens it
+    pc_launch_coop(ix, A, T, ix->tiny_q_dev, m, qs, d_i, d_f, ix->stream);
     ix->launches++;
     PC_CHECK_LAUNCH(ix);
     PC_CUDA(ix, cudaStreamSynchronize(ix->stream));
@@ -1086,16 +1004,9 @@ static int pc_query_dispatch(pc_index *ix, const pc_qargs &A, const float *q, in
     }
     const int64_t chunk = ix->host_chunk;
     int li = 0;
-    // ramp: the first chunks are smaller (1/4, 1/2 of the chunk size) so that the first kernel starts after a short copy
-    // instead of a full one -- the call is bound by the chain copy(first chunk) -> kernels of all chunks -> copy-back(last)
-    int64_t c = chunk;
-    int ramp = (ix->host_ramp && m > 2 * chunk) ? 2 : 0;
-    for (int64_t off = 0; off < m; off += c, li = (li + 1) % PC_PIPE_LANES) {
+    for (int64_t off = 0; off < m; off += chunk, li = (li + 1) % PC_PIPE_LANES) {
         pc_lane &L = ix->lane[li];
-        c = chunk >> ramp;
-        if (ramp > 0) ramp--;
-        if (c < PC_SORT_MIN_BATCH) c = chunk;
-        if (m - off < c) c = m - off;
+        const int64_t c = m - off < chunk ? m - off : chunk;
         int rc;
         // a multi-chunk call sizes the lane buffers for full chunks at once; a small call allocates only what it needs
         const int64_t floor_q = m > chunk ? chunk : 0;

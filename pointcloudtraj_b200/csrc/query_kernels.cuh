@@ -28,10 +28,6 @@
                                     // arithmetic the kernel waits on record loads more than on issue slots: 10 CTAs 0.77 ms,
                                     // 9: 0.80, 8: 0.82, 12 (40 registers, the hot loop spills): 1.03 (profiles/r2_variants_ab.txt)
 #endif
-#ifndef PC_PACKET_PREFETCH
-#define PC_PACKET_PREFETCH 0        // 1: when a record arrives, pull the records of its two children towards L1 (measured:
-                                    // +10 % search time -- the extra requests cost more than the latency they hide)
-#endif
 
 struct pc_tree {
     const float4 *__restrict__ rec;      // inner node i -> rec[4i .. 4i+3] = [min0 | max0 | min1 | max1], children in the .w words
@@ -295,24 +291,19 @@ __device__ __forceinline__ void pc_write_result(const pc_radius_dev &R, const pc
 }
 
 // ---- one thread per query -------------------------------------------------------------------------------------------
-// perm (nullable): process query perm[t] in slot t (curve-ordered batches); results go to the original slot.
-// ordered (nullable, instead of perm): slot t holds the query itself, (x, y, z, original slot) -- the cell-binned batch.
-// m_eff (nullable): device-side number of leading entries of perm that need a search (the rest were answered by the
-// ordering pass).
+// Unordered batches too large for the lane groups and too small for the ordering pass: query t in slot t.
 template <int KIND>
 __global__ void __launch_bounds__(PC_QUERY_THREADS)
 pc_query_simple_kernel(pc_tree T, pc_radius_dev R, const float *__restrict__ q, int64_t m, int qstride,
-                       const uint32_t *__restrict__ perm, const float4 *__restrict__ ordered, const unsigned long long *__restrict__ m_eff,
                        int32_t *__restrict__ out_idx, float *__restrict__ out_f)
 {
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= m || (m_eff && t >= (int64_t)*m_eff)) return;
-    uint32_t k;
-    float qx, qy, qz;
-    if (ordered) { const float4 v = __ldg(ordered + t); qx = v.x; qy = v.y; qz = v.z; k = __float_as_uint(v.w); }
-    else { k = perm ? perm[t] : (uint32_t)t; const float *qq = q + (size_t)k * qstride; qx = qq[0]; qy = qq[1]; qz = qq[2]; }
+    if (t >= m) return;
+    const uint32_t k = (uint32_t)t;
+    const float *qq = q + (size_t)k * qstride;
+    const float qx = qq[0], qy = qq[1], qz = qq[2];
     bool search = T.n_points > 0;
-    if (KIND == PC_KIND_RADIUS && search && !m_eff && pc_radius_early_out((double)qx, (double)qy, (double)qz, R)) search = false;
+    if (KIND == PC_KIND_RADIUS && search && pc_radius_early_out((double)qx, (double)qy, (double)qz, R)) search = false;
     if (!search) { pc_write_trivial<KIND>(R, k, out_idx, out_f); return; }
     pc_best b; b.d2 = INFINITY; b.idx = -1; b.thr = (KIND == PC_KIND_RADIUS) ? R.bound_thr : FLT_MAX;
     pc_nearest_traverse(T, qx, qy, qz, b);
@@ -355,16 +346,6 @@ __device__ __forceinline__ void pc_packet_traverse(const pc_tree &T, const float
     uint32_t ref = T.root;
     for (;;) {
         const pc_rec rec = pc_load_rec(T.rec + 4ull * ref);
-#if PC_PACKET_PREFETCH
-        {   // the next visit is one of the two children (or a stack entry): start their records' trip from L2 now, while the
-            // box tests and votes below run (a leaf reference fetches a line of the points instead, also the next access)
-            const uint32_t c0 = pc_rec_ref(rec, 0), c1 = pc_rec_ref(rec, 1);
-            const float4 *a0 = (c0 & PC_REF_LEAF) ? T.points + (c0 & ~PC_REF_LEAF) : T.rec + 4ull * c0;
-            const float4 *a1 = (c1 & PC_REF_LEAF) ? T.points + (c1 & ~PC_REF_LEAF) : T.rec + 4ull * c1;
-            asm volatile("prefetch.global.L1 [%0];" ::"l"(a0));
-            asm volatile("prefetch.global.L1 [%0];" ::"l"(a1));
-        }
-#endif
         float d0[NQ], d1[NQ];
         bool want0 = false, want1 = false;
         if constexpr (NQ == 2) {
@@ -419,7 +400,7 @@ __device__ __forceinline__ void pc_packet_traverse(const pc_tree &T, const float
 }
 
 template <int KIND, int NQ>
-__global__ void __launch_bounds__(PC_QUERY_THREADS, NQ <= 2 ? PC_PACKET_MIN_CTAS : PC_PACKET_MIN_CTAS / 2)
+__global__ void __launch_bounds__(PC_QUERY_THREADS, PC_PACKET_MIN_CTAS)
 pc_query_packet_kernel(pc_tree T, pc_radius_dev R, const float *__restrict__ q, int64_t m, int qstride,
                        const uint32_t *__restrict__ perm, const float4 *__restrict__ ordered, const unsigned long long *__restrict__ m_eff,
                        int32_t *__restrict__ out_idx, float *__restrict__ out_f)
@@ -952,7 +933,8 @@ pc_hilbert_lut_kernel(uint16_t *__restrict__ lut4, uint16_t *__restrict__ lut5)
     if (i < PC_LUT5_WORDS) lut5[i] = (uint16_t)pc_hilbert_cells_n<5>(i & 31u, (i >> 5) & 31u, (i >> 10) & 31u);
 }
 
-template <int KIND, bool SHARDED>
+// bounded radius batches only (pc_sort_queries): unbounded ones keep the radix sort
+template <bool SHARDED>
 __global__ void __launch_bounds__(256)
 pc_bin_count_kernel(const float *__restrict__ q, int64_t m, int qstride, const uint32_t *__restrict__ bbox,
                     pc_radius_dev R, int32_t *__restrict__ out_idx, float *__restrict__ out_f,
@@ -995,9 +977,9 @@ pc_bin_count_kernel(const float *__restrict__ q, int64_t m, int qstride, const u
         for (int j = 0; j < PC_KEY_ITEMS; j++) {
             if (!have[j]) continue;
             bool search = true;
-            if (KIND == PC_KIND_RADIUS && pc_radius_early_out((double)x[j], (double)y[j], (double)z[j], R)) {
+            if (pc_radius_early_out((double)x[j], (double)y[j], (double)z[j], R)) {
                 search = false;
-                pc_write_trivial<KIND>(R, slot[j], out_idx, out_f);
+                pc_write_trivial<PC_KIND_RADIUS>(R, slot[j], out_idx, out_f);
             }
             uint32_t key = PC_BIN_SKIP;
             if (search) {

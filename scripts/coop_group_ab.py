@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""Mid-size unordered batches (C2's own 50 k RRT* samples and around): one thread per query against a group of 8 / 4 lanes per
+"""Mid-size unordered batches (C2's own 50 k RRT* samples and around): one thread per query against a group of 8 lanes per
 query (pc_query_coop_kernel).  Device buffers, CUDA events around the call, median of 8; results compared."""
 import ctypes as C, os, sys
 import numpy as np
@@ -15,7 +15,7 @@ t_pts = torch.from_numpy(pts).to(dev)
 P = PcRadiusParams.make(0.25, 1.5, 30.0, (0.0, 0.0, 2.0))
 handles = {}
 for name, env in (("thread", {"PC_COOP_MAX_BATCH": "0"}), ("g8", {"PC_COOP_MAX_BATCH": "100000000", "PC_COOP_GROUP": "8"}),
-                  ("g4", {"PC_COOP_MAX_BATCH": "100000000", "PC_COOP_GROUP": "4"}), ("auto", {})):
+                  ("auto", {})):
     for k in ("PC_COOP_MAX_BATCH", "PC_COOP_GROUP"):
         os.environ.pop(k, None)
     os.environ.update(env)

@@ -20,9 +20,8 @@ qp, rp = q.numpy(), r.numpy()
 P = PcRadiusParams.make(0.25, 1.5, 30.0, (0.0, 0.0, 2.0))
 print(f"# e2e pc_radius_batch PC_HOST, {M} queries, pinned buffers")
 ref = None
-for chunk, ramp in [(c, rmp) for c in (1 << 19, 1 << 20, 1 << 21, 3 << 20, 1 << 22) for rmp in (0, 1)]:
+for chunk in (1 << 19, 1 << 20, 1 << 21, 3 << 20, 1 << 22):
     os.environ["PC_HOST_CHUNK_QUERIES"] = str(chunk)
-    os.environ["PC_HOST_RAMP"] = str(ramp)
     ix = PointCloudIndex(max_points=len(pts))
     ix.build(pts)
     L = ix._L
@@ -36,5 +35,5 @@ for chunk, ramp in [(c, rmp) for c in (1 << 19, 1 << 20, 1 << 21, 3 << 20, 1 << 
     dt = (time.perf_counter() - t0) / n
     if ref is None:
         ref = rp.copy()
-    print(f"chunk {chunk:9d} ramp {ramp}: {dt * 1e3:7.3f} ms/step  {M / dt / 1e9:6.3f} Gq/s  same={bool((rp == ref).all())}", flush=True)
+    print(f"chunk {chunk:9d}: {dt * 1e3:7.3f} ms/step  {M / dt / 1e9:6.3f} Gq/s  same={bool((rp == ref).all())}", flush=True)
     ix.close()

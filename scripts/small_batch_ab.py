@@ -12,15 +12,14 @@ stream = torch.cuda.current_stream().cuda_stream
 pts, half = synth.forest_cloud(1_000_000, seed=1, variant="J", return_half=True)
 t_pts = torch.from_numpy(pts).to(dev)
 P = PcRadiusParams.make(0.25, 1.5, 30.0, (0.0, 0.0, 2.0))
-print(f"{'m':>8s} {'kernel':>6s} {'flags':>9s} {'G':>3s} {'ms':>8s}")
+print(f"{'m':>8s} {'flags':>9s} {'G':>3s} {'ms':>8s}")
 for m in (1000, 4000, 8000, 16000, 32000, 50000, 100000, 200000):
     q = torch.from_numpy(synth.rrt_queries(m, half, seed=5)).to(dev)
     out = torch.empty(m, dtype=torch.float32, device=dev)
-    # kernel 1 = one thread per query; 3 unsorted = one warp per query (pc_query_coop_kernel); 3 sorted = ordered warp packets
-    for kern in (1, 3):
-        for flags, fname in ((2, "unsorted"), (4, "sorted")):
-          for group in ((32, 16, 8) if (kern == 3 and flags == 2) else (0,)):
-            os.environ["PC_QUERY_KERNEL"] = str(kern)
+    # unsorted = a group of G lanes per query (pc_query_coop_kernel); sorted = ordered 32-query warp packets
+    for flags, fname in ((2, "unsorted"), (4, "sorted")):
+        for group in ((32, 16, 8) if flags == 2 else (0,)):
+            os.environ["PC_QUERY_KERNEL"] = "3"
             os.environ["PC_COOP_MAX_BATCH"] = str(1 << 30)
             os.environ["PC_COOP_GROUP"] = str(group)
             ix = PointCloudIndex(max_points=len(pts), stream=stream)
@@ -32,5 +31,5 @@ for m in (1000, 4000, 8000, 16000, 32000, 50000, 100000, 200000):
                 e0.record()
                 L.pc_radius_batch(ix._h, C.c_void_p(q.data_ptr()), m, 3, 1, flags, C.byref(P), C.c_void_p(out.data_ptr()), None)
                 e1.record(); torch.cuda.synchronize(); ts.append(e0.elapsed_time(e1))
-            print(f"{m:8d} {kern:6d} {fname:>9s} {group:3d} {np.median(ts[3:]):8.4f}", flush=True)
+            print(f"{m:8d} {fname:>9s} {group:3d} {np.median(ts[3:]):8.4f}", flush=True)
             ix.close()

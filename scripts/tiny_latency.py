@@ -1,6 +1,6 @@
 #!/usr/bin/env python
-"""Latency of small blocking PC_HOST radius calls (run on the GPU box): the mapped-memory path with one warp per query (default), the
-same with one thread per query (PC_QUERY_KERNEL=1), and staged copies (PC_TINY_BATCH_QUERIES=0).  m = 1 is what the unmodified planner loop issues once per RRT* iteration.
+"""Latency of small blocking PC_HOST radius calls (run on the GPU box): the mapped-memory path with one warp per query (default) and
+staged copies (PC_TINY_BATCH_QUERIES=0).  m = 1 is what the unmodified planner loop issues once per RRT* iteration.
 
     python scripts/tiny_latency.py > gpurun_out/tiny_latency.txt
 """
@@ -24,12 +24,11 @@ def main():
     P = PcRadiusParams.make(0.25, 1.5, 30.0, (0.0, 0.0, 2.0))
     out = np.empty(len(q), np.float32)
     print("# blocking pc_radius_batch(PC_HOST, m) on a 200k-point map, microseconds per call (median of 5 x 400 calls, ctypes included)")
-    print(f"{'m':>6s} {'warp/query':>11s} {'thread/query':>13s} {'staged':>9s}")
+    print(f"{'m':>6s} {'warp/query':>11s} {'staged':>9s}")
     handles = {}
-    names = ("warp/query", "thread/query", "staged")
-    for name, env in zip(names, ({}, {"PC_QUERY_KERNEL": "1"}, {"PC_TINY_BATCH_QUERIES": "0"})):
-        for k in ("PC_TINY_BATCH_QUERIES", "PC_QUERY_KERNEL"):
-            os.environ.pop(k, None)
+    names = ("warp/query", "staged")
+    for name, env in zip(names, ({}, {"PC_TINY_BATCH_QUERIES": "0"})):
+        os.environ.pop("PC_TINY_BATCH_QUERIES", None)
         os.environ.update(env)
         h = C.c_void_p()
         assert L.pc_index_create(C.byref(h), 0, len(pts), None) == 0
@@ -48,7 +47,7 @@ def main():
                 meds.append((time.perf_counter() - t0) / 400 * 1e6)
                 assert rc == 0
             row.append(float(np.median(meds[1:])))
-        print(f"{m:6d} {row[0]:11.1f} {row[1]:13.1f} {row[2]:9.1f}", flush=True)
+        print(f"{m:6d} {row[0]:11.1f} {row[1]:9.1f}", flush=True)
     for h in handles.values():
         L.pc_index_destroy(h)
 

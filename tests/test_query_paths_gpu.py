@@ -46,19 +46,23 @@ MID_SIZES = [1, 31, 32, 33, 63, 64, 65, 4096, 4097, 6144, 6145, 8192, 8193, 1228
 
 # one handle per switch; each is read once, at pc_index_create
 SWITCHES = [
-    {"PC_QUERY_KERNEL": 1}, {"PC_QUERY_KERNEL": 4}, {"PC_QUERY_KERNEL": 5},
-    {"PC_SORT_BITS": 0}, {"PC_SORT_BITS": 16}, {"PC_SORT_BITS": 32},
-    {"PC_ORDER_BINS": 0}, {"PC_ORDER_BINS": 2},
+    # 32-query packets on the dense batches too, 64-query packets on the sparse ones
+    {"PC_QUERY_KERNEL": 3}, {"PC_QUERY_KERNEL": 4},
+    # 24 bits: cell binning (bounded radius) and the 24-bit radix order on batches dense enough for 32 bits
+    {"PC_SORT_BITS": 0}, {"PC_SORT_BITS": 16}, {"PC_SORT_BITS": 24}, {"PC_SORT_BITS": 32},
     {"PC_BIN_BITS": 12}, {"PC_BIN_BITS": 24},
-    {"PC_ONESWEEP": 0, "PC_SORT_ITEMS": 8},
+    {"PC_ONESWEEP": 0},
     {"PC_PACKET_SPLIT": 0}, {"PC_PACKET_SPLIT": 0.5},
-    {"PC_COOP_GROUP": 4},
+    # one lane-group width for every small unordered batch
+    {"PC_COOP_GROUP": 32}, {"PC_COOP_GROUP": 16}, {"PC_COOP_GROUP": 8},
     {"PC_COOP_MAX_BATCH": 0}, {"PC_COOP_MAX_BATCH": 1 << 30},
     {"PC_SORT_MIN_BATCH": 1},
-    {"PC_HOST_CHUNK_QUERIES": 1024}, {"PC_HOST_CHUNK_QUERIES": 1024, "PC_HOST_RAMP": 1},
-    # the ramp halves chunks only down to PC_SORT_MIN_BATCH (2^17): 2^19-query chunks ramp as 2^17, 2^18, 2^19, ...
-    {"PC_HOST_CHUNK_QUERIES": 1 << 19, "PC_HOST_RAMP": 1},
-    {"PC_GRID": 1},
+    # small blocking PC_HOST calls through the staged pipeline: always, and above 64 queries (the mid sizes straddle 64)
+    {"PC_TINY_BATCH_QUERIES": 0}, {"PC_TINY_BATCH_QUERIES": 64},
+    {"PC_HOST_CHUNK_QUERIES": 1024},
+    # the 700 k batch in a 524 288-query chunk and a 175 712-query tail: the first chunk is above PC_SORT_MIN_NEAREST and below
+    # PC_SORT_MIN_RADIUS, so the chunks of one call take different paths
+    {"PC_HOST_CHUNK_QUERIES": 1 << 19},
 ]
 
 
@@ -84,8 +88,8 @@ def build(h, pts):
 
 
 def per_cell(pts, m):
-    """Restatement of the density estimate of pc_sort_queries (pc_index.cu:685-698): queries per cell of 1/256 of the cloud's
-    largest extent, with thin axes counted as one cell.  pc_run_batch (:875) takes 64-query packets from 3, and the ordering
+    """Restatement of the density estimate of pc_sort_queries (pc_index.cu:633-647): queries per cell of 1/256 of the cloud's
+    largest extent, with thin axes counted as one cell.  pc_run_batch (:814) takes 64-query packets from 3, and the ordering
     pass the 32-bit order above 16."""
     ext = (pts.max(0) - pts.min(0)).astype(np.float32)
     cell = float(ext.max()) / 256.0
@@ -465,24 +469,6 @@ def test_switch_dense(dense, two_clusters, env):
             for sp in ("host", "device"):
                 got = run(h, two_clusters.q, kind, sp, PC_QUERY_SORTED)
                 assert same(got[0], two_clusters.want(kind)[0]) and same(got[1], two_clusters.want(kind)[1]), (kind, sp)
-    finally:
-        h.close()
-
-
-def test_grid_answers_deferred_packets(two_clusters):
-    """PC_GRID=1 answers ordered bounded radius batches on the voxel grid, but nearest and FULL_NN batches still walk the tree
-    in packets; the packets those put aside must still be answered by the deferred kernel."""
-    ds = two_clusters
-    h = build(make_handle({"PC_GRID": 1}), ds.pts)
-    try:
-        for kind in ("nearest", "full"):
-            got = run(h, ds.q, kind, "device", PC_QUERY_SORTED)
-            assert deferred_packets(h) >= 1
-            assert same(got[0], ds.want(kind)[0]) and same(got[1], ds.want(kind)[1]), kind
-            got = run(h, ds.q, kind, "host", PC_QUERY_SORTED)
-            assert same(got[0], ds.want(kind)[0]) and same(got[1], ds.want(kind)[1]), kind
-        got = run(h, ds.q, "bounded", "device", PC_QUERY_SORTED)
-        assert same(got[0], ds.want("bounded")[0]) and same(got[1], ds.want("bounded")[1])
     finally:
         h.close()
 
