@@ -13,6 +13,8 @@
  *   pc_knn_batch                pcl::search::KdTree nearestKSearch, radiusSearch with max_nn (no counterpart in Utils/kdtree)
  *   pc_knn_large_batch          pcl::search::KdTree nearestKSearch with 32 < k <= 1024
  *   pc_segment_nearest_batch    (no counterpart: the reference samples points along an edge) nearest point to a segment
+ *   pc_sphere_sweep_batch       (no counterpart: the reference checks sampled positions) first contact of a sphere moved
+ *                               along a segment
  *   pc_range_batch              kd_nearest_range3 + kd_res_size/next/item   kdtree.h:92,100-113 (kdtree.c:595-602)
  *   pc_range_sorted_batch       pcl::search::KdTree radiusSearch(q, r, k_indices, k_sqr_distances, max_nn), any max_nn
  *   pc_radius_batch             safeRegionRrtStar::radiusSearch     Planner/src/corridor_finder.cpp:113-133
@@ -70,7 +72,8 @@ extern "C" {
 /* flags for pc_radius_batch / pc_clearance_batch */
 #define PC_RADIUS_BOUNDED   0  /* default: search only within max_radius + search_margin (exact for the radius) */
 #define PC_RADIUS_FULL_NN   1  /* unbounded search: out_idx is the true nearest point even where the radius clamps */
-/* flags for pc_nearest_batch / pc_radius_batch / pc_knn_batch / pc_knn_large_batch / pc_segment_nearest_batch: reorder the batch along a space-filling (Hilbert) curve first (same results) */
+/* flags for pc_nearest_batch / pc_radius_batch / pc_knn_batch / pc_knn_large_batch / pc_segment_nearest_batch /
+ * pc_sphere_sweep_batch: reorder the batch along a space-filling (Hilbert) curve first (same results) */
 #define PC_QUERY_AUTO      0
 #define PC_QUERY_UNSORTED  2
 #define PC_QUERY_SORTED    4
@@ -203,6 +206,26 @@ int  pc_knn_large_batch(pc_index *ix, const float *q_xyz, int64_t m, int64_t q_s
  * a_xyz / b_xyz with m > 0, the ASYNC spaces, unknown flags, a NaN max_range, a pc_batch_shard handle (n_ranks > 1). */
 int  pc_segment_nearest_batch(pc_index *ix, const float *a_xyz, const float *b_xyz, int64_t m, int64_t stride,
                               int space, int flags, double max_range, int32_t *out_idx, float *out_d2);
+
+/* First contact of a sphere of radius `radius` moved from a_i to b_i: the smallest parameter t in [0, 1] at which a cloud
+ * point lies in the sphere, and that point.  Per point p, with A, B, P widened to double, D, W, L2 and s exactly as in
+ * pc_segment_nearest_batch, R2 = radius * radius (pc_range_batch's r2), every operation rounded to nearest, never fused,
+ * sqrt and division IEEE:
+ *   c0 = the reference's expression of P against A  (= (Wx*Wx + Wy*Wy) + Wz*Wz)
+ *   c0 <= R2                                     t(p) = 0
+ *   else if L2 != 0 and s > 0:  h = c0 - R2, disc = s*s - L2*h;
+ *        disc >= 0 and t' = h / (s + sqrt(disc)) <= 1      t(p) = t'
+ *   otherwise, if the reference's expression of P against B <= R2     t(p) = 1
+ *   otherwise                                    p makes no contact.
+ * out_idx[i] is the contacting point with the smallest (t(p), original index); out_t[i] that t rounded once toward -inf to
+ * float32, so that a + out_t * (b - a) never passes the fp64 contact.  t = 0 exactly when pc_range_batch(a, radius) is
+ * non-empty, and out_idx is then that list's first (lowest) index.  No contact, or an empty index: idx -1, t +inf.  A
+ * non-finite endpoint coordinate: idx -1, t NaN.  A polyline of n points is checked with b_xyz = a_xyz + stride and
+ * m = n - 1.  Either output may be NULL.  space: PC_HOST or PC_DEVICE.  flags as pc_segment_nearest_batch (SORTED orders by
+ * the midpoints; same results).  PC_EINVAL: a radius that is negative, NaN or infinite, and every refusal of
+ * pc_segment_nearest_batch (bad stride, NULL a_xyz / b_xyz with m > 0, the ASYNC spaces, unknown flags, pc_batch_shard). */
+int  pc_sphere_sweep_batch(pc_index *ix, const float *a_xyz, const float *b_xyz, int64_t m, int64_t stride,
+                           int space, int flags, double radius, int32_t *out_idx, float *out_t);
 
 /* Arithmetic of the radiusSearch epilogue (pc_radius_batch, pc_clearance_batch) on this handle:
  *   PC_ARITH_FP64 (default)  radius = sqrt(d2) - search_margin in double precision from the kd-tree's fp64 d2 -- the parity

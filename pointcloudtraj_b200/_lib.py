@@ -32,7 +32,7 @@ ABI_SYMBOLS = [
     "pc_comm_unique_id", "pc_comm_init", "pc_comm_destroy", "pc_index_broadcast", "pc_shard_range",
     "pc_launch_count", "pc_profile_enable", "pc_profile_last_batch", "pc_batch_shard", "pc_index_set_radius_arith",
     "pc_profile_last_order_detail", "pc_profile_last_deferred_packets", "pc_sample_batch", "pc_expand_batch",
-    "pc_knn_batch", "pc_range_sorted_batch", "pc_knn_large_batch", "pc_segment_nearest_batch",
+    "pc_knn_batch", "pc_range_sorted_batch", "pc_knn_large_batch", "pc_segment_nearest_batch", "pc_sphere_sweep_batch",
 ]
 
 
@@ -124,6 +124,7 @@ def load():
     L.pc_knn_batch.argtypes = [vp, vp, i64, i64, i32, i32, i32, C.c_double, vp, vp]
     L.pc_knn_large_batch.argtypes = [vp, vp, i64, i64, i32, i32, i32, C.c_double, vp, vp]
     L.pc_segment_nearest_batch.argtypes = [vp, vp, vp, i64, i64, i32, i32, C.c_double, vp, vp]
+    L.pc_sphere_sweep_batch.argtypes = [vp, vp, vp, i64, i64, i32, i32, C.c_double, vp, vp]
     L.pc_radius_batch.argtypes = [vp, vp, i64, i64, i32, i32, C.POINTER(PcRadiusParams), vp, vp]
     L.pc_range_batch.argtypes = [vp, vp, i64, i64, i32, vp, i32, vp, vp, i64]
     L.pc_range_sorted_batch.argtypes = [vp, vp, i64, i64, i32, vp, i32, i64, vp, vp, vp, i64]

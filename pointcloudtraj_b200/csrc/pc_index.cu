@@ -21,6 +21,7 @@
 #include "knn_large_kernels.cuh"
 #include "range_sorted_kernels.cuh"
 #include "segment_kernels.cuh"
+#include "sweep_kernels.cuh"
 #include "clearance_kernels.cuh"
 #include "sampler_kernels.cuh"
 
@@ -1092,6 +1093,7 @@ extern "C" int pc_radius_batch(pc_index *ix, const float *q_xyz, int64_t m, int6
 #include "knn_host.inl"
 #include "knn_large_host.inl"
 #include "segment_host.inl"
+#include "sweep_host.inl"
 #include "clearance_host.inl"
 #include "sampler_host.inl"
 #include "comm_host.inl"

@@ -5,8 +5,9 @@
 //
 //   pc_segment_kernel   one WARP per segment: the frontier walk of pc_knn_warp_search (seeds, then up to 32 frontier nodes a
 //                       step, depth-first close to the frontier's capacity) with the k = 1 list of pc_knn_wlist.  The walk is a
-//                       copy, not an instantiation: the node test and the leaf scan differ, and the existing kNN kernels stay
-//                       byte-identical.
+//                       copy, not an instantiation of the kNN walk: the node test and the leaf scan differ, and the existing kNN
+//                       kernels stay byte-identical.  pc_seg_search is itself a template over the geometry, shared with
+//                       pc_sphere_sweep_kernel (sweep_kernels.cuh).
 //
 // Node test (pc_seg_box): a child is pruned only if no point of its box can have fp64 d2 <= the current best (or the bound).
 // Such a point lies within rho = sqrt(thr) + tau of the segment, where thr >= best (1 + 2^-20) is the kNN walks' fp32
@@ -61,7 +62,8 @@ __device__ __forceinline__ void pc_seg_set_thr(float thr, pc_seg_geo &G)
     G.thr2 = __fmul_ru(G.rho, G.rho);
 }
 
-__device__ __forceinline__ void pc_seg_setup(const float *a, const float *b, pc_seg_geo &G)
+// returns |b - a| rounded up
+__device__ __forceinline__ float pc_seg_setup(const float *a, const float *b, pc_seg_geo &G)
 {
     G.ax = a[0]; G.ay = a[1]; G.az = a[2];
     G.bx = b[0]; G.by = b[1]; G.bz = b[2];
@@ -81,15 +83,18 @@ __device__ __forceinline__ void pc_seg_setup(const float *a, const float *b, pc_
         G.inv_hi[i] = s == e ? INFINITY : __frcp_ru(dlo);
         len2 = __fadd_ru(len2, __fmul_ru(dhi, dhi));
     }
-    G.tau = __fmaf_ru(__fsqrt_ru(len2), PC_SEG_TAU_REL, PC_SEG_TAU_ABS);
+    const float len = __fsqrt_ru(len2);
+    G.tau = __fmaf_ru(len, PC_SEG_TAU_REL, PC_SEG_TAU_ABS);
+    return len;
 }
 
-// Node test of the box [lo, hi]: INFINITY if the slab test proves it farther than rho from the segment, else the squared gap
-// between the box and the segment's AABB, rounded down (a lower bound of the squared distance of any of its points).
-__device__ __forceinline__ float pc_seg_box(float lx, float ly, float lz, float hx, float hy, float hz, const pc_seg_geo &G)
+// The box [lo, hi] against the segment: g2 = the squared gap between the box and the segment's AABB, rounded down (a lower
+// bound of the squared distance of any of its points); [t0, t1] clipped against the box dilated by rho on each axis (entry
+// rounded down, exit rounded up).  t0 > t1: every point of the clipped stretch is more than rho from the box.
+__device__ __forceinline__ void pc_seg_clip(float lx, float ly, float lz, float hx, float hy, float hz, const pc_seg_geo &G,
+                                            float &g2, float &t0, float &t1)
 {
     const float lo[3] = { lx, ly, lz }, hi[3] = { hx, hy, hz };
-    float g2 = 0.f, t0 = 0.f, t1 = 1.f;
 #pragma unroll
     for (int i = 0; i < 3; i++) {
         const float g = fmaxf(fmaxf(__fsub_rd(lo[i], G.hi[i]), __fsub_rd(G.lo[i], hi[i])), 0.f);
@@ -102,13 +107,36 @@ __device__ __forceinline__ float pc_seg_box(float lx, float ly, float lz, float 
         t0 = fmaxf(t0, __fmul_rd(nl, nl >= 0.f ? G.inv_lo[i] : G.inv_hi[i]));
         t1 = fminf(t1, __fmul_ru(nh, nh >= 0.f ? G.inv_hi[i] : G.inv_lo[i]));
     }
+}
+
+// Node test of the box [lo, hi]: INFINITY if the slab test of [0, 1] proves it farther than rho from the segment, else the
+// squared gap g2 of pc_seg_clip.
+__device__ __forceinline__ float pc_seg_box(float lx, float ly, float lz, float hx, float hy, float hz, const pc_seg_geo &G)
+{
+    float g2 = 0.f, t0 = 0.f, t1 = 1.f;
+    pc_seg_clip(lx, ly, lz, hx, hy, hz, G, g2, t0, t1);
     return t0 <= t1 ? g2 : INFINITY;
 }
 
+// the segment's leaf evaluation: the list key d2, and whether the bound keeps it
+__device__ __forceinline__ bool pc_seg_leaf(float px, float py, float pz, const pc_seg_dev &S, const pc_seg_geo &G, double &e)
+{
+    e = pc_seg_exact_d2(px, py, pz, G);
+    return e <= S.r2;
+}
+
+// the limit the frontier's keys are tested against: rho^2 (the gap is a squared distance)
+__device__ __forceinline__ float pc_seg_lim(const pc_seg_geo &G) { return G.thr2; }
+
+// The walk below is shared by pc_segment_kernel (GEO = pc_seg_geo) and pc_sphere_sweep_kernel (GEO = pc_sweep_geo,
+// sweep_kernels.cuh).  GEO supplies, by overload: pc_seg_box (node test: the frontier key, INFINITY when pruned), pc_seg_lim
+// (the key limit), pc_seg_leaf (list key of a point, and whether it counts) and pc_seg_set_thr (refresh after the list's
+// threshold changed).
+
 // scan NL leaves per lane (cnt points each; 0 = none) and offer the survivors to the k = 1 list
-template <int NL>
+template <int NL, class GEO>
 __device__ __forceinline__ void pc_seg_scan(const pc_tree &T, const uint32_t (&ref)[NL], const uint32_t (&cnt)[NL], int lane,
-                                            const pc_seg_dev &S, const pc_knn_dev &K, pc_seg_geo &G, pc_knn_wlist &W)
+                                            const pc_seg_dev &S, const pc_knn_dev &K, GEO &G, pc_knn_wlist &W)
 {
     float4 p[NL * PC_LEAF];
 #pragma unroll
@@ -121,9 +149,8 @@ __device__ __forceinline__ void pc_seg_scan(const pc_tree &T, const uint32_t (&r
         double e = 0.0;
         uint32_t id = 0u;
         if (have) {
-            e = pc_seg_exact_d2(p[j].x, p[j].y, p[j].z, G);
+            have = pc_seg_leaf(p[j].x, p[j].y, p[j].z, S, G, e);
             id = (uint32_t)__float_as_int(p[j].w);
-            have = e <= S.r2;
         }
         const float before = W.thr;
         pc_knn_warp_insert(have, e, id, lane, K, W);
@@ -131,16 +158,17 @@ __device__ __forceinline__ void pc_seg_scan(const pc_tree &T, const uint32_t (&r
     }
 }
 
-// the frontier walk of pc_knn_warp_search with the segment's node test
+// the frontier walk of pc_knn_warp_search with GEO's node test
+template <class GEO>
 __device__ __forceinline__ void pc_seg_search(const pc_tree &T, const pc_seg_dev &S, const pc_knn_dev &K, uint2 *__restrict__ F,
-                                              int lane, pc_seg_geo &G, pc_knn_wlist &W)
+                                              int lane, GEO &G, pc_knn_wlist &W)
 {
     const uint32_t lt = (1u << lane) - 1u;
     const int n_seed = (int)T.seeds[0], n_seed_leaf = (int)T.seeds[1];
     for (int base = 0; base < n_seed_leaf; base += 32) {
         uint32_t ref[1] = { 0u }, cnt[1] = { 0u };
         if (base + lane < n_seed_leaf) { ref[0] = T.seeds[PC_SEED_LEAF + 2 * (base + lane)]; cnt[0] = T.seeds[PC_SEED_LEAF + 2 * (base + lane) + 1]; }
-        pc_seg_scan<1>(T, ref, cnt, lane, S, K, G, W);
+        pc_seg_scan<1, GEO>(T, ref, cnt, lane, S, K, G, W);
     }
     if (lane < n_seed) F[lane] = make_uint2(T.seeds[PC_SEED_INNER + lane], 0u);
     int size = n_seed;
@@ -152,7 +180,7 @@ __device__ __forceinline__ void pc_seg_search(const pc_tree &T, const pc_seg_dev
         if (active) en = F[size - 1 - lane];
         size -= take;
         __syncwarp();
-        active = active && __uint_as_float(en.y) <= G.thr2;
+        active = active && __uint_as_float(en.y) <= pc_seg_lim(G);
         float dn = INFINITY, df = INFINITY;
         uint32_t cn = 0, cf = 0;
         uint32_t ref[2] = { 0u, 0u }, cnt[2] = { 0u, 0u };
@@ -165,17 +193,17 @@ __device__ __forceinline__ void pc_seg_search(const pc_tree &T, const pc_seg_dev
             const uint32_t rn = first0 ? r0 : r1, rf = first0 ? r1 : r0;
             const uint32_t kn = pc_rec_cnt(rec, first0 ? 0 : 1), kf = pc_rec_cnt(rec, first0 ? 1 : 0);
             const float dnn = fminf(d0, d1), dff = fmaxf(d0, d1);
-            if (dnn <= G.thr2) {
+            if (dnn <= pc_seg_lim(G)) {
                 if (rn & PC_REF_LEAF) { ref[0] = rn; cnt[0] = kn; }
                 else { cn = rn; dn = dnn; }
             }
-            if (dff <= G.thr2) {
+            if (dff <= pc_seg_lim(G)) {
                 if (rf & PC_REF_LEAF) { ref[1] = rf; cnt[1] = kf; }
                 else { cf = rf; df = dff; }
             }
         }
-        if (__ballot_sync(PC_FULL_MASK, (cnt[0] | cnt[1]) != 0u)) pc_seg_scan<2>(T, ref, cnt, lane, S, K, G, W);
-        const bool wn = dn <= G.thr2, wf = df <= G.thr2;
+        if (__ballot_sync(PC_FULL_MASK, (cnt[0] | cnt[1]) != 0u)) pc_seg_scan<2, GEO>(T, ref, cnt, lane, S, K, G, W);
+        const bool wn = dn <= pc_seg_lim(G), wf = df <= pc_seg_lim(G);
         const uint32_t mf = __ballot_sync(PC_FULL_MASK, wf), mn = __ballot_sync(PC_FULL_MASK, wn);
         const int nf = __popc(mf), nn = __popc(mn);
         if (wf) F[size + __popc(mf & lt)] = make_uint2(cf, __float_as_uint(df));

@@ -198,6 +198,22 @@ class PointCloudIndex:
         self._torch_fence(tm, after=True)
         return idx, d2
 
+    def sphere_sweep(self, a, b, radius, flags=L.PC_QUERY_AUTO):
+        """First contact of a sphere of the given radius moved from a[i] to b[i] (pc_sphere_sweep_batch).  Returns (idx int32,
+        t float32): the contacting point with the smallest (t, index) and that t rounded down, so a + t (b - a) never passes
+        the contact; -1 / inf without contact, -1 / NaN for a non-finite endpoint.  a and b are both numpy arrays or both
+        torch CUDA tensors of the same shape."""
+        pa, m, stride, space, keep_a, tm = self._rows(a, "a")
+        pb, mb, stride_b, space_b, keep_b, _ = self._rows(b, "b")
+        if (mb, stride_b, space_b) != (m, stride, space):
+            raise ValueError("sphere_sweep: a and b need the same shape and memory space")
+        idx, pi = self._out(m, np.int32, tm, keep_a)
+        t, pt = self._out(m, np.float32, tm, keep_a)
+        self._torch_fence(tm)
+        self._check(self._L.pc_sphere_sweep_batch(self._h, pa, pb, m, stride, space, int(flags), float(radius), pi, pt))
+        self._torch_fence(tm, after=True)
+        return idx, t
+
     def radius(self, q, params: L.PcRadiusParams, flags=L.PC_RADIUS_BOUNDED, want_idx=False):
         """safeRegionRrtStar::radiusSearch for every row of q.  Returns radius float32 (and idx int32)."""
         p, m, stride, space, keep, tm = self._rows(q, "q")
