@@ -108,7 +108,9 @@ typedef struct pc_index_view {
     const void *records;   /* float4[4 * n_nodes]: node i -> 16 words, the boxes of its two children interleaved per axis:
                               [min0.x min1.x min0.y min1.y min0.z min1.z ref0 ref1 | max0.x max1.x max0.y max1.y max0.z max1.z cnt0 cnt1]
                               ref = child reference (bit 31: leaf, low bits: first point), cnt = leaf point count       */
-    float bbox_lo[3], bbox_hi[3];
+    float bbox_lo[3], bbox_hi[3];  /* per-axis min / max over the points whose x, y and z are all finite: the frame of the
+                              curve keys.  Points with a NaN or infinite coordinate are indexed but do not widen it.  A cloud
+                              without a finite point gives bbox_lo = +inf and bbox_hi = -inf; an empty index gives zeros  */
 } pc_index_view;
 
 /* ---- lifetime ------------------------------------------------------------------------------- */

@@ -26,18 +26,19 @@
 #define PC_BUILD_THREADS 256
 
 // ---- bounding box of the cloud: bbox[0..2] = ordered(min), bbox[3..5] = ordered(max) ----------------
+// Only points whose three coordinates are all finite count: one infinite coordinate would make the extent infinite, the
+// cell size zero and every key 0 (the tree would follow the input order).  Points with a NaN or an infinity are still
+// indexed; their cells clamp to the frame.  A cloud without a finite point keeps the initial +inf / -inf.
 __global__ void __launch_bounds__(PC_BUILD_THREADS)
 pc_bbox_kernel(const float *__restrict__ xyz, int64_t n, int stride, uint32_t *__restrict__ bbox)
 {
     float lo[3] = { INFINITY, INFINITY, INFINITY }, hi[3] = { -INFINITY, -INFINITY, -INFINITY };
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
         const float *p = xyz + i * stride;
-#pragma unroll
-        for (int a = 0; a < 3; a++) {
-            float v = p[a];
-            lo[a] = fminf(lo[a], v);   // fminf/fmaxf drop NaNs
-            hi[a] = fmaxf(hi[a], v);
-        }
+        const float x = p[0], y = p[1], z = p[2];
+        if (!(isfinite(x) && isfinite(y) && isfinite(z))) continue;
+        lo[0] = fminf(lo[0], x); lo[1] = fminf(lo[1], y); lo[2] = fminf(lo[2], z);
+        hi[0] = fmaxf(hi[0], x); hi[1] = fmaxf(hi[1], y); hi[2] = fmaxf(hi[2], z);
     }
 #pragma unroll
     for (int a = 0; a < 3; a++) {
