@@ -14,7 +14,8 @@
 //                         (lane j holds the j-th entry); also answers the queries of the packets the packet kernel puts aside
 //   pc_knn_packet_kernel  one warp walks the tree once for the 32 neighbouring queries of a curve-ordered batch (the walk of
 //                         pc_packet_traverse); every lane keeps its query's k-list in shared memory
-// The warp walk (pc_knn_warp_search) is a template over the list, shared with pc_knn_large_kernel (knn_large_kernels.cuh).
+// The warp walk (pc_warp_walk) is a template over the geometry and the list, shared with pc_knn_large_kernel
+// (knn_large_kernels.cuh), pc_segment_kernel and pc_sphere_sweep_kernel.
 #pragma once
 #include "query_kernels.cuh"
 
@@ -111,9 +112,28 @@ __device__ __forceinline__ void pc_knn_warp_scan(const pc_tree &T, const uint32_
     }
 }
 
+// The bounded warp walk below is shared by the kNN kernels (GEO = pc_point_geo) and the segment kernels (pc_seg_geo and
+// pc_sweep_geo, segment_kernels.cuh / sweep_kernels.cuh).  GEO supplies, by overload: pc_walk_keys (the frontier keys of a
+// record's two children, INFINITY when pruned), pc_walk_lim (the limit the keys are compared to) and pc_walk_scan (the leaf
+// scan of NL leaves per lane, which offers its survivors to the list W).
+struct pc_point_geo {                   // a query point
+    float qx, qy, qz;
+};
+
+__device__ __forceinline__ float2 pc_walk_keys(const pc_rec &rec, const pc_point_geo &G) { return pc_rec_d2(rec, G.qx, G.qy, G.qz); }
+
 template <typename LIST>
-__device__ __forceinline__ void pc_knn_warp_search(const pc_tree &T, const pc_knn_dev &K, float qx, float qy, float qz,
-                                                   uint2 *__restrict__ F, int lane, LIST &W)
+__device__ __forceinline__ float pc_walk_lim(const pc_point_geo &, const LIST &W) { return W.thr; }
+
+template <int NL, typename LIST>
+__device__ __forceinline__ void pc_walk_scan(const pc_tree &T, const uint32_t (&ref)[NL], const uint32_t (&cnt)[NL], int lane,
+                                             const pc_knn_dev &K, const pc_point_geo &G, LIST &W)
+{
+    pc_knn_warp_scan<NL>(T, ref, cnt, G.qx, G.qy, G.qz, lane, K, W);
+}
+
+template <class GEO, typename LIST>
+__device__ __forceinline__ void pc_warp_walk(const pc_tree &T, const pc_knn_dev &K, uint2 *__restrict__ F, int lane, GEO &G, LIST &W)
 {
     const uint32_t lt = (1u << lane) - 1u;
     // the seeds: leaves met while the top of the tree was expanded (one per lane, their own counts) and <= 32 inner nodes
@@ -121,7 +141,7 @@ __device__ __forceinline__ void pc_knn_warp_search(const pc_tree &T, const pc_kn
     for (int base = 0; base < n_seed_leaf; base += 32) {
         uint32_t ref[1] = { 0u }, cnt[1] = { 0u };
         if (base + lane < n_seed_leaf) { ref[0] = T.seeds[PC_SEED_LEAF + 2 * (base + lane)]; cnt[0] = T.seeds[PC_SEED_LEAF + 2 * (base + lane) + 1]; }
-        pc_knn_warp_scan<1>(T, ref, cnt, qx, qy, qz, lane, K, W);
+        pc_walk_scan<1>(T, ref, cnt, lane, K, G, W);
     }
     if (lane < n_seed) F[lane] = make_uint2(T.seeds[PC_SEED_INNER + lane], 0u);
     int size = n_seed;
@@ -134,30 +154,30 @@ __device__ __forceinline__ void pc_knn_warp_search(const pc_tree &T, const pc_kn
         if (active) en = F[size - 1 - lane];
         size -= take;
         __syncwarp();
-        active = active && __uint_as_float(en.y) <= W.thr;
+        active = active && __uint_as_float(en.y) <= pc_walk_lim(G, W);
         float dn = INFINITY, df = INFINITY;          // inner children to push (INFINITY: none)
         uint32_t cn = 0, cf = 0;
         uint32_t ref[2] = { 0u, 0u }, cnt[2] = { 0u, 0u };   // leaf children to scan
         if (active) {
             const pc_rec rec = pc_load_rec(T.rec + 4ull * en.x);
-            const float2 dd = pc_rec_d2(rec, qx, qy, qz);
+            const float2 dd = pc_walk_keys(rec, G);
             const bool first0 = dd.x <= dd.y;
             const uint32_t r0 = pc_rec_ref(rec, 0), r1 = pc_rec_ref(rec, 1);
             const uint32_t rn = first0 ? r0 : r1, rf = first0 ? r1 : r0;
             const uint32_t kn = pc_rec_cnt(rec, first0 ? 0 : 1), kf = pc_rec_cnt(rec, first0 ? 1 : 0);
             const float dnn = fminf(dd.x, dd.y), dff = fmaxf(dd.x, dd.y);
-            if (dnn <= W.thr) {
+            if (dnn <= pc_walk_lim(G, W)) {
                 if (rn & PC_REF_LEAF) { ref[0] = rn; cnt[0] = kn; }
                 else { cn = rn; dn = dnn; }
             }
-            if (dff <= W.thr) {
+            if (dff <= pc_walk_lim(G, W)) {
                 if (rf & PC_REF_LEAF) { ref[1] = rf; cnt[1] = kf; }
                 else { cf = rf; df = dff; }
             }
         }
-        if (__ballot_sync(PC_FULL_MASK, (cnt[0] | cnt[1]) != 0u)) pc_knn_warp_scan<2>(T, ref, cnt, qx, qy, qz, lane, K, W);
+        if (__ballot_sync(PC_FULL_MASK, (cnt[0] | cnt[1]) != 0u)) pc_walk_scan<2>(T, ref, cnt, lane, K, G, W);
         // push the inner children that survive the (possibly tightened) bound, the nearer ones on top
-        const bool wn = dn <= W.thr, wf = df <= W.thr;
+        const bool wn = dn <= pc_walk_lim(G, W), wf = df <= pc_walk_lim(G, W);
         const uint32_t mf = __ballot_sync(PC_FULL_MASK, wf), mn = __ballot_sync(PC_FULL_MASK, wn);
         const int nf = __popc(mf), nn = __popc(mn);
         if (wf) F[size + __popc(mf & lt)] = make_uint2(cf, __float_as_uint(df));
@@ -183,11 +203,11 @@ pc_knn_coop_kernel(pc_tree T, pc_knn_dev K, const float *__restrict__ q, int64_t
         const long long t = K.defer_count ? (long long)K.defer_list[it >> 5] * 32 + (long long)(it & 31u) : (long long)it;
         if (t >= m_search) continue;
         uint32_t slot;
-        float qx, qy, qz;
-        pc_knn_fetch(q, qstride, perm, ordered, t, slot, qx, qy, qz);
+        pc_point_geo G;
+        pc_knn_fetch(q, qstride, perm, ordered, t, slot, G.qx, G.qy, G.qz);
         pc_knn_wlist W;
         W.ld = W.kd = INFINITY; W.li = W.ki = PC_KNN_NONE; W.thr = K.bound_thr;
-        if (T.n_points > 0) pc_knn_warp_search(T, K, qx, qy, qz, s_front[w], lane, W);
+        if (T.n_points > 0) pc_warp_walk(T, K, s_front[w], lane, G, W);
         if (lane < K.k) {
             const size_t o = (size_t)slot * K.k + lane;
             if (out_idx) out_idx[o] = (int32_t)W.li;

@@ -1,7 +1,7 @@
 // knn_large_kernels.cuh -- pc_knn_large_batch: exact k-nearest-neighbour rows for PC_KNN_MAX < k <= PC_KNN_LARGE_MAX.
 //
 // Same rows as pc_knn_batch (knn_kernels.cuh): the k smallest (fp64 d2 = pc_exact_d2, original index), the optional bound
-// d2 <= r2, padding (-1, +inf).  The walk is pc_knn_warp_search, one WARP per query (seeds, then up to 32 frontier nodes a
+// d2 <= r2, padding (-1, +inf).  The walk is pc_warp_walk, one WARP per query (seeds, then up to 32 frontier nodes a
 // step, fp32 box / point filter against thr, the fp64 re-check of every survivor, leaves over their own counts).  Only the
 // list differs: a k-list spread over the lanes holds at most 32 entries, so here it lives in shared memory:
 //   list   the first n (<= k) entries, ascending by (d2, index): 12 k bytes per warp
@@ -130,11 +130,11 @@ pc_knn_large_kernel(pc_tree T, pc_knn_dev K, const float *__restrict__ q, int64_
     const long long n_warps = (long long)gridDim.x * PC_KNN_LARGE_WARPS;
     for (long long t = (long long)blockIdx.x * PC_KNN_LARGE_WARPS + w; t < m_search; t += n_warps) {
         uint32_t slot;
-        float qx, qy, qz;
-        pc_knn_fetch(q, qstride, perm, ordered, t, slot, qx, qy, qz);
+        pc_point_geo G;
+        pc_knn_fetch(q, qstride, perm, ordered, t, slot, G.qx, G.qy, G.qz);
         W.n = W.qn = 0;
         W.kd = INFINITY; W.ki = PC_KNN_NONE; W.thr = K.bound_thr;
-        if (T.n_points > 0) pc_knn_warp_search(T, K, qx, qy, qz, F, lane, W);
+        if (T.n_points > 0) pc_warp_walk(T, K, F, lane, G, W);
         if (W.qn > 0) pc_knnl_flush(lane, K, W);
         const size_t o = (size_t)slot * K.k;
         for (int j = lane; j < K.k; j += 32) {

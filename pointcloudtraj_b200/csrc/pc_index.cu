@@ -213,6 +213,20 @@ static int pc_grow(pc_index *ix, T **ptr, int64_t *cap, int64_t want, int64_t mi
     return PC_OK;
 }
 
+// the lane's sort buffers (two key and two value buffers of 32-bit words): exactly `want` entries each when they have to grow
+static int pc_grow_sort(pc_index *ix, pc_lane &L, int64_t want)
+{
+    if (want <= L.sort_cap) return PC_OK;
+    pc_pool_free(ix, L.keys_a); pc_pool_free(ix, L.keys_b); pc_pool_free(ix, L.vals_a); pc_pool_free(ix, L.vals_b);
+    L.keys_a = L.keys_b = L.vals_a = L.vals_b = nullptr; L.sort_cap = 0;
+    PC_CUDA(ix, pc_pool_alloc(ix, (void **)&L.keys_a, (size_t)want * 4));
+    PC_CUDA(ix, pc_pool_alloc(ix, (void **)&L.keys_b, (size_t)want * 4));
+    PC_CUDA(ix, pc_pool_alloc(ix, (void **)&L.vals_a, (size_t)want * 4));
+    PC_CUDA(ix, pc_pool_alloc(ix, (void **)&L.vals_b, (size_t)want * 4));
+    L.sort_cap = want;
+    return PC_OK;
+}
+
 // scratch words a sort of n pairs needs: the three-kernel path's tile histograms or the onesweep path's tickets + digit
 // histograms + per-pass tile status, whichever is larger
 static int64_t pc_sort_scratch_words(int64_t n, int items, int passes)
@@ -615,17 +629,9 @@ static int pc_sort_queries(pc_index *ix, pc_lane &L, const pc_qargs &A, const fl
     // 8 bytes and one synchronisation of the ordering stream -- and size every later launch by it.  PC_DEVICE calls only:
     // the pipelined spaces (chunked PC_HOST, the ASYNC ones) must not stall the host between their copies.
     const bool exact = may_sync && ix->shard_n > 1 && ix->shard_exact && m >= PC_SHARD_EXACT_MIN;
-    if (m > L.sort_cap) {
-        int64_t c = m;
-        pc_pool_free(ix, L.keys_a); pc_pool_free(ix, L.keys_b); pc_pool_free(ix, L.vals_a); pc_pool_free(ix, L.vals_b);
-        L.keys_a = L.keys_b = L.vals_a = L.vals_b = nullptr; L.sort_cap = 0;
-        PC_CUDA(ix, pc_pool_alloc(ix, (void **)&L.keys_a, (size_t)c * 4));
-        PC_CUDA(ix, pc_pool_alloc(ix, (void **)&L.keys_b, (size_t)c * 4));
-        PC_CUDA(ix, pc_pool_alloc(ix, (void **)&L.vals_a, (size_t)c * 4));
-        PC_CUDA(ix, pc_pool_alloc(ix, (void **)&L.vals_b, (size_t)c * 4));
-        L.sort_cap = c;
-    }
-    int rc = pc_grow(ix, &L.tile_hist, &L.hist_cap, pc_sort_scratch_words(m, 8, 4));
+    int rc = pc_grow_sort(ix, L, m);
+    if (rc != PC_OK) return rc;
+    rc = pc_grow(ix, &L.tile_hist, &L.hist_cap, pc_sort_scratch_words(m, 8, 4));
     if (rc != PC_OK) return rc;
     // sort_bits (16 / 24 / 32) = radix-sorted key width = how many of the top curve bits order the batch; queries that
     // need no search (sensing-range early-outs) are answered by the key kernel and never enter the sort
@@ -777,6 +783,18 @@ static void pc_launch_coop(const pc_index *ix, const pc_qargs &A, const pc_tree 
     else pc_launch_coop_g<8>(A, T, d_q, m, qstride, d_idx, d_f, st);
 }
 
+// Unbounded packet walks are shared by queries within a few packet extents of each other only (pc_query_packet_kernel,
+// pc_knn_packet_kernel): 64 queries fill a cube of edge e0 = cell * cbrt(64 / per_cell) at the density of the batch lane L has
+// just ordered (cell = 1/256 of the cloud's extent).  Returns ix->packet_split times e0, or 0 (no split).
+static float pc_packet_split(const pc_index *ix, const pc_lane &L)
+{
+    if (!(ix->packet_split > 0.f && L.per_cell > 0.0)) return 0.f;
+    float emax = 0.f;
+    for (int a = 0; a < 3; a++) { const float e = pc_ordered_to_float(ix->h_bbox[3 + a]) - pc_ordered_to_float(ix->h_bbox[a]); emax = e > emax ? e : emax; }
+    const float split = ix->packet_split * (emax / 256.f) * (float)cbrt(64.0 / L.per_cell);
+    return split > 0.f ? split : 0.f;
+}
+
 // run one device-resident batch on lane L
 static int pc_run_batch(pc_index *ix, pc_lane &L, const pc_qargs &A, const float *d_q, int64_t m, int qstride,
                         int32_t *d_idx, float *d_f, bool split_streams = false, bool may_sync = false)
@@ -815,16 +833,12 @@ static int pc_run_batch(pc_index *ix, pc_lane &L, const pc_qargs &A, const float
     const bool two_per_lane = ix->query_kernel == 4 || (ix->query_kernel_auto && L.per_cell >= 3.0);
     const bool is_ordered = perm || ordered;
     const int64_t ml = is_ordered ? m_launch : m;        // entries the search launch has to cover
-    // unbounded packet walks are shared by queries within a few packet extents of each other only (pc_query_packet_kernel):
-    // 64 queries fill a cube of edge e0 = cell * cbrt(64 / per_cell) at the batch's density (cell = 1/256 of the cloud's extent)
+    // unbounded packet walks put their incoherent packets aside (pc_packet_split)
     pc_radius_dev RN = A.R;
     if ((A.kind == PC_Q_NEAREST || !A.R.bounded) && ix->packet_split > 0.f && L.per_cell > 0.0) {
-        float emax = 0.f;
-        for (int a = 0; a < 3; a++) { const float e = pc_ordered_to_float(ix->h_bbox[3 + a]) - pc_ordered_to_float(ix->h_bbox[a]); emax = e > emax ? e : emax; }
-        RN.packet_split = ix->packet_split * (emax / 256.f) * (float)cbrt(64.0 / L.per_cell);
+        RN.packet_split = is_ordered ? pc_packet_split(ix, L) : 0.f;
         RN.defer_count = L.counter;             // zeroed above
         RN.defer_list = L.keys_a;               // the ordering pass is done with its key buffer; one entry per packet at most
-        if (!(RN.packet_split > 0.f) || !is_ordered) RN.packet_split = 0.f;
     }
     if (ml == 0) {
         // pc_batch_shard: nothing of this batch belongs to this rank

@@ -3,11 +3,10 @@
 // d2(p) is the fp64 expression of the contract (pc_index.h, DESIGN.md §4.11), evaluated by pc_seg_exact_d2 in exactly that
 // operation order; the answer is the smallest (d2, original index), with the optional bound d2 <= r2 of pc_knn_batch.
 //
-//   pc_segment_kernel   one WARP per segment: the frontier walk of pc_knn_warp_search (seeds, then up to 32 frontier nodes a
-//                       step, depth-first close to the frontier's capacity) with the k = 1 list of pc_knn_wlist.  The walk is a
-//                       copy, not an instantiation of the kNN walk: the node test and the leaf scan differ, and the existing kNN
-//                       kernels stay byte-identical.  pc_seg_search is itself a template over the geometry, shared with
-//                       pc_sphere_sweep_kernel (sweep_kernels.cuh).
+//   pc_segment_kernel   one WARP per segment: the frontier walk of the kNN kernels (pc_warp_walk, knn_kernels.cuh: seeds, then
+//                       up to 32 frontier nodes a step, depth-first close to the frontier's capacity) with the k = 1 list of
+//                       pc_knn_wlist.  The segment's geometry pc_seg_geo supplies the walk's node test and leaf scan, as
+//                       pc_sweep_geo does for pc_sphere_sweep_kernel (sweep_kernels.cuh).
 //
 // Node test (pc_seg_box): a child is pruned only if no point of its box can have fp64 d2 <= the current best (or the bound).
 // Such a point lies within rho = sqrt(thr) + tau of the segment, where thr >= best (1 + 2^-20) is the kNN walks' fp32
@@ -21,6 +20,7 @@
 // test on the box [p, p] -- measured 10 % slower on long unbounded segments and 1-2 % faster bounded; DESIGN.md §4.11).
 #pragma once
 #include "knn_kernels.cuh"
+#include <type_traits>
 
 #define PC_SEG_WARPS 4                  // warps per CTA (32 KB of frontier)
 #define PC_SEG_TAU_REL 0x1p-48f         // tau = |b - a| * 2^-48 + 2^-100 (DESIGN.md §4.11: 3.001 * 2^-53 |b - a| suffices)
@@ -118,25 +118,34 @@ __device__ __forceinline__ float pc_seg_box(float lx, float ly, float lz, float 
     return t0 <= t1 ? g2 : INFINITY;
 }
 
-// the segment's leaf evaluation: the list key d2, and whether the bound keeps it
-__device__ __forceinline__ bool pc_seg_leaf(float px, float py, float pz, const pc_seg_dev &S, const pc_seg_geo &G, double &e)
+// the segment's leaf evaluation: the list key d2, and whether the bound K.r2 keeps it
+__device__ __forceinline__ bool pc_seg_leaf(float px, float py, float pz, const pc_knn_dev &K, const pc_seg_geo &G, double &e)
 {
     e = pc_seg_exact_d2(px, py, pz, G);
-    return e <= S.r2;
+    return e <= K.r2;
 }
 
-// the limit the frontier's keys are tested against: rho^2 (the gap is a squared distance)
-__device__ __forceinline__ float pc_seg_lim(const pc_seg_geo &G) { return G.thr2; }
+// The hooks of pc_warp_walk (knn_kernels.cuh) for pc_seg_geo and pc_sweep_geo (sweep_kernels.cuh).  Each geometry supplies,
+// by overload: pc_seg_box (node test: the frontier key, INFINITY when pruned), pc_walk_lim (the key limit), pc_seg_leaf (list
+// key of a point, and whether it counts) and pc_seg_set_thr (refresh after the list's threshold changed).  The templates are
+// constrained to the segment geometries: unconstrained, they would tie with pc_point_geo's hooks.
+template <class GEO>
+using pc_if_seg_geo = typename std::enable_if<std::is_base_of<pc_seg_geo, GEO>::value, int>::type;
 
-// The walk below is shared by pc_segment_kernel (GEO = pc_seg_geo) and pc_sphere_sweep_kernel (GEO = pc_sweep_geo,
-// sweep_kernels.cuh).  GEO supplies, by overload: pc_seg_box (node test: the frontier key, INFINITY when pruned), pc_seg_lim
-// (the key limit), pc_seg_leaf (list key of a point, and whether it counts) and pc_seg_set_thr (refresh after the list's
-// threshold changed).
+// the limit the frontier's keys are tested against: rho^2 (the gap is a squared distance)
+__device__ __forceinline__ float pc_walk_lim(const pc_seg_geo &G, const pc_knn_wlist &) { return G.thr2; }
+
+template <class GEO, pc_if_seg_geo<GEO> = 0>
+__device__ __forceinline__ float2 pc_walk_keys(const pc_rec &rec, const GEO &G)
+{
+    return make_float2(pc_seg_box(rec.L[0], rec.L[2], rec.L[4], rec.H[0], rec.H[2], rec.H[4], G),
+                       pc_seg_box(rec.L[1], rec.L[3], rec.L[5], rec.H[1], rec.H[3], rec.H[5], G));
+}
 
 // scan NL leaves per lane (cnt points each; 0 = none) and offer the survivors to the k = 1 list
-template <int NL, class GEO>
-__device__ __forceinline__ void pc_seg_scan(const pc_tree &T, const uint32_t (&ref)[NL], const uint32_t (&cnt)[NL], int lane,
-                                            const pc_seg_dev &S, const pc_knn_dev &K, GEO &G, pc_knn_wlist &W)
+template <int NL, class GEO, pc_if_seg_geo<GEO> = 0>
+__device__ __forceinline__ void pc_walk_scan(const pc_tree &T, const uint32_t (&ref)[NL], const uint32_t (&cnt)[NL], int lane,
+                                             const pc_knn_dev &K, GEO &G, pc_knn_wlist &W)
 {
     float4 p[NL * PC_LEAF];
 #pragma unroll
@@ -149,67 +158,12 @@ __device__ __forceinline__ void pc_seg_scan(const pc_tree &T, const uint32_t (&r
         double e = 0.0;
         uint32_t id = 0u;
         if (have) {
-            have = pc_seg_leaf(p[j].x, p[j].y, p[j].z, S, G, e);
+            have = pc_seg_leaf(p[j].x, p[j].y, p[j].z, K, G, e);
             id = (uint32_t)__float_as_int(p[j].w);
         }
         const float before = W.thr;
         pc_knn_warp_insert(have, e, id, lane, K, W);
         if (W.thr != before) pc_seg_set_thr(W.thr, G);
-    }
-}
-
-// the frontier walk of pc_knn_warp_search with GEO's node test
-template <class GEO>
-__device__ __forceinline__ void pc_seg_search(const pc_tree &T, const pc_seg_dev &S, const pc_knn_dev &K, uint2 *__restrict__ F,
-                                              int lane, GEO &G, pc_knn_wlist &W)
-{
-    const uint32_t lt = (1u << lane) - 1u;
-    const int n_seed = (int)T.seeds[0], n_seed_leaf = (int)T.seeds[1];
-    for (int base = 0; base < n_seed_leaf; base += 32) {
-        uint32_t ref[1] = { 0u }, cnt[1] = { 0u };
-        if (base + lane < n_seed_leaf) { ref[0] = T.seeds[PC_SEED_LEAF + 2 * (base + lane)]; cnt[0] = T.seeds[PC_SEED_LEAF + 2 * (base + lane) + 1]; }
-        pc_seg_scan<1, GEO>(T, ref, cnt, lane, S, K, G, W);
-    }
-    if (lane < n_seed) F[lane] = make_uint2(T.seeds[PC_SEED_INNER + lane], 0u);
-    int size = n_seed;
-    __syncwarp();
-    while (size > 0) {
-        const int take = (size + 32 + PC_STACK <= PC_KNN_FRONT) ? min(size, 32) : 1;
-        bool active = lane < take;
-        uint2 en = make_uint2(0u, 0u);
-        if (active) en = F[size - 1 - lane];
-        size -= take;
-        __syncwarp();
-        active = active && __uint_as_float(en.y) <= pc_seg_lim(G);
-        float dn = INFINITY, df = INFINITY;
-        uint32_t cn = 0, cf = 0;
-        uint32_t ref[2] = { 0u, 0u }, cnt[2] = { 0u, 0u };
-        if (active) {
-            const pc_rec rec = pc_load_rec(T.rec + 4ull * en.x);
-            const float d0 = pc_seg_box(rec.L[0], rec.L[2], rec.L[4], rec.H[0], rec.H[2], rec.H[4], G);
-            const float d1 = pc_seg_box(rec.L[1], rec.L[3], rec.L[5], rec.H[1], rec.H[3], rec.H[5], G);
-            const bool first0 = d0 <= d1;
-            const uint32_t r0 = pc_rec_ref(rec, 0), r1 = pc_rec_ref(rec, 1);
-            const uint32_t rn = first0 ? r0 : r1, rf = first0 ? r1 : r0;
-            const uint32_t kn = pc_rec_cnt(rec, first0 ? 0 : 1), kf = pc_rec_cnt(rec, first0 ? 1 : 0);
-            const float dnn = fminf(d0, d1), dff = fmaxf(d0, d1);
-            if (dnn <= pc_seg_lim(G)) {
-                if (rn & PC_REF_LEAF) { ref[0] = rn; cnt[0] = kn; }
-                else { cn = rn; dn = dnn; }
-            }
-            if (dff <= pc_seg_lim(G)) {
-                if (rf & PC_REF_LEAF) { ref[1] = rf; cnt[1] = kf; }
-                else { cf = rf; df = dff; }
-            }
-        }
-        if (__ballot_sync(PC_FULL_MASK, (cnt[0] | cnt[1]) != 0u)) pc_seg_scan<2, GEO>(T, ref, cnt, lane, S, K, G, W);
-        const bool wn = dn <= pc_seg_lim(G), wf = df <= pc_seg_lim(G);
-        const uint32_t mf = __ballot_sync(PC_FULL_MASK, wf), mn = __ballot_sync(PC_FULL_MASK, wn);
-        const int nf = __popc(mf), nn = __popc(mn);
-        if (wf) F[size + __popc(mf & lt)] = make_uint2(cf, __float_as_uint(df));
-        if (wn) F[size + nf + (nn - 1 - __popc(mn & lt))] = make_uint2(cn, __float_as_uint(dn));
-        size += nf + nn;
-        __syncwarp();
     }
 }
 
@@ -237,7 +191,7 @@ pc_segment_kernel(pc_tree T, pc_seg_dev S, const float *__restrict__ a_xyz, cons
             pc_seg_geo G;
             pc_seg_setup(av, bv, G);
             pc_seg_set_thr(W.thr, G);
-            pc_seg_search(T, S, K, s_front[w], lane, G, W);
+            pc_warp_walk(T, K, s_front[w], lane, G, W);
         }
         if (lane == 0) {
             if (out_idx) out_idx[slot] = finite ? (int32_t)W.li : -1;

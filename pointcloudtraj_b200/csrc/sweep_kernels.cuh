@@ -3,7 +3,7 @@
 // t(p) is the fp64 expression of the contract (pc_index.h, DESIGN.md §4.12), evaluated by pc_sweep_exact_t in exactly that
 // operation order; the answer is the smallest (t, original index).
 //
-//   pc_sphere_sweep_kernel  one WARP per segment: the walk of pc_segment_kernel (pc_seg_search, segment_kernels.cuh) with
+//   pc_sphere_sweep_kernel  one WARP per segment: the walk of pc_segment_kernel (pc_warp_walk, knn_kernels.cuh) with
 //                           t(p) as the key of the k = 1 list (pc_knn_wlist: (key, index) order, the lowest index on ties).
 //
 // Node test (pc_seg_box of pc_sweep_geo): a point with a computed contact at t lies within rho of the exact segment point
@@ -49,11 +49,11 @@ __device__ __forceinline__ float pc_seg_box(float lx, float ly, float lz, float 
     return t0 <= t1 && g2 <= G.thr2 ? t0 : INFINITY;
 }
 
-__device__ __forceinline__ float pc_seg_lim(const pc_sweep_geo &G) { return G.tmax; }
+__device__ __forceinline__ float pc_walk_lim(const pc_sweep_geo &G, const pc_knn_wlist &) { return G.tmax; }
 
-__device__ __forceinline__ bool pc_seg_leaf(float px, float py, float pz, const pc_seg_dev &S, const pc_sweep_geo &G, double &e)
+__device__ __forceinline__ bool pc_seg_leaf(float px, float py, float pz, const pc_knn_dev &K, const pc_sweep_geo &G, double &e)
 {
-    e = pc_sweep_exact_t(px, py, pz, G, S.r2);
+    e = pc_sweep_exact_t(px, py, pz, G, K.r2);
     return e <= 1.0;
 }
 
@@ -85,7 +85,7 @@ pc_sphere_sweep_kernel(pc_tree T, pc_seg_dev S, float r_up, const float *__restr
             G.rho = __fadd_ru(r_up, __fmaf_ru(__fadd_ru(r_up, len), PC_SWEEP_RHO_REL, PC_SEG_TAU_ABS));
             G.thr2 = __fmul_ru(G.rho, G.rho);
             pc_seg_set_thr(W.thr, G);
-            pc_seg_search(T, S, K, s_front[w], lane, G, W);
+            pc_warp_walk(T, K, s_front[w], lane, G, W);
         }
         if (lane == 0) {
             if (out_idx) out_idx[slot] = finite ? (int32_t)W.li : -1;
