@@ -108,16 +108,19 @@ def _radius_for_count(pts, c, want):
 
 def test_range_sorted_long_lists(ix):
     """Every size class of the sort: up to 512 hits (the capturing warp; one list of exactly 512 and one of 513), up to
-    16384 (one CTA in shared memory) and beyond (one CTA in global memory), untruncated and cut to 50."""
+    16384 (one CTA in shared memory; one list of exactly 16384 and one of 16385) and beyond (one CTA in global memory),
+    untruncated and cut to 50."""
     pts, half = synth.forest_cloud(150_000, seed=6, variant="J", return_half=True)
     ix.build(pts)
     q = synth.rrt_queries(24, half, seed=5)
     radii = np.array([0.5, 2.0, 4.0, 6.0, 9.0, 12.0, 40.0, 5.0] * 3)
     radii[1] = _radius_for_count(pts, q[1], 512)
     radii[9] = _radius_for_count(pts, q[9], 513)
+    radii[17] = _radius_for_count(pts, q[17], 16384)
+    radii[18] = _radius_for_count(pts, q[18], 16385)
     full = brute_range_sorted(pts, q, radii)
     sizes = np.diff(full[0])
-    assert sizes[1] == 512 and sizes[9] == 513
+    assert sizes[1] == 512 and sizes[9] == 513 and sizes[17] == 16384 and sizes[18] == 16385
     assert (sizes > 32768).any() and ((sizes > 513) & (sizes <= 16384)).any() and ((sizes > 0) & (sizes < 512)).any()
     for max_nn in (0, 50):
         b = _truncate(*full, max_nn)
