@@ -21,6 +21,8 @@
  *                               (parameters of setParam :17-23, start point of setStartPt :43-50)
  *   pc_clearance_batch          checkSafeTrajectory + getPosFromBezier + checkTrajPtCol
  *                               Planner/src/sim_planning_demo.cpp:729-781, :715-727; corridor_finder.cpp:412-416
+ *   pc_trajectory_sweep_batch   (no counterpart: the reference samples every dt) certified first contact of a sphere moved
+ *                               along a piecewise Bezier trajectory
  *   pc_comm_* / pc_index_broadcast   (no counterpart: the reference is single-process) -- replicate the
  *                               built index to the other GPUs of the host with one ncclBroadcast.
  *
@@ -258,6 +260,35 @@ int  pc_clearance_batch(pc_index *ix, const pc_traj *traj, int64_t n_traj,
                         int64_t n_seg, const double *coef, int64_t n_coef, int space,
                         double dt, double horizon, const pc_radius_params *params,
                         int32_t *out_first_hit, float *out_min_radius, int32_t *out_n_samples);
+
+/* Certified first contact of a sphere of radius `radius` moved along each trajectory, in continuous time (not the dt walk of
+ * pc_clearance_batch).  Trajectory arrays, their validation and their spaces as pc_clearance_batch.  Segment s (order
+ * n = seg_order[s], duration T = seg_T[s]) is at local time sigma in [0, T] at the exact real value
+ * C_s(sigma) = T * sum_j C(n,j) c_j u^j (1-u)^(n-j), u = sigma / T: the Bezier curve of the control points T * c_j.
+ * The motion starts where pc_clearance_batch starts (t_s = max(0, t_now), then its fp64 segment-skipping loop: segment i0,
+ * local time sigma0), covers the rest of segment i0 and the following segments of the trajectory in order, and stops where
+ * the elapsed time reaches `horizon` (horizon == 0: the start point only; the end is rounded up, never cut short).  It is
+ * empty when horizon < 0, when the trajectory has no segment, or when sigma0 > T on its last segment.
+ * A cloud point p (float32 widened; non-finite points never touch) touches at (s, sigma) when |C_s(sigma) - p| <= radius.
+ * With F(rho) the first such (segment, sigma) of the motion in time order at radius rho, the answer (out_seg[t], out_s[t],
+ * out_idx[t]) = (s_c, sigma_c, i) satisfies
+ *   1. nothing earlier: (s_c, sigma_c) <= F(radius) -- every point of the motion before it is farther than radius from the cloud;
+ *   2. witness: |C_{s_c}(sigma_c) - p_i| <= radius + tol, so F(radius + tol) <= (s_c, sigma_c);
+ *   3. complete: a contact is reported whenever F(radius) exists (with closest approach in (radius, radius + tol] either
+ *      answer may come).
+ * out_seg is an index into the segment arrays; out_s is rounded down so that rule 1 holds.  No contact (or an empty motion,
+ * or an empty index): -1, +inf, -1.  A segment of the motion with a non-finite T or coefficient, or a control point T * c_j
+ * beyond 1e37 in magnitude: -1, NaN, -1 ("not checked").  Deterministic: PC_HOST and PC_DEVICE, and repeated calls, give the
+ * same bits.  Rule 2 is guaranteed for tol >= 2^-37 ((n + 1) S + radius) on the contact's segment, S = max_j |T * c_j|
+ * (DESIGN.md §4.13); the subdivision depth is capped at 50 levels so that every call terminates, and a piece still undecided
+ * there is reported at its start -- rule 1 holds, rule 2 may not (only below that tol).  Outputs are nullable.
+ * PC_EINVAL: radius negative, NaN or infinite; tol not finite or <= 0; horizon NaN; every argument pc_clearance_batch refuses
+ * (including its host-side validation of segment ranges, orders, offsets and T); the ASYNC spaces; a pc_batch_shard handle. */
+int  pc_trajectory_sweep_batch(pc_index *ix, const pc_traj *traj, int64_t n_traj,
+                               const int32_t *seg_order, const double *seg_T, const int64_t *seg_coef_off,
+                               int64_t n_seg, const double *coef, int64_t n_coef, int space,
+                               double horizon, double radius, double tol,
+                               int32_t *out_seg, double *out_s, int32_t *out_idx);
 
 /* ---- the RRT* sample stream and one speculative expansion batch, generated on the device ----------- */
 /* genSample's state (corridor_finder.cpp:333-358, the branches taken while no path is known: inform_status == false).

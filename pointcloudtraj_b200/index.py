@@ -336,10 +336,9 @@ class PointCloudIndex:
             sampler.engine_state = st.value
         return out[: cnt.value]
 
-    def clearance(self, traj_first_seg, seg_order, seg_T, seg_coef_off, coef, params: L.PcRadiusParams,
-                  t_now=None, dt=0.02, horizon=2.0):
-        """checkSafeTrajectory for a batch of piecewise Bezier trajectories (host arrays, CSR layout of
-        synth.bezier_trajectories).  Returns (first_hit int32, min_radius float32, n_samples int32)."""
+    @staticmethod
+    def _traj_arrays(traj_first_seg, seg_order, seg_T, seg_coef_off, coef, t_now):
+        """pc_traj records and the segment arrays of the CSR layout of synth.bezier_trajectories, contiguous for the C ABI."""
         first = np.ascontiguousarray(traj_first_seg, dtype=np.int32)
         n_traj = first.shape[0] - 1
         tn = np.zeros(n_traj) if t_now is None else np.ascontiguousarray(t_now, dtype=np.float64)
@@ -353,12 +352,33 @@ class PointCloudIndex:
         sT = np.ascontiguousarray(seg_T, dtype=np.float64)
         sc = np.ascontiguousarray(seg_coef_off, dtype=np.int64)
         cf = np.ascontiguousarray(coef, dtype=np.float64)
+        return n_traj, traj, so, sT, sc, cf
+
+    def clearance(self, traj_first_seg, seg_order, seg_T, seg_coef_off, coef, params: L.PcRadiusParams,
+                  t_now=None, dt=0.02, horizon=2.0):
+        """checkSafeTrajectory for a batch of piecewise Bezier trajectories (host arrays, CSR layout of
+        synth.bezier_trajectories).  Returns (first_hit int32, min_radius float32, n_samples int32)."""
+        n_traj, traj, so, sT, sc, cf = self._traj_arrays(traj_first_seg, seg_order, seg_T, seg_coef_off, coef, t_now)
         fh = np.empty(n_traj, np.int32); mr = np.empty(n_traj, np.float32); ns = np.empty(n_traj, np.int32)
         vp = lambda a: C.c_void_p(a.ctypes.data)
         self._check(self._L.pc_clearance_batch(self._h, C.c_void_p(traj.ctypes.data), n_traj, vp(so), vp(sT), vp(sc), so.shape[0],
                                                vp(cf), cf.shape[0], L.PC_HOST, float(dt), float(horizon), C.byref(params),
                                                vp(fh), vp(mr), vp(ns)))
         return fh, mr, ns
+
+    def trajectory_sweep(self, traj_first_seg, seg_order, seg_T, seg_coef_off, coef, radius, tol, t_now=None, horizon=2.0):
+        """Certified first contact of a sphere of the given radius moved along each trajectory in continuous time
+        (pc_trajectory_sweep_batch; host arrays, the layout of clearance()).  Returns (seg int32, s float64, idx int32): the
+        contact's segment (index into the segment arrays), its local time -- nothing on the trajectory before it is within
+        radius of the cloud -- and a cloud point within radius + tol of the position there; -1 / inf / -1 without contact,
+        -1 / NaN / -1 where a segment of the motion is not finite."""
+        n_traj, traj, so, sT, sc, cf = self._traj_arrays(traj_first_seg, seg_order, seg_T, seg_coef_off, coef, t_now)
+        seg = np.empty(n_traj, np.int32); s = np.empty(n_traj, np.float64); idx = np.empty(n_traj, np.int32)
+        vp = lambda a: C.c_void_p(a.ctypes.data)
+        self._check(self._L.pc_trajectory_sweep_batch(self._h, C.c_void_p(traj.ctypes.data), n_traj, vp(so), vp(sT), vp(sc),
+                                                      so.shape[0], vp(cf), cf.shape[0], L.PC_HOST, float(horizon), float(radius),
+                                                      float(tol), vp(seg), vp(s), vp(idx)))
+        return seg, s, idx
 
 
 def shard_range(m, rank, n_ranks):
