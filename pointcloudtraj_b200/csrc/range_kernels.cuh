@@ -42,11 +42,9 @@ __device__ __forceinline__ void pc_sort_list(int32_t *__restrict__ a, int64_t n)
 }
 
 // ---- one WARP per range query -----------------------------------------------------------------------------------------
-// Same frontier walk as pc_query_coop_kernel (query_kernels.cuh), without a bound to tighten: the open inner nodes sit on a
-// LIFO frontier in shared memory, every step each lane takes one of them and tests its two child boxes; a child that is a
-// leaf is scanned on the spot (only its own `count` points: its neighbours' points belong to other leaves) and the hits are
-// appended at ballot-computed positions, inner children are pushed.  The count / capture pass and the fill pass are the same
-// walk; the fill pass then sorts its list by original index with a bitonic network in the same shared memory (lists up to 1024 hits);
+// Same frontier walk as pc_query_coop_kernel (query_kernels.cuh), without a bound to tighten (pc_range_walk below); the hits
+// are appended at ballot-computed positions.  The count / capture pass and the fill pass are the same walk; the fill pass
+// then sorts its list by original index with a bitonic network in the same shared memory (lists up to 1024 hits);
 // longer lists are queued and sorted afterwards by pc_range_sort_long_kernel, one CTA per list (up to 32768 hits in shared
 // memory; beyond that a single-thread heap sort -- a query that returns more than that is a job for pc_sphere_gather).
 #define PC_RCOOP_CAP 1024
@@ -122,51 +120,41 @@ __device__ __forceinline__ uint32_t *pc_warp_radix_sort(uint32_t *A, uint32_t *B
     return A;
 }
 
-struct pc_range_stage {                // PC_RANGE_CAPTURE: where the counting pass parks the short lists
-    int32_t *stage;                    // stage_cap entries
-    unsigned long long stage_cap;
-    unsigned long long *cursor;        // next free entry
-    int64_t *pos;                      // per query: start of its parked list, -1 = not parked (walk it again)
+// ---- the range walk, shared by pc_range_coop_kernel and pc_range_sorted_kernel (range_sorted_kernels.cuh) ----------------
+// Query k of a range batch: its point (and in fp64), r2 = range^2 (the inclusive bound of the fp64 test) and the fp32 filter
+// thr.  False for an empty index or a NaN range: the query has no hits.
+struct pc_range_q {
+    float qx, qy, qz;
+    double qxd, qyd, qzd;
+    double r2;
+    float thr;
 };
 
-#define PC_RCAP_FRONT 768         // frontier entries of the capturing pass: 512 double as the sort's second buffer, 256 as its histogram
-template <int MODE>
-__global__ void __launch_bounds__(32 * PC_RCOOP_WARPS, MODE == PC_RANGE_CAPTURE ? PC_RCAP_MIN_CTAS : (MODE == PC_RANGE_COUNT ? 12 : 8))
-pc_range_coop_kernel(pc_tree T, const float *__restrict__ q, int64_t m, int qstride,
-                     const double *__restrict__ range, int range_is_scalar,
-                     int64_t *__restrict__ counts, const int64_t *__restrict__ offsets, int32_t *__restrict__ out_idx,
-                     unsigned long long *__restrict__ long_count, int64_t *__restrict__ long_list,
-                     pc_range_stage S, const int64_t *__restrict__ qlist, const unsigned long long *__restrict__ qlist_count)
+__device__ __forceinline__ bool pc_range_query(const pc_tree &T, const float *__restrict__ q, int64_t k, int qstride,
+                                               const double *__restrict__ range, int range_is_scalar, pc_range_q &Q)
 {
-    constexpr bool FILL = MODE == PC_RANGE_FILL;
-    constexpr bool CAPTURE = MODE == PC_RANGE_CAPTURE;
-    constexpr int FCAP = CAPTURE ? PC_RCAP_FRONT : PC_RCOOP_CAP;
-    __shared__ uint32_t s_front[PC_RCOOP_WARPS][FCAP];
-    __shared__ uint32_t s_hits[CAPTURE ? PC_RCOOP_WARPS : 1][CAPTURE ? PC_RCAP_HITS : 1];
-    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    int64_t k = (int64_t)blockIdx.x * PC_RCOOP_WARPS + w;
-    if (qlist) {                       // fill pass over the queries the capture left behind
-        if ((unsigned long long)k >= *qlist_count) return;
-        k = qlist[k];
-    }
-    if (k >= m) return;
-    uint32_t *H = s_hits[CAPTURE ? w : 0];
-    int64_t begin = 0, want = 0;
-    if (FILL) {
-        begin = offsets[k]; want = offsets[k + 1] - begin;
-        if (want == 0) return;
-    }
     const float *qq = q + k * qstride;
-    const float qx = qq[0], qy = qq[1], qz = qq[2];
-    const double qxd = (double)qx, qyd = (double)qy, qzd = (double)qz;
+    Q.qx = qq[0]; Q.qy = qq[1]; Q.qz = qq[2];
+    Q.qxd = (double)Q.qx; Q.qyd = (double)Q.qy; Q.qzd = (double)Q.qz;
     const double r = range[range_is_scalar ? 0 : k];
-    const double r2 = __dmul_rn(r, r);
-    if (T.n_points == 0 || !(r2 == r2)) {          // empty index, NaN range
-        if (!FILL && lane == 0) counts[k] = 0;
-        return;
-    }
-    const float thr = fminf(__fmul_ru(__double2float_ru(r2), PC_THR_SLACK), FLT_MAX);
-    uint32_t *F = s_front[w];
+    Q.r2 = __dmul_rn(r, r);
+    if (T.n_points == 0 || !(Q.r2 == Q.r2)) return false;
+    Q.thr = fminf(__fmul_ru(__double2float_ru(Q.r2), PC_THR_SLACK), FLT_MAX);
+    return true;
+}
+
+// One warp walks the tree for one query and returns its number of hits.  The open inner nodes sit on a LIFO frontier of FCAP
+// words in F; every step each lane takes one of them and tests its two child boxes; a child that is a leaf is scanned on the
+// spot (only its own `count` points: its neighbours' points belong to other leaves), inner children are pushed.  Every
+// scanned candidate goes to the sink S, in walk order, as pc_range_hit(S, hit, at, pos, id): `hit` whether it passed the
+// test, at() its place in the list, `pos` the point's position in the tree's point array, `id` its original index.  at()
+// is a callable so that each sink evaluates it where it needs it: inside or before its `hit` branch.  That choice shapes
+// the compiled walk, and each sink keeps the one its kernel was tuned with.  F is free again when the walk returns.
+template <int FCAP, class SINK>
+__device__ __forceinline__ int64_t pc_range_walk(const pc_tree &T, const pc_range_q &Q, uint32_t *F, int lane, SINK &S)
+{
+    const float qx = Q.qx, qy = Q.qy, qz = Q.qz, thr = Q.thr;
+    const double qxd = Q.qxd, qyd = Q.qyd, qzd = Q.qzd, r2 = Q.r2;
     const uint32_t lt = (1u << lane) - 1u;
     int64_t total = 0;
     int size = 0;
@@ -176,11 +164,13 @@ pc_range_coop_kernel(pc_tree T, const float *__restrict__ q, int64_t m, int qstr
         const int n_seed = (int)T.seeds[0], n_seed_leaf = (int)T.seeds[1];
         bool hit[PC_LEAF];
         int32_t id[PC_LEAF];
+        uint32_t at0 = 0;
 #pragma unroll
         for (int i = 0; i < PC_LEAF; i++) { hit[i] = false; id[i] = 0; }
         if (lane < n_seed_leaf) {
             const uint32_t ref = T.seeds[PC_SEED_LEAF + 2 * lane], cnt = T.seeds[PC_SEED_LEAF + 2 * lane + 1];
-            const float4 *pts = T.points + (ref & ~PC_REF_LEAF);
+            at0 = ref & ~PC_REF_LEAF;
+            const float4 *pts = T.points + at0;
 #pragma unroll
             for (int i = 0; i < PC_LEAF; i++) {
                 if ((uint32_t)i < cnt) {
@@ -195,8 +185,7 @@ pc_range_coop_kernel(pc_tree T, const float *__restrict__ q, int64_t m, int qstr
 #pragma unroll
             for (int i = 0; i < PC_LEAF; i++) {
                 const uint32_t mask = __ballot_sync(PC_FULL_MASK, hit[i]);
-                if (FILL && hit[i]) out_idx[begin + total + __popc(mask & lt)] = id[i];
-                if (CAPTURE && hit[i]) { const int64_t at = total + __popc(mask & lt); if (at < PC_RCAP_HITS) H[at] = (uint32_t)id[i]; }
+                pc_range_hit(S, hit[i], [&] { return total + __popc(mask & lt); }, at0 + i, (uint32_t)id[i]);
                 total += __popc(mask);
             }
         }
@@ -247,8 +236,8 @@ pc_range_coop_kernel(pc_tree T, const float *__restrict__ q, int64_t m, int qstr
 #pragma unroll
             for (int i = 0; i < 2 * PC_LEAF; i++) {
                 const uint32_t mask = __ballot_sync(PC_FULL_MASK, hit[i]);
-                if (FILL && hit[i]) out_idx[begin + total + __popc(mask & lt)] = id[i];
-                if (CAPTURE && hit[i]) { const int64_t at = total + __popc(mask & lt); if (at < PC_RCAP_HITS) H[at] = (uint32_t)id[i]; }
+                const uint32_t pos = ((i < PC_LEAF ? r0 : r1) & ~PC_REF_LEAF) + (i % PC_LEAF);
+                pc_range_hit(S, hit[i], [&] { return total + __popc(mask & lt); }, pos, (uint32_t)id[i]);
                 total += __popc(mask);
             }
         }
@@ -259,6 +248,67 @@ pc_range_coop_kernel(pc_tree T, const float *__restrict__ q, int64_t m, int qstr
         size += n0 + __popc(m1);
         __syncwarp();
     }
+    return total;
+}
+
+struct pc_range_stage {                // PC_RANGE_CAPTURE: where the counting pass parks the short lists
+    int32_t *stage;                    // stage_cap entries
+    unsigned long long stage_cap;
+    unsigned long long *cursor;        // next free entry
+    int64_t *pos;                      // per query: start of its parked list, -1 = not parked (walk it again)
+};
+
+// where pc_range_coop_kernel<MODE> puts a hit's original index: nowhere (COUNT), into its CSR row (FILL), into the warp's
+// hit buffer while the list is short enough to be captured (CAPTURE)
+template <int MODE>
+struct pc_range_sink {
+    int32_t *out_idx;
+    int64_t begin;
+    uint32_t *H;
+};
+
+template <int MODE, class AT>
+__device__ __forceinline__ void pc_range_hit(pc_range_sink<MODE> &S, bool hit, AT at, uint32_t, uint32_t id)
+{
+    if (MODE == PC_RANGE_FILL && hit) S.out_idx[S.begin + at()] = (int32_t)id;
+    if (MODE == PC_RANGE_CAPTURE && hit) { const int64_t a = at(); if (a < PC_RCAP_HITS) S.H[a] = id; }
+}
+
+#define PC_RCAP_FRONT 768         // frontier entries of the capturing pass: 512 double as the sort's second buffer, 256 as its histogram
+template <int MODE>
+__global__ void __launch_bounds__(32 * PC_RCOOP_WARPS, MODE == PC_RANGE_CAPTURE ? PC_RCAP_MIN_CTAS : (MODE == PC_RANGE_COUNT ? 12 : 8))
+pc_range_coop_kernel(pc_tree T, const float *__restrict__ q, int64_t m, int qstride,
+                     const double *__restrict__ range, int range_is_scalar,
+                     int64_t *__restrict__ counts, const int64_t *__restrict__ offsets, int32_t *__restrict__ out_idx,
+                     unsigned long long *__restrict__ long_count, int64_t *__restrict__ long_list,
+                     pc_range_stage S, const int64_t *__restrict__ qlist, const unsigned long long *__restrict__ qlist_count)
+{
+    constexpr bool FILL = MODE == PC_RANGE_FILL;
+    constexpr bool CAPTURE = MODE == PC_RANGE_CAPTURE;
+    constexpr int FCAP = CAPTURE ? PC_RCAP_FRONT : PC_RCOOP_CAP;
+    __shared__ uint32_t s_front[PC_RCOOP_WARPS][FCAP];
+    __shared__ uint32_t s_hits[CAPTURE ? PC_RCOOP_WARPS : 1][CAPTURE ? PC_RCAP_HITS : 1];
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    int64_t k = (int64_t)blockIdx.x * PC_RCOOP_WARPS + w;
+    if (qlist) {                       // fill pass over the queries the capture left behind
+        if ((unsigned long long)k >= *qlist_count) return;
+        k = qlist[k];
+    }
+    if (k >= m) return;
+    uint32_t *H = s_hits[CAPTURE ? w : 0];
+    int64_t begin = 0, want = 0;
+    if (FILL) {
+        begin = offsets[k]; want = offsets[k + 1] - begin;
+        if (want == 0) return;
+    }
+    pc_range_q Q;
+    if (!pc_range_query(T, q, k, qstride, range, range_is_scalar, Q)) {
+        if (!FILL && lane == 0) counts[k] = 0;
+        return;
+    }
+    uint32_t *F = s_front[w];
+    pc_range_sink<MODE> sink = { out_idx, begin, H };
+    const int64_t total = pc_range_walk<FCAP>(T, Q, F, lane, sink);
     if (!FILL) {
         if (lane == 0) counts[k] = total;
         if (CAPTURE) {

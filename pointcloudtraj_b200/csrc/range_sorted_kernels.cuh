@@ -1,7 +1,7 @@
 // range_sorted_kernels.cuh -- pc_range_sorted_batch: the hit lists of range queries ordered by (fp64 d2, original index) and
 // cut to max_nn (pcl::search::KdTree::radiusSearch with k_sqr_distances and max_nn).
 //
-// The hit set is pc_range_batch's (range_kernels.cuh): the same walk, fp32 filter and inclusive fp64 test.  What differs is
+// The hit set is pc_range_batch's (range_kernels.cuh): the same walk (pc_range_walk), fp32 filter and inclusive fp64 test.  What differs is
 // what a hit is remembered by and how a list is sorted:
 //   - the walk records a hit by its POSITION in the tree's point array (4 bytes).  After the walk the warp reads the point
 //     again (L1 / L2), recomputes its fp64 d2 with pc_exact_d2 -- the value the hit test used -- and its original index;
@@ -67,7 +67,22 @@ __device__ __forceinline__ void pc_pair_bitonic(double *D, uint32_t *I, IT n, in
     }
 }
 
-// one warp per query: the walk of pc_range_coop_kernel (seed leaves, then the LIFO frontier), recording hit positions
+// where pc_range_sorted_kernel<MODE> puts a hit's tree position: into the scratch area of its long list (FILL), into the warp's
+// hit buffer while the list is short enough to be captured (CAPTURE)
+template <int MODE>
+struct pc_rs_sink {
+    uint32_t *out;
+    uint32_t *H;
+};
+
+template <int MODE, class AT>
+__device__ __forceinline__ void pc_range_hit(pc_rs_sink<MODE> &S, bool hit, AT at, uint32_t pos, uint32_t)
+{
+    if (MODE == PC_RS_FILL && hit) S.out[at()] = pos;
+    if (MODE == PC_RS_CAPTURE) { const int64_t a = at(); if (hit && a < PC_RS_CAP_HITS) S.H[a] = pos; }
+}
+
+// one warp per query: pc_range_walk, recording hit positions
 template <int MODE>
 __global__ void __launch_bounds__(32 * PC_RS_WARPS, MODE == PC_RS_CAPTURE ? PC_RS_MIN_CTAS : 8)
 pc_range_sorted_kernel(pc_tree T, const float *__restrict__ q, int64_t m, int qstride, const double *__restrict__ range,
@@ -87,112 +102,20 @@ pc_range_sorted_kernel(pc_tree T, const float *__restrict__ q, int64_t m, int qs
     if (k >= m) return;
     uint32_t *H = s_hits[CAPTURE ? w : 0];
     uint32_t *out = A.long_ref + base;
-    const float *qq = q + k * qstride;
-    const float qx = qq[0], qy = qq[1], qz = qq[2];
-    const double qxd = (double)qx, qyd = (double)qy, qzd = (double)qz;
-    const double r = range[range_is_scalar ? 0 : k];
-    const double r2 = __dmul_rn(r, r);
-    if (T.n_points == 0 || !(r2 == r2)) {          // empty index, NaN range
+    pc_range_q Q;
+    if (!pc_range_query(T, q, k, qstride, range, range_is_scalar, Q)) {
         if (CAPTURE && lane == 0) A.counts[k] = 0;
         return;
     }
-    const float thr = fminf(__fmul_ru(__double2float_ru(r2), PC_THR_SLACK), FLT_MAX);
     uint32_t *F = s_front[w];
-    const uint32_t lt = (1u << lane) - 1u;
-    int64_t total = 0;
-    int size = 0;
-    {
-        const int n_seed = (int)T.seeds[0], n_seed_leaf = (int)T.seeds[1];
-        bool hit[PC_LEAF];
-        uint32_t at0 = 0;
-#pragma unroll
-        for (int i = 0; i < PC_LEAF; i++) hit[i] = false;
-        if (lane < n_seed_leaf) {
-            const uint32_t ref = T.seeds[PC_SEED_LEAF + 2 * lane], cnt = T.seeds[PC_SEED_LEAF + 2 * lane + 1];
-            at0 = ref & ~PC_REF_LEAF;
-            const float4 *pts = T.points + at0;
-#pragma unroll
-            for (int i = 0; i < PC_LEAF; i++) {
-                if ((uint32_t)i < cnt) {
-                    const float4 p = __ldg(pts + i);
-                    const float dx = p.x - qx, dy = p.y - qy, dz = p.z - qz;
-                    if (fmaf(dz, dz, fmaf(dy, dy, dx * dx)) <= thr) hit[i] = pc_exact_d2(p.x, p.y, p.z, qxd, qyd, qzd) <= r2;
-                }
-            }
-        }
-        if (n_seed_leaf > 0) {
-#pragma unroll
-            for (int i = 0; i < PC_LEAF; i++) {
-                const uint32_t mask = __ballot_sync(PC_FULL_MASK, hit[i]);
-                const int64_t at = total + __popc(mask & lt);
-                if (FILL && hit[i]) out[at] = at0 + i;
-                if (CAPTURE && hit[i] && at < PC_RS_CAP_HITS) H[at] = at0 + i;
-                total += __popc(mask);
-            }
-        }
-        if (lane < n_seed) F[lane] = T.seeds[PC_SEED_INNER + lane];
-        size = n_seed;
-    }
-    __syncwarp();
-    while (size > 0) {
-        const int take = (size + 64 + PC_STACK <= PC_RS_FRONT) ? min(size, 32) : 1;
-        const bool active = lane < take;
-        uint32_t node = 0;
-        if (active) node = F[size - 1 - lane];
-        size -= take;
-        __syncwarp();
-        bool push0 = false, push1 = false, leaf0 = false, leaf1 = false;
-        uint32_t r0 = 0, r1 = 0, c0 = 0, c1 = 0;
-        if (active) {
-            const pc_rec rec = pc_load_rec(T.rec + 4ull * node);
-            const float2 dd = pc_rec_d2(rec, qx, qy, qz);
-            const bool in0 = dd.x <= thr, in1 = dd.y <= thr;
-            r0 = pc_rec_ref(rec, 0); r1 = pc_rec_ref(rec, 1);
-            c0 = pc_rec_cnt(rec, 0); c1 = pc_rec_cnt(rec, 1);
-            leaf0 = in0 && (r0 & PC_REF_LEAF); leaf1 = in1 && (r1 & PC_REF_LEAF);
-            push0 = in0 && !(r0 & PC_REF_LEAF); push1 = in1 && !(r1 & PC_REF_LEAF);
-        }
-        if (__ballot_sync(PC_FULL_MASK, leaf0 || leaf1)) {
-            bool hit[2 * PC_LEAF];
-#pragma unroll
-            for (int c = 0; c < 2; c++) {
-                const bool leaf = c ? leaf1 : leaf0;
-                const uint32_t cnt = leaf ? (c ? c1 : c0) : 0u;
-                const float4 *pts = T.points + ((c ? r1 : r0) & ~PC_REF_LEAF);
-#pragma unroll
-                for (int i = 0; i < PC_LEAF; i++) {
-                    hit[c * PC_LEAF + i] = false;
-                    if ((uint32_t)i < cnt) {
-                        const float4 p = __ldg(pts + i);
-                        const float dx = p.x - qx, dy = p.y - qy, dz = p.z - qz;
-                        const float d = fmaf(dz, dz, fmaf(dy, dy, dx * dx));
-                        if (d <= thr) hit[c * PC_LEAF + i] = pc_exact_d2(p.x, p.y, p.z, qxd, qyd, qzd) <= r2;
-                    }
-                }
-            }
-#pragma unroll
-            for (int i = 0; i < 2 * PC_LEAF; i++) {
-                const uint32_t mask = __ballot_sync(PC_FULL_MASK, hit[i]);
-                const int64_t at = total + __popc(mask & lt);
-                const uint32_t ref = ((i < PC_LEAF ? r0 : r1) & ~PC_REF_LEAF) + (i % PC_LEAF);
-                if (FILL && hit[i]) out[at] = ref;
-                if (CAPTURE && hit[i] && at < PC_RS_CAP_HITS) H[at] = ref;
-                total += __popc(mask);
-            }
-        }
-        const uint32_t m0 = __ballot_sync(PC_FULL_MASK, push0), m1 = __ballot_sync(PC_FULL_MASK, push1);
-        const int n0 = __popc(m0);
-        if (push0) F[size + __popc(m0 & lt)] = r0;
-        if (push1) F[size + n0 + __popc(m1 & lt)] = r1;
-        size += n0 + __popc(m1);
-        __syncwarp();
-    }
+    pc_rs_sink<MODE> sink = { out, H };
+    const int64_t total = pc_range_walk<PC_RS_FRONT>(T, Q, F, lane, sink);
     __syncwarp();
     if (FILL) {
         // positions -> (fp64 d2, original index), in place; the CTA sort (pc_range_sorted_long_kernel) takes it from here
         for (int64_t i = lane; i < total; i += 32) {
             const float4 p = __ldg(T.points + out[i]);
-            A.long_d2[base + i] = pc_exact_d2(p.x, p.y, p.z, qxd, qyd, qzd);
+            A.long_d2[base + i] = pc_exact_d2(p.x, p.y, p.z, Q.qxd, Q.qyd, Q.qzd);
             out[i] = __float_as_uint(p.w);
         }
         return;
@@ -205,7 +128,7 @@ pc_range_sorted_kernel(pc_tree T, const float *__restrict__ q, int64_t m, int qs
         double *D = reinterpret_cast<double *>(F);
         for (int i = lane; i < (int)total; i += 32) {
             const float4 p = __ldg(T.points + H[i]);
-            D[i] = pc_exact_d2(p.x, p.y, p.z, qxd, qyd, qzd);
+            D[i] = pc_exact_d2(p.x, p.y, p.z, Q.qxd, Q.qyd, Q.qzd);
             H[i] = __float_as_uint(p.w);
         }
         __syncwarp();
