@@ -23,6 +23,8 @@
  *                               Planner/src/sim_planning_demo.cpp:729-781, :715-727; corridor_finder.cpp:412-416
  *   pc_trajectory_sweep_batch   (no counterpart: the reference samples every dt) certified first contact of a sphere moved
  *                               along a piecewise Bezier trajectory
+ *   pc_trajectory_nearest_batch (no counterpart: the reference samples every dt) certified clearance of a piecewise Bezier
+ *                               trajectory: its distance to the nearest cloud point to within tol, with a witness
  *   pc_comm_* / pc_index_broadcast   (no counterpart: the reference is single-process) -- replicate the
  *                               built index to the other GPUs of the host with one ncclBroadcast.
  *
@@ -289,6 +291,29 @@ int  pc_trajectory_sweep_batch(pc_index *ix, const pc_traj *traj, int64_t n_traj
                                int64_t n_seg, const double *coef, int64_t n_coef, int space,
                                double horizon, double radius, double tol,
                                int32_t *out_seg, double *out_s, int32_t *out_idx);
+
+/* Certified clearance of each trajectory: the distance from its motion to the nearest cloud point, to within tol, with a
+ * witness.  Trajectory arrays, their validation, their spaces and the motion are those of pc_trajectory_sweep_batch.  Let D*
+ * be the infimum of |C_s(sigma) - p| over the positions of the motion and the cloud points p with finite coordinates.  The
+ * answer (out_seg[t], out_s[t], out_idx[t], out_dist[t]) = (s_c, sigma_c, i, d) satisfies
+ *   1. witness: sigma_c lies in the motion's part of segment s_c and |C_{s_c}(sigma_c) - p_i| <= d, so D* <= d;
+ *   2. certificate: D* >= d - tol -- nothing on the motion comes closer than d - tol to any cloud point;
+ *   3. bound: max_range < 0 is unbounded (a witness whenever the index has a finite point within 2^60 m of the motion and the
+ *      motion is not empty; farther points are never searched, bounded or not).  With
+ *      max_range >= 0 a row without a witness means D* >= max_range, a reported row has d <= max_range + tol, and with
+ *      max_range <= D* <= max_range + tol either answer may come.
+ * No witness (under the bound, an empty motion, an empty index, no finite cloud point): -1, +inf, -1, +inf.  A segment of the
+ * motion with a non-finite or unusable T, order or coefficient, or a control point T * c_j beyond 1e37 in magnitude: -1, NaN,
+ * -1, NaN ("not checked").  Deterministic: PC_HOST and PC_DEVICE, and repeated calls, give the same bits.  Rule 2 is
+ * guaranteed for tol >= 2^-37 ((n + 1) S + d) on every segment of the motion, S = max_j |T * c_j| (DESIGN.md §4.14); the
+ * subdivision depth is capped at 50 levels so that every call terminates -- below that tol rule 1 holds, rules 2 and 3 may
+ * not.  Outputs are nullable.  PC_EINVAL: max_range NaN; tol not finite or <= 0; horizon NaN; every argument
+ * pc_clearance_batch refuses (including its host-side validation); the ASYNC spaces; a pc_batch_shard handle. */
+int  pc_trajectory_nearest_batch(pc_index *ix, const pc_traj *traj, int64_t n_traj,
+                                 const int32_t *seg_order, const double *seg_T, const int64_t *seg_coef_off,
+                                 int64_t n_seg, const double *coef, int64_t n_coef, int space,
+                                 double horizon, double max_range, double tol,
+                                 int32_t *out_seg, double *out_s, int32_t *out_idx, double *out_dist);
 
 /* ---- the RRT* sample stream and one speculative expansion batch, generated on the device ----------- */
 /* genSample's state (corridor_finder.cpp:333-358, the branches taken while no path is known: inform_status == false).

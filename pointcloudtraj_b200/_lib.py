@@ -33,7 +33,7 @@ ABI_SYMBOLS = [
     "pc_launch_count", "pc_profile_enable", "pc_profile_last_batch", "pc_batch_shard", "pc_index_set_radius_arith",
     "pc_profile_last_order_detail", "pc_profile_last_deferred_packets", "pc_sample_batch", "pc_expand_batch",
     "pc_knn_batch", "pc_range_sorted_batch", "pc_knn_large_batch", "pc_segment_nearest_batch", "pc_sphere_sweep_batch",
-    "pc_trajectory_sweep_batch",
+    "pc_trajectory_sweep_batch", "pc_trajectory_nearest_batch",
 ]
 
 
@@ -133,6 +133,8 @@ def load():
                                      C.POINTER(PcRadiusParams), vp, vp, vp]
     L.pc_trajectory_sweep_batch.argtypes = [vp, vp, i64, vp, vp, vp, i64, vp, i64, i32, C.c_double, C.c_double, C.c_double,
                                             vp, vp, vp]
+    L.pc_trajectory_nearest_batch.argtypes = [vp, vp, i64, vp, vp, vp, i64, vp, i64, i32, C.c_double, C.c_double, C.c_double,
+                                              vp, vp, vp, vp]
     L.pc_sphere_gather.argtypes = [vp, C.POINTER(C.c_double), C.c_double, i32, vp, i64, C.POINTER(i64)]
     L.pc_host_alloc.argtypes = [i64]
     L.pc_host_alloc.restype = vp

@@ -24,6 +24,7 @@
 #include "sweep_kernels.cuh"
 #include "clearance_kernels.cuh"
 #include "traj_sweep_kernels.cuh"
+#include "traj_nearest_kernels.cuh"
 #include "sampler_kernels.cuh"
 
 #define PC_VERSION_STRING "pcindex 0.2 (sm_100a)"
@@ -1111,6 +1112,7 @@ extern "C" int pc_radius_batch(pc_index *ix, const float *q_xyz, int64_t m, int6
 #include "sweep_host.inl"
 #include "clearance_host.inl"
 #include "traj_sweep_host.inl"
+#include "traj_nearest_host.inl"
 #include "sampler_host.inl"
 #include "comm_host.inl"
 #include "kd_compat.inl"

@@ -380,6 +380,21 @@ class PointCloudIndex:
                                                       float(tol), vp(seg), vp(s), vp(idx)))
         return seg, s, idx
 
+    def trajectory_nearest(self, traj_first_seg, seg_order, seg_T, seg_coef_off, coef, tol, max_range=-1.0, t_now=None, horizon=2.0):
+        """Certified clearance of each trajectory in continuous time (pc_trajectory_nearest_batch; host arrays, the layout of
+        clearance()).  Returns (seg int32, s float64, idx int32, dist float64): a witness position (segment index into the
+        segment arrays and its local time) and cloud point at most dist apart, with nothing on the trajectory closer than
+        dist - tol to the cloud.  max_range >= 0 bounds the search: a row without a witness is at least max_range clear.
+        -1 / inf / -1 / inf without a witness, -1 / NaN / -1 / NaN where a segment of the motion is not finite."""
+        n_traj, traj, so, sT, sc, cf = self._traj_arrays(traj_first_seg, seg_order, seg_T, seg_coef_off, coef, t_now)
+        seg = np.empty(n_traj, np.int32); s = np.empty(n_traj, np.float64); idx = np.empty(n_traj, np.int32)
+        dist = np.empty(n_traj, np.float64)
+        vp = lambda a: C.c_void_p(a.ctypes.data)
+        self._check(self._L.pc_trajectory_nearest_batch(self._h, C.c_void_p(traj.ctypes.data), n_traj, vp(so), vp(sT), vp(sc),
+                                                        so.shape[0], vp(cf), cf.shape[0], L.PC_HOST, float(horizon), float(max_range),
+                                                        float(tol), vp(seg), vp(s), vp(idx), vp(dist)))
+        return seg, s, idx, dist
+
 
 def shard_range(m, rank, n_ranks):
     """Contiguous slice of m units owned by `rank` (pc_shard_range)."""
