@@ -25,6 +25,8 @@
  *                               along a piecewise Bezier trajectory
  *   pc_trajectory_nearest_batch (no counterpart: the reference samples every dt) certified clearance of a piecewise Bezier
  *                               trajectory: its distance to the nearest cloud point to within tol, with a witness
+ *   pc_distance_field           (no counterpart) the truncated distance field (ESDF) of the cloud on a voxel lattice, with
+ *                               the nearest point of every voxel centre
  *   pc_comm_* / pc_index_broadcast   (no counterpart: the reference is single-process) -- replicate the
  *                               built index to the other GPUs of the host with one ncclBroadcast.
  *
@@ -314,6 +316,33 @@ int  pc_trajectory_nearest_batch(pc_index *ix, const pc_traj *traj, int64_t n_tr
                                  int64_t n_seg, const double *coef, int64_t n_coef, int space,
                                  double horizon, double max_range, double tol,
                                  int32_t *out_seg, double *out_s, int32_t *out_idx, double *out_dist);
+
+/* A regular voxel lattice: nx x ny x nz cubic voxels of edge `voxel`, voxel (0, 0, 0) with its outer corner at origin. */
+typedef struct pc_lattice {
+    double  origin[3];   /* world position of the outer corner of voxel (0, 0, 0), finite */
+    double  voxel;       /* edge length, finite and > 0 */
+    int64_t dims[3];     /* nx, ny, nz >= 0 */
+} pc_lattice;
+
+/* The truncated (unsigned) Euclidean distance field of the cloud on a lattice: for every voxel, the nearest cloud point to its
+ * centre and the distance to it.
+ *   centre   voxel (i, j, k) = (i_0, i_1, i_2) has c_a = (float)(origin_a + ((double)i_a + 0.5) * voxel) on axis a, every fp64
+ *            operation rounded to nearest and never fused, then rounded once to float32.
+ *   layout   element v = i + nx * (j + ny * k) of out_dist[nx*ny*nz] and out_idx[nx*ny*nz]: x fastest, z slowest.
+ *   index    out_idx[v] is the row pc_knn_batch(k = 1, max_range) returns for the centre: the lowest original index among the
+ *            exact fp64 minimisers of d2 (the exactness contract above), -1 when no point counts.
+ *   distance out_dist[v] = sqrt(d2) of that point, correctly rounded in fp64, then rounded once to float32; +inf where idx is -1.
+ *   bound    max_range < 0 is unbounded; max_range >= 0 keeps only points with d2 <= max_range^2 in fp64 (pc_range_batch's
+ *            test); +inf is accepted.
+ * An empty index gives -1 / +inf everywhere.  An empty lattice (a dim 0) returns PC_OK and writes nothing.  Either output may
+ * be NULL.  Repeated calls, and PC_HOST and PC_DEVICE, give the same bits.  PC_DEVICE is one kernel launch on the handle's
+ * stream with no scratch memory; PC_HOST copies the field home in chunks of whole brick layers (PC_HOST_CHUNK_QUERIES voxels
+ * each, about).  For a position x in the voxel of centre c the nearest point is at least out_dist - |x - c| away (c is the
+ * float32 centre above, not the exact middle of the voxel).
+ * PC_EINVAL: a NULL lat; a non-finite origin; a voxel that is not finite or <= 0; a negative dim; more than 2^40 voxels; a
+ * non-empty lattice whose first or last centre on an axis is not finite in float32; a NaN max_range; the ASYNC spaces; a
+ * pc_batch_shard handle (n_ranks > 1). */
+int  pc_distance_field(pc_index *ix, const pc_lattice *lat, double max_range, int space, float *out_dist, int32_t *out_idx);
 
 /* ---- the RRT* sample stream and one speculative expansion batch, generated on the device ----------- */
 /* genSample's state (corridor_finder.cpp:333-358, the branches taken while no path is known: inform_status == false).

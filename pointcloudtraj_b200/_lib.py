@@ -33,7 +33,7 @@ ABI_SYMBOLS = [
     "pc_launch_count", "pc_profile_enable", "pc_profile_last_batch", "pc_batch_shard", "pc_index_set_radius_arith",
     "pc_profile_last_order_detail", "pc_profile_last_deferred_packets", "pc_sample_batch", "pc_expand_batch",
     "pc_knn_batch", "pc_range_sorted_batch", "pc_knn_large_batch", "pc_segment_nearest_batch", "pc_sphere_sweep_batch",
-    "pc_trajectory_sweep_batch", "pc_trajectory_nearest_batch",
+    "pc_trajectory_sweep_batch", "pc_trajectory_nearest_batch", "pc_distance_field",
 ]
 
 
@@ -81,6 +81,19 @@ PC_CANDIDATE_DTYPE = [("center", "<f8", (3,)), ("radius", "<f4"), ("nearest", "<
 
 class PcTraj(C.Structure):
     _fields_ = [("first_seg", C.c_int32), ("num_seg", C.c_int32), ("t_now", C.c_double)]
+
+
+class PcLattice(C.Structure):
+    """pc_lattice: nx x ny x nz voxels of edge `voxel`, the outer corner of voxel (0, 0, 0) at origin."""
+    _fields_ = [("origin", C.c_double * 3), ("voxel", C.c_double), ("dims", C.c_int64 * 3)]
+
+    @classmethod
+    def make(cls, origin, voxel, dims):
+        lat = cls()
+        for a in range(3):
+            lat.origin[a], lat.dims[a] = float(origin[a]), int(dims[a])
+        lat.voxel = float(voxel)
+        return lat
 
 
 class PcIndexView(C.Structure):
@@ -135,6 +148,7 @@ def load():
                                             vp, vp, vp]
     L.pc_trajectory_nearest_batch.argtypes = [vp, vp, i64, vp, vp, vp, i64, vp, i64, i32, C.c_double, C.c_double, C.c_double,
                                               vp, vp, vp, vp]
+    L.pc_distance_field.argtypes = [vp, C.POINTER(PcLattice), C.c_double, i32, vp, vp]
     L.pc_sphere_gather.argtypes = [vp, C.POINTER(C.c_double), C.c_double, i32, vp, i64, C.POINTER(i64)]
     L.pc_host_alloc.argtypes = [i64]
     L.pc_host_alloc.restype = vp

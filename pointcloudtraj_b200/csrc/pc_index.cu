@@ -25,6 +25,7 @@
 #include "clearance_kernels.cuh"
 #include "traj_sweep_kernels.cuh"
 #include "traj_nearest_kernels.cuh"
+#include "field_kernels.cuh"
 #include "sampler_kernels.cuh"
 
 #define PC_VERSION_STRING "pcindex 0.2 (sm_100a)"
@@ -1108,6 +1109,7 @@ extern "C" int pc_radius_batch(pc_index *ix, const float *q_xyz, int64_t m, int6
 #include "range_sorted_host.inl"
 #include "knn_host.inl"
 #include "knn_large_host.inl"
+#include "field_host.inl"
 #include "segment_host.inl"
 #include "sweep_host.inl"
 #include "clearance_host.inl"

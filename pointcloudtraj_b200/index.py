@@ -214,6 +214,29 @@ class PointCloudIndex:
         self._torch_fence(tm, after=True)
         return idx, t
 
+    def distance_field(self, origin, voxel, dims, max_range=None, on_device=False):
+        """The distance field of the cloud on a voxel lattice (pc_distance_field): dims = (nx, ny, nz) voxels of edge `voxel`,
+        the outer corner of voxel (0, 0, 0) at origin.  Returns (dist float32, idx int32), both shaped (nz, ny, nx): the
+        nearest cloud point to every voxel centre, as pc_knn_batch(k = 1, max_range) finds it, and its distance; -1 / inf
+        where no point is within max_range.  numpy arrays, or with on_device torch CUDA tensors (PC_DEVICE)."""
+        lat = L.PcLattice.make(origin, voxel, dims)
+        nx, ny, nz = (int(d) for d in dims)
+        n = max(nx, 0) * max(ny, 0) * max(nz, 0)
+        r = -1.0 if max_range is None else float(max_range)
+        if on_device:
+            import torch
+            dist = torch.empty(n, dtype=torch.float32, device=f"cuda:{self.device}")
+            idx = torch.empty(n, dtype=torch.int32, device=f"cuda:{self.device}")
+            pd, pi, space = C.c_void_p(dist.data_ptr()), C.c_void_p(idx.data_ptr()), L.PC_DEVICE
+        else:
+            dist, pd = self._out(n, np.float32, False)
+            idx, pi = self._out(n, np.int32, False)
+            space = L.PC_HOST
+        self._torch_fence(on_device)
+        self._check(self._L.pc_distance_field(self._h, C.byref(lat), r, space, pd, pi))
+        self._torch_fence(on_device, after=True)
+        return dist.reshape(nz, ny, nx), idx.reshape(nz, ny, nx)
+
     def radius(self, q, params: L.PcRadiusParams, flags=L.PC_RADIUS_BOUNDED, want_idx=False):
         """safeRegionRrtStar::radiusSearch for every row of q.  Returns radius float32 (and idx int32)."""
         p, m, stride, space, keep, tm = self._rows(q, "q")
