@@ -39,6 +39,7 @@
 #define PC_COOP_MAX_BATCH 24576         // unordered batches up to this size: a group of lanes per query (profiles/r2_small_batch_ab.txt)
 #define PC_COOP_MAX_BATCH_UNBOUNDED 8192
 #define PC_SHARD_EXACT_MIN (1 << 20)    // pc_batch_shard: batches at least this large read their share's size back (see pc_share_size)
+#define PC_STAGE_BYTES ((int64_t)1 << 18)   // each half of ix->h_stage: a small PC_HOST call's inputs go in, its results come back
 
 static thread_local char g_create_error[256] = "";
 
@@ -95,8 +96,9 @@ struct pc_index {
     void *scratch = nullptr; int64_t scratch_cap = 0;
     // pc_range_sorted_batch: the lists too long for the capturing warp, untruncated (fp64 d2, then original index)
     uint32_t *range_long = nullptr; int64_t range_long_cap = 0;
+    // pinned staging block of small PC_HOST calls (pc_stage_upload): 2 * PC_STAGE_BYTES, inputs in the first half, results in the second
+    char *h_stage = nullptr;
     // pc_expand_batch: running candidate totals per chunk (pinned) and the events the host waits on before copying a chunk back
-    char *h_stage = nullptr;           // pc_clearance_batch: pinned staging block of small PC_HOST calls
     unsigned long long *h_totals = nullptr;
     cudaEvent_t ev_chunk[2] = { nullptr, nullptr };
 
@@ -227,6 +229,26 @@ static int pc_grow_sort(pc_index *ix, pc_lane &L, int64_t want)
     PC_CUDA(ix, pc_pool_alloc(ix, (void **)&L.vals_a, (size_t)want * 4));
     PC_CUDA(ix, pc_pool_alloc(ix, (void **)&L.vals_b, (size_t)want * 4));
     L.sort_cap = want;
+    return PC_OK;
+}
+
+static inline int64_t pc_align_up(int64_t v, int64_t a) { return (v + a - 1) / a * a; }
+
+// a host array bound for the device (pc_stage_upload)
+struct pc_up { const void *src; int64_t bytes; };
+
+// Copy a[0 .. n) to consecutive 256-byte-aligned slots of the device block at dst, on the handle's stream: with `pinned` (the
+// slots fit PC_STAGE_BYTES) through the pinned block ix->h_stage in one copy, else one pageable copy per array.  A pageable copy
+// costs ~10 us, so the planner's small calls pay for one copy instead of several.
+static int pc_stage_upload(pc_index *ix, char *dst, const pc_up *a, int n, bool pinned)
+{
+    if (pinned && !ix->h_stage) PC_CUDA(ix, cudaHostAlloc((void **)&ix->h_stage, 2 * PC_STAGE_BYTES, cudaHostAllocDefault));
+    int64_t o = 0;
+    for (int i = 0; i < n; o += pc_align_up(a[i].bytes, 256), i++) {
+        if (!pinned) PC_CUDA(ix, cudaMemcpyAsync(dst + o, a[i].src, (size_t)a[i].bytes, cudaMemcpyHostToDevice, ix->stream));
+        else if (a[i].bytes > 0) memcpy(ix->h_stage + o, a[i].src, (size_t)a[i].bytes);
+    }
+    if (pinned) PC_CUDA(ix, cudaMemcpyAsync(dst, ix->h_stage, (size_t)o, cudaMemcpyHostToDevice, ix->stream));
     return PC_OK;
 }
 
@@ -600,7 +622,6 @@ static pc_tree pc_tree_of(const pc_index *ix)
     return T;
 }
 
-// Morton-order a device-resident batch on lane L: returns the permutation (device pointer) in *perm
 enum pc_qkind { PC_Q_NEAREST, PC_Q_RADIUS };
 
 struct pc_qargs {
@@ -609,8 +630,14 @@ struct pc_qargs {
     int flags;
 };
 
-// Morton-order a device-resident batch on lane L: *perm = permutation (device), L.counter[1] = number of leading
-// entries that still need a search (radius batches answer the sensing-range early-outs in this pass)
+static pc_qargs pc_nearest_qargs(int flags)
+{
+    pc_qargs A;
+    memset(&A, 0, sizeof A);
+    A.kind = PC_Q_NEAREST; A.flags = flags;
+    return A;
+}
+
 // pc_batch_shard: the number of queries of this rank's share (L.counter[1], written by the ordering kernels queued on L.os)
 static int pc_share_size(pc_index *ix, pc_lane &L, int64_t m, int64_t *out)
 {
@@ -621,11 +648,53 @@ static int pc_share_size(pc_index *ix, pc_lane &L, int64_t m, int64_t *out)
     return PC_OK;
 }
 
-// *m_launch: host-side bound of the number of entries to search (m, or the exact share in pc_batch_shard mode)
-static int pc_sort_queries(pc_index *ix, pc_lane &L, const pc_qargs &A, const float *d_q, int64_t m, int qstride,
-                           int32_t *d_idx, float *d_f, const uint32_t **perm, const float4 **ordered, int64_t *m_launch, bool may_sync)
+// Whether a row-per-query batch of m entries is put in curve order: always on a pc_batch_shard handle (the share is selected
+// by the ordering pass), as PC_QUERY_SORTED / PC_QUERY_UNSORTED say, and under PC_QUERY_AUTO from the caller's sort_min on.
+static bool pc_want_order(const pc_index *ix, int flags, int64_t m, int64_t sort_min)
 {
-    *perm = nullptr; *ordered = nullptr; *m_launch = m;
+    if (ix->n == 0 || ix->sort_bits == 0) return false;
+    if (ix->shard_n > 1) return true;
+    if (flags & PC_QUERY_SORTED) return true;
+    if (flags & PC_QUERY_UNSORTED) return false;
+    return m >= sort_min;
+}
+
+// the smallest nearest / radius batch that PC_QUERY_AUTO orders
+static int64_t pc_sort_min(const pc_index *ix, const pc_qargs &A)
+{
+    return A.kind == PC_Q_NEAREST || !A.R.bounded ? ix->sort_min_nearest : ix->sort_min_radius;
+}
+
+// The ordering step of every row-per-query batch (pc_run_batch, the kNN, kNN-large and segment runs) on lane L, queued on
+// L.os: when pc_want_order says so, the m entries are put in curve order over the points d_a (stride floats per row), or with
+// d_b over the midpoints of the segments [d_a, d_b].  L.counter is zeroed first (counter[0]: the packet walks' deferred
+// packets, counter[1]: the entries left to search, written by this pass).  Radius batches (A) answer their sensing-range
+// early-outs here, into d_idx / d_f.  A batch left in its own order gets perm = ordered = m_eff = nullptr, m_launch = m.
+struct pc_order {
+    const uint32_t *perm;
+    const float4 *ordered;
+    const unsigned long long *m_eff;    // entries to search (written by the ordering pass)
+    int64_t m_launch;                   // host-side bound of *m_eff: the launches are sized by it (the exact share in pc_batch_shard mode)
+};
+
+static int pc_order_batch(pc_index *ix, pc_lane &L, const pc_qargs &A, int64_t sort_min, const float *d_a, const float *d_b,
+                          int64_t m, int stride, int32_t *d_idx, float *d_f, bool may_sync, pc_order &O)
+{
+    O.perm = nullptr; O.ordered = nullptr; O.m_eff = nullptr; O.m_launch = m;
+    if (!pc_want_order(ix, A.flags, m, sort_min)) return PC_OK;
+    const float *d_q = d_a;
+    int qstride = stride;
+    if (d_b) {
+        int rcm = pc_grow(ix, &L.d_mid, &L.mid_cap, m);
+        if (rcm != PC_OK) return rcm;
+        const int64_t blocks = (m + 255) / 256;
+        pc_seg_mid_kernel<<<(int)(blocks < ix->sm_count * 8 ? blocks : ix->sm_count * 8), 256, 0, L.os>>>(d_a, d_b, m, stride, L.d_mid);
+        ix->launches++;
+        d_q = reinterpret_cast<const float *>(L.d_mid);
+        qstride = 4;
+    }
+    PC_CUDA(ix, cudaMemsetAsync(L.counter, 0, 2 * sizeof(unsigned long long), L.os));
+    O.m_eff = L.counter + 1;
     // pc_batch_shard: a rank searches about 1 / shard_n of the batch, but how many exactly is known on the device only, and
     // launches sized for the whole batch are mostly CTAs that find nothing to do (C5 on 8 GPUs: 683 k of 781 k search CTAs and
     // 7 of 8 sort tiles; more than a millisecond of an 8 ms call).  Large sharded batches therefore read the count back --
@@ -697,8 +766,8 @@ static int pc_sort_queries(pc_index *ix, pc_lane &L, const pc_qargs &A, const fl
             pc_bin_scatter_kernel<false><<<grid, 256, 0, L.os>>>(d_q, m, qstride, L.keys_a, L.bins, L.ordered);
         ix->launches += 5;
         PC_CHECK_LAUNCH(ix);
-        *ordered = L.ordered;
-        if (exact) return pc_share_size(ix, L, m, m_launch);
+        O.ordered = L.ordered;
+        if (exact) return pc_share_size(ix, L, m, &O.m_launch);
         return PC_OK;
     }
     const int drop = 30 - bits > 0 ? 30 - bits : 0;     // 24-bit sort = top 24 curve bits, 32-bit sort = all 30
@@ -739,8 +808,8 @@ static int pc_sort_queries(pc_index *ix, pc_lane &L, const pc_qargs &A, const fl
     if (exact) {
         int rcs = pc_share_size(ix, L, m, &n_sort);
         if (rcs != PC_OK) return rcs;
-        *m_launch = n_sort;
-        if (n_sort == 0) { *perm = L.vals_a; return PC_OK; }
+        O.m_launch = n_sort;
+        if (n_sort == 0) { O.perm = L.vals_a; return PC_OK; }
         if (fused_hist) {
             const int64_t tiles = (n_sort + (int64_t)RS_THREADS * items - 1) / ((int64_t)RS_THREADS * items);
             PC_CUDA(ix, cudaMemsetAsync(L.tile_hist + os_scratch_words(0, bits / 8), 0, (size_t)(os_scratch_words(tiles, bits / 8) - os_scratch_words(0, bits / 8)) * sizeof(uint32_t), L.os));
@@ -749,17 +818,8 @@ static int pc_sort_queries(pc_index *ix, pc_lane &L, const pc_qargs &A, const fl
     // only the L.counter[1] compacted entries (device-side count <= m; n_sort bounds it on the host) are sorted
     int which = pc_sort_pairs<uint32_t, items>(ix, L.keys_a, L.vals_a, L.keys_b, L.vals_b, n_sort, 0, bits, L.tile_hist, L.digit_total, L.os, L.counter + 1, fused_hist);
     PC_CHECK_LAUNCH(ix);
-    *perm = which ? L.vals_b : L.vals_a;
+    O.perm = which ? L.vals_b : L.vals_a;
     return PC_OK;
-}
-
-static bool pc_want_sort(const pc_index *ix, int flags, int64_t m, bool unbounded)
-{
-    if (ix->n == 0 || ix->sort_bits == 0) return false;
-    if (ix->shard_n > 1) return true;          // the share is selected by the ordering pass
-    if (flags & PC_QUERY_SORTED) return true;
-    if (flags & PC_QUERY_UNSORTED) return false;
-    return m >= (unbounded ? ix->sort_min_nearest : ix->sort_min_radius);
 }
 
 // small unordered batch: G lanes per query.  A whole warp per query has the lowest latency while the batch fits the GPU's
@@ -806,25 +866,21 @@ static int pc_run_batch(pc_index *ix, pc_lane &L, const pc_qargs &A, const float
     // Pipelined (ASYNC) batches run their ordering pass on the lane's high-priority stream: its short, memory-bound kernels
     // are scheduled ahead of the queued CTAs of OTHER lanes' search kernels (issue-bound) and overlap with them.  Everything
     // already queued on the lane (input copy, the lane's previous batch, which still reads the sort buffers) comes first.
+    const int64_t sort_min = pc_sort_min(ix, A);
+    const bool order = pc_want_order(ix, A.flags, m, sort_min);
     L.os = L.stream;
-    if (split_streams && pc_want_sort(ix, A.flags, m, A.kind == PC_Q_NEAREST || !A.R.bounded)) {
+    if (split_streams && order) {
         PC_CUDA(ix, cudaEventRecord(L.ev_deps, L.stream));
         PC_CUDA(ix, cudaStreamWaitEvent(L.order_stream, L.ev_deps, 0));
         L.os = L.order_stream;
     }
-    const uint32_t *perm = nullptr;
-    const float4 *ordered = nullptr;
-    const unsigned long long *m_eff = nullptr;
     const bool prof = ix->profile && &L == &ix->lane[0];
     if (prof) PC_CUDA(ix, cudaEventRecord(L.t0, L.stream));
-    // counter[1]: queries that need a search after the ordering pass
-    PC_CUDA(ix, cudaMemsetAsync(L.counter, 0, 2 * sizeof(unsigned long long), L.os));
-    int64_t m_launch = m;             // launches of the search are sized by this (the exact share in pc_batch_shard mode)
-    if (pc_want_sort(ix, A.flags, m, A.kind == PC_Q_NEAREST || !A.R.bounded)) {
-        int rc = pc_sort_queries(ix, L, A, d_q, m, qstride, d_idx, d_f, &perm, &ordered, &m_launch, may_sync);
-        if (rc != PC_OK) return rc;
-        m_eff = L.counter + 1;
-    }
+    // every batch starts with a zero L.counter (pc_profile_last_deferred_packets); the ordering step clears it when it orders
+    if (!order) PC_CUDA(ix, cudaMemsetAsync(L.counter, 0, 2 * sizeof(unsigned long long), L.os));
+    pc_order O;
+    int rc = pc_order_batch(ix, L, A, sort_min, d_q, nullptr, m, qstride, d_idx, d_f, may_sync, O);
+    if (rc != PC_OK) return rc;
     if (L.os != L.stream) {
         PC_CUDA(ix, cudaEventRecord(L.ev_ordered, L.os));
         PC_CUDA(ix, cudaStreamWaitEvent(L.stream, L.ev_ordered, 0));
@@ -834,8 +890,11 @@ static int pc_run_batch(pc_index *ix, pc_lane &L, const pc_qargs &A, const float
     // dense batches (>= 3 queries per cell of 1/256 of the cloud's extent): 64-query packets, two queries per lane
     // (profiles/r1_sweep5*: +10 % radius, +18 % nearest at 10 M queries; -3 % at 2 M, hence the threshold)
     const bool two_per_lane = ix->query_kernel == 4 || (ix->query_kernel_auto && L.per_cell >= 3.0);
+    const uint32_t *perm = O.perm;
+    const float4 *ordered = O.ordered;
+    const unsigned long long *m_eff = O.m_eff;
     const bool is_ordered = perm || ordered;
-    const int64_t ml = is_ordered ? m_launch : m;        // entries the search launch has to cover
+    const int64_t ml = O.m_launch;       // entries the search launch has to cover (the exact share in pc_batch_shard mode)
     // unbounded packet walks put their incoherent packets aside (pc_packet_split)
     pc_radius_dev RN = A.R;
     if ((A.kind == PC_Q_NEAREST || !A.R.bounded) && ix->packet_split > 0.f && L.per_cell > 0.0) {
@@ -879,6 +938,39 @@ static int pc_run_batch(pc_index *ix, pc_lane &L, const pc_qargs &A, const float
     }
     PC_CHECK_LAUNCH(ix);
     if (prof) { PC_CUDA(ix, cudaEventRecord(L.t2, L.stream)); ix->profiled = true; }
+    return PC_OK;
+}
+
+// One PC_HOST chunk on lane L: rows [off, off + c) of `width` outputs each.  The lane's output buffers grow to hold the chunk
+// (at least `rows` rows), run(L, off, c, d_idx, d_f) stages the chunk's inputs on the lane and runs them into d_idx / d_f, and
+// the rows go home on the lane's stream.
+template <class RUN>
+static int pc_host_chunk(pc_index *ix, pc_lane &L, int64_t off, int64_t c, int64_t rows, int64_t width, int32_t *out_idx, float *out_f,
+                         RUN &run)
+{
+    int rc;
+    if (out_idx && (rc = pc_grow(ix, &L.d_i32, &L.i32_cap, c * width, rows * width)) != PC_OK) return rc;
+    if (out_f && (rc = pc_grow(ix, &L.d_f32, &L.f32_cap, c * width, rows * width)) != PC_OK) return rc;
+    if ((rc = run(L, off, c, out_idx ? L.d_i32 : nullptr, out_f ? L.d_f32 : nullptr)) != PC_OK) return rc;
+    if (out_idx) PC_CUDA(ix, cudaMemcpyAsync(out_idx + off * width, L.d_i32, (size_t)c * width * sizeof(int32_t), cudaMemcpyDeviceToHost, L.stream));
+    if (out_f) PC_CUDA(ix, cudaMemcpyAsync(out_f + off * width, L.d_f32, (size_t)c * width * sizeof(float), cudaMemcpyDeviceToHost, L.stream));
+    return PC_OK;
+}
+
+// Blocking PC_HOST batches of the row-per-query calls: chunks of `chunk` rows over the pipeline lanes (pc_host_chunk), after
+// the last index build on the handle's stream.  A multi-chunk call sizes the lane buffers for full chunks at once; a small
+// call allocates only what it needs.
+template <class RUN>
+static int pc_host_chunks(pc_index *ix, int64_t m, int64_t chunk, int64_t width, int32_t *out_idx, float *out_f, RUN run)
+{
+    for (int l = 1; l < PC_PIPE_LANES; l++) PC_CUDA(ix, cudaStreamWaitEvent(ix->lane[l].stream, ix->ev_ready, 0));
+    const int64_t rows = m > chunk ? chunk : 0;
+    int li = 0;
+    for (int64_t off = 0; off < m; off += chunk, li = (li + 1) % PC_PIPE_LANES) {
+        int rc = pc_host_chunk(ix, ix->lane[li], off, m - off < chunk ? m - off : chunk, rows, width, out_idx, out_f, run);
+        if (rc != PC_OK) return rc;
+    }
+    for (int l = 0; l < PC_PIPE_LANES; l++) PC_CUDA(ix, cudaStreamSynchronize(ix->lane[l].stream));
     return PC_OK;
 }
 
@@ -981,68 +1073,43 @@ static int pc_query_dispatch(pc_index *ix, const pc_qargs &A, const float *q, in
     if (m == 0) return PC_OK;
     const int qs = (int)q_stride;
     if (space == PC_DEVICE) return pc_run_batch(ix, ix->lane[0], A, q, m, qs, out_idx, out_f, false, true);
-    if (space == PC_HOST && m <= ix->tiny_batch && !pc_want_sort(ix, A.flags, m, A.kind == PC_Q_NEAREST || !A.R.bounded)) return pc_tiny_host_batch(ix, A, q, m, qs, out_idx, out_f);
+    if (space == PC_HOST && m <= ix->tiny_batch && !pc_want_order(ix, A.flags, m, pc_sort_min(ix, A))) return pc_tiny_host_batch(ix, A, q, m, qs, out_idx, out_f);
+
+    // PC_HOST: the queries staged per chunk, and on a pc_batch_shard handle the caller's current outputs too (the entries of
+    // other ranks' queries must come back untouched); PC_HOST_ASYNC: the whole batch as one such chunk (below)
+    auto run = [&](pc_lane &L, int64_t off, int64_t c, int32_t *d_idx, float *d_f) {
+        // (a chunk of a multi-chunk call: room for a full chunk of 4-float rows at once, as pc_host_chunks gives the outputs)
+        int rc = pc_grow(ix, &L.d_q, &L.q_cap, c * qs, c < m ? ix->host_chunk * 4 : 0);
+        if (rc != PC_OK) return rc;
+        PC_CUDA(ix, cudaMemcpyAsync(L.d_q, q + off * qs, (size_t)c * qs * sizeof(float), cudaMemcpyHostToDevice, L.stream));
+        if (ix->shard_n > 1) {
+            if (d_idx) PC_CUDA(ix, cudaMemcpyAsync(d_idx, out_idx + off, (size_t)c * sizeof(int32_t), cudaMemcpyHostToDevice, L.stream));
+            if (d_f) PC_CUDA(ix, cudaMemcpyAsync(d_f, out_f + off, (size_t)c * sizeof(float), cudaMemcpyHostToDevice, L.stream));
+        }
+        return pc_run_batch(ix, L, A, L.d_q, c, qs, d_idx, d_f, space == PC_HOST_ASYNC);
+    };
+    if (space == PC_HOST) return pc_host_chunks(ix, m, ix->host_chunk, 1, out_idx, out_f, run);
 
     // order the side lanes after the last (possibly still running) index build / broadcast on the handle's stream
     for (int l = 1; l < PC_PIPE_LANES; l++) PC_CUDA(ix, cudaStreamWaitEvent(ix->lane[l].stream, ix->ev_ready, 0));
+    pc_lane &L = ix->lane[ix->next_lane];
+    ix->next_lane = (ix->next_lane + 1) % PC_PIPE_LANES;
+    int rc;
     if (space == PC_DEVICE_ASYNC) {
         // device-resident batch on the next lane: consecutive calls overlap one batch's ordering pass (memory-bound) with the
         // previous batch's search (issue-bound).  The lane starts after whatever the handle's stream holds now (the
         // caller's producers of q); results are valid after pc_index_sync.
-        pc_lane &L = ix->lane[ix->next_lane];
-        ix->next_lane = (ix->next_lane + 1) % PC_PIPE_LANES;
         if (&L != &ix->lane[0]) {
             PC_CUDA(ix, cudaEventRecord(ix->ev_in, ix->stream));
             PC_CUDA(ix, cudaStreamWaitEvent(L.stream, ix->ev_in, 0));
         }
-        int rc = pc_run_batch(ix, L, A, q, m, qs, out_idx, out_f, true);
-        if (rc != PC_OK) return rc;
-        PC_CUDA(ix, cudaEventRecord(L.done, L.stream));
-        return PC_OK;
+        rc = pc_run_batch(ix, L, A, q, m, qs, out_idx, out_f, true);
+    } else {
+        // PC_HOST_ASYNC: the whole batch on the next lane, no wait: consecutive calls overlap their H2D / kernels / D2H
+        rc = pc_host_chunk(ix, L, 0, m, 0, 1, out_idx, out_f, run);
     }
-    if (space == PC_HOST_ASYNC) {
-        // the whole batch on the next lane, no wait: consecutive calls overlap their H2D / kernels / D2H
-        pc_lane &L = ix->lane[ix->next_lane];
-        ix->next_lane = (ix->next_lane + 1) % PC_PIPE_LANES;
-        int rc;
-        if ((rc = pc_grow(ix, &L.d_q, &L.q_cap, m * qs)) != PC_OK) return rc;
-        if (out_idx && (rc = pc_grow(ix, &L.d_i32, &L.i32_cap, m)) != PC_OK) return rc;
-        if (out_f && (rc = pc_grow(ix, &L.d_f32, &L.f32_cap, m)) != PC_OK) return rc;
-        PC_CUDA(ix, cudaMemcpyAsync(L.d_q, q, (size_t)m * qs * sizeof(float), cudaMemcpyHostToDevice, L.stream));
-        if (ix->shard_n > 1) {
-            if (out_idx) PC_CUDA(ix, cudaMemcpyAsync(L.d_i32, out_idx, (size_t)m * sizeof(int32_t), cudaMemcpyHostToDevice, L.stream));
-            if (out_f) PC_CUDA(ix, cudaMemcpyAsync(L.d_f32, out_f, (size_t)m * sizeof(float), cudaMemcpyHostToDevice, L.stream));
-        }
-        rc = pc_run_batch(ix, L, A, L.d_q, m, qs, out_idx ? L.d_i32 : nullptr, out_f ? L.d_f32 : nullptr, true);
-        if (rc != PC_OK) return rc;
-        if (out_idx) PC_CUDA(ix, cudaMemcpyAsync(out_idx, L.d_i32, (size_t)m * sizeof(int32_t), cudaMemcpyDeviceToHost, L.stream));
-        if (out_f) PC_CUDA(ix, cudaMemcpyAsync(out_f, L.d_f32, (size_t)m * sizeof(float), cudaMemcpyDeviceToHost, L.stream));
-        PC_CUDA(ix, cudaEventRecord(L.done, L.stream));      // a later rebuild must wait for this batch
-        return PC_OK;
-    }
-    const int64_t chunk = ix->host_chunk;
-    int li = 0;
-    for (int64_t off = 0; off < m; off += chunk, li = (li + 1) % PC_PIPE_LANES) {
-        pc_lane &L = ix->lane[li];
-        const int64_t c = m - off < chunk ? m - off : chunk;
-        int rc;
-        // a multi-chunk call sizes the lane buffers for full chunks at once; a small call allocates only what it needs
-        const int64_t floor_q = m > chunk ? chunk : 0;
-        if ((rc = pc_grow(ix, &L.d_q, &L.q_cap, c * qs, floor_q * 4)) != PC_OK) return rc;
-        if (out_idx && (rc = pc_grow(ix, &L.d_i32, &L.i32_cap, c, floor_q)) != PC_OK) return rc;
-        if (out_f && (rc = pc_grow(ix, &L.d_f32, &L.f32_cap, c, floor_q)) != PC_OK) return rc;
-        PC_CUDA(ix, cudaMemcpyAsync(L.d_q, q + off * qs, (size_t)c * qs * sizeof(float), cudaMemcpyHostToDevice, L.stream));
-        if (ix->shard_n > 1) {
-            // entries of other ranks' queries must come back untouched: stage the caller's current output contents
-            if (out_idx) PC_CUDA(ix, cudaMemcpyAsync(L.d_i32, out_idx + off, (size_t)c * sizeof(int32_t), cudaMemcpyHostToDevice, L.stream));
-            if (out_f) PC_CUDA(ix, cudaMemcpyAsync(L.d_f32, out_f + off, (size_t)c * sizeof(float), cudaMemcpyHostToDevice, L.stream));
-        }
-        rc = pc_run_batch(ix, L, A, L.d_q, c, qs, out_idx ? L.d_i32 : nullptr, out_f ? L.d_f32 : nullptr);
-        if (rc != PC_OK) return rc;
-        if (out_idx) PC_CUDA(ix, cudaMemcpyAsync(out_idx + off, L.d_i32, (size_t)c * sizeof(int32_t), cudaMemcpyDeviceToHost, L.stream));
-        if (out_f) PC_CUDA(ix, cudaMemcpyAsync(out_f + off, L.d_f32, (size_t)c * sizeof(float), cudaMemcpyDeviceToHost, L.stream));
-    }
-    for (int l = 0; l < PC_PIPE_LANES; l++) PC_CUDA(ix, cudaStreamSynchronize(ix->lane[l].stream));
+    if (rc != PC_OK) return rc;
+    PC_CUDA(ix, cudaEventRecord(L.done, L.stream));      // a later rebuild must wait for this batch
     return PC_OK;
 }
 
@@ -1060,10 +1127,7 @@ extern "C" int pc_nearest_batch(pc_index *ix, const float *q_xyz, int64_t m, int
 {
     int rc = pc_check_query_args(ix, "pc_nearest_batch", q_xyz, m, q_stride, space);
     if (rc != PC_OK) return rc;
-    pc_qargs A;
-    memset(&A, 0, sizeof A);
-    A.kind = PC_Q_NEAREST; A.flags = flags;
-    return pc_query_dispatch(ix, A, q_xyz, m, q_stride, space, out_idx, out_d2);
+    return pc_query_dispatch(ix, pc_nearest_qargs(flags), q_xyz, m, q_stride, space, out_idx, out_d2);
 }
 
 static int pc_make_radius_dev(pc_index *ix, const pc_radius_params *p, int flags, pc_radius_dev *R)

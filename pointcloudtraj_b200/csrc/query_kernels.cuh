@@ -933,7 +933,7 @@ pc_hilbert_lut_kernel(uint16_t *__restrict__ lut4, uint16_t *__restrict__ lut5)
     if (i < PC_LUT5_WORDS) lut5[i] = (uint16_t)pc_hilbert_cells_n<5>(i & 31u, (i >> 5) & 31u, (i >> 10) & 31u);
 }
 
-// bounded radius batches only (pc_sort_queries): unbounded ones keep the radix sort
+// bounded radius batches only (pc_order_batch): unbounded ones keep the radix sort
 template <bool SHARDED>
 __global__ void __launch_bounds__(256)
 pc_bin_count_kernel(const float *__restrict__ q, int64_t m, int qstride, const uint32_t *__restrict__ bbox,

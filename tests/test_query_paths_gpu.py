@@ -88,9 +88,9 @@ def build(h, pts):
 
 
 def per_cell(pts, m):
-    """Restatement of the density estimate of pc_sort_queries (pc_index.cu:633-647): queries per cell of 1/256 of the cloud's
-    largest extent, with thin axes counted as one cell.  pc_run_batch (:814) takes 64-query packets from 3, and the ordering
-    pass the 32-bit order above 16."""
+    """Restatement of the density estimate of the ordering step (pc_order_batch in pc_index.cu): queries per cell of 1/256 of
+    the cloud's largest extent, with thin axes counted as one cell.  pc_run_batch takes 64-query packets from 3, and the
+    ordering pass the 32-bit order above 16."""
     ext = (pts.max(0) - pts.min(0)).astype(np.float32)
     cell = float(ext.max()) / 256.0
     vol = float(np.prod([max(float(e), cell) for e in ext]))

@@ -277,6 +277,40 @@ def test_planner_single_trajectory_call(forest):
     check_rules(tr, 0.3, cloud, 0.4, 1e-3, 2.0, seg, s, idx)
 
 
+def _prefix(tr, n):
+    """The first n trajectories and only their segments and coefficients."""
+    s = int(tr["traj_first_seg"][n])
+    off = tr["seg_coef_off"][: s + 1]
+    return dict(traj_first_seg=tr["traj_first_seg"][: n + 1], seg_order=tr["seg_order"][:s], seg_T=tr["seg_T"][:s],
+                seg_coef_off=off, coef=tr["coef"][: off[-1]])
+
+
+def staged_bytes(tr, n):
+    """What a PC_HOST call on _prefix(tr, n) uploads, each array padded to 256 B: up to 256 KB it travels through one pinned
+    staging block, beyond that array by array (pc_traj_upload)."""
+    s = int(tr["traj_first_seg"][n])
+    pad = lambda b: -(-b // 256) * 256
+    return pad(16 * n) + pad(4 * s) + 2 * pad(8 * s) + pad(8 * int(tr["seg_coef_off"][s]))
+
+
+def test_host_staging_threshold(forest):
+    """The last batch that goes through the pinned staging block and the first that does not: PC_HOST returns bit for bit
+    what PC_DEVICE returns."""
+    pts, half, ix, cloud = forest
+    tr = synth.bezier_trajectories(400, half * 0.9, seed=15, order_range=(1, 12))
+    size = [staged_bytes(tr, k) for k in range(401)]
+    n = max(k for k in range(401) if size[k] <= 1 << 18)
+    assert n < 400 and size[n + 1] > 1 << 18
+    t_now = _mixed_t_now(400, np.random.default_rng(6))
+    for m in (n, n + 1):
+        p = _prefix(tr, m)
+        host = sweep(ix, p, t_now[:m], 0.3, 1e-3, 2.0)
+        dev = sweep(ix, p, t_now[:m], 0.3, 1e-3, 2.0, L.PC_DEVICE)
+        for a, b in zip(host, dev):
+            assert a.tobytes() == b.tobytes(), f"{m} trajectories"
+        assert (host[0] >= 0).any()
+
+
 def test_refusals(forest):
     pts, half, ix, cloud = forest
     tr = synth.bezier_trajectories(3, 8.0, seed=1)
