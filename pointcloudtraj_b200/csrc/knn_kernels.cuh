@@ -12,8 +12,9 @@
 //
 //   pc_knn_coop_kernel    one WARP per query: the frontier walk of pc_query_coop_kernel, the k-list spread over the warp
 //                         (lane j holds the j-th entry); also answers the queries of the packets the packet kernel puts aside
-//   pc_knn_packet_kernel  one warp walks the tree once for the 32 neighbouring queries of a curve-ordered batch (the walk of
-//                         pc_packet_traverse); every lane keeps its query's k-list in shared memory
+//   pc_knn_packet_kernel  one warp walks the tree once for the 32 neighbouring queries of a curve-ordered batch:
+//                         pc_packet_traverse<1> (query_kernels.cuh) over pc_knn_lane states, whose leaf hook scans a leaf
+//                         per lane; every lane keeps its query's k-list in shared memory
 // The warp walk (pc_warp_walk) is a template over the geometry and the list, shared with pc_knn_large_kernel
 // (knn_large_kernels.cuh), pc_segment_kernel and pc_sphere_sweep_kernel.
 #pragma once
@@ -38,13 +39,8 @@ __device__ __forceinline__ bool pc_knn_less(double e, uint32_t id, double d, uin
     return e < d || (e == d && id < di);
 }
 
-// query t of a batch: slot t, perm[t] (radix-sorted order) or the gathered float4 of the cell-binned order
-__device__ __forceinline__ void pc_knn_fetch(const float *__restrict__ q, int qstride, const uint32_t *__restrict__ perm,
-                                             const float4 *__restrict__ ordered, long long t, uint32_t &slot, float &qx, float &qy, float &qz)
-{
-    if (ordered) { const float4 v = ordered[t]; qx = v.x; qy = v.y; qz = v.z; slot = __float_as_uint(v.w); }
-    else { slot = perm ? perm[t] : (uint32_t)t; const float *qq = q + (size_t)slot * qstride; qx = qq[0]; qy = qq[1]; qz = qq[2]; }
-}
+// the k = 1 list of the walks that keep one nearest entry (segment, sweep and trajectory walks): no packets to defer
+__device__ __forceinline__ pc_knn_dev pc_knn_dev_k1(double r2, float bound_thr) { return pc_knn_dev{ 1, r2, bound_thr, 0.f, nullptr, nullptr }; }
 
 // ---- one warp per query ------------------------------------------------------------------------------------------------
 // The warp's k-list: lane j < k holds entry j (ld, li); every lane holds a copy of the k-th entry (kd, ki) and of thr.
@@ -53,6 +49,8 @@ struct pc_knn_wlist {
     uint32_t li, ki;
     float thr;
 };
+
+__device__ __forceinline__ pc_knn_wlist pc_knn_wlist_empty(float thr) { return pc_knn_wlist{ INFINITY, INFINITY, PC_KNN_NONE, PC_KNN_NONE, thr }; }
 
 // Offer every lane's candidate (have: passed the fp32 filter, the fp64 re-check and the bound) to the list, one lane at a
 // time: rank = number of entries before it (ballot), entries from there on move up one lane.  Called by the whole warp.
@@ -200,13 +198,12 @@ pc_knn_coop_kernel(pc_tree T, pc_knn_dev K, const float *__restrict__ q, int64_t
     const unsigned long long n_items = K.defer_count ? *K.defer_count * 32ull : (unsigned long long)m;
     const unsigned long long n_warps = (unsigned long long)gridDim.x * PC_KNN_WARPS;
     for (unsigned long long it = (unsigned long long)blockIdx.x * PC_KNN_WARPS + w; it < n_items; it += n_warps) {
-        const long long t = K.defer_count ? (long long)K.defer_list[it >> 5] * 32 + (long long)(it & 31u) : (long long)it;
+        const long long t = K.defer_count ? pc_deferred_query(K.defer_list, it, 32) : (long long)it;
         if (t >= m_search) continue;
         uint32_t slot;
         pc_point_geo G;
-        pc_knn_fetch(q, qstride, perm, ordered, t, slot, G.qx, G.qy, G.qz);
-        pc_knn_wlist W;
-        W.ld = W.kd = INFINITY; W.li = W.ki = PC_KNN_NONE; W.thr = K.bound_thr;
+        pc_query_fetch(q, qstride, perm, ordered, t, slot, G.qx, G.qy, G.qz);
+        pc_knn_wlist W = pc_knn_wlist_empty(K.bound_thr);
         if (T.n_points > 0) pc_warp_walk(T, K, s_front[w], lane, G, W);
         if (lane < K.k) {
             const size_t o = (size_t)slot * K.k + lane;
@@ -220,30 +217,49 @@ pc_knn_coop_kernel(pc_tree T, pc_knn_dev K, const float *__restrict__ q, int64_t
 // ---- warp packets of 32 curve-ordered queries ------------------------------------------------------------------------------
 // Lane-private k-lists in dynamic shared memory, [entry][lane] so that the lanes of a warp never share a bank: per warp
 // k x 32 doubles, then (after all warps' doubles) k x 32 indices -- 12 k bytes per query, 48 KB per CTA at k = 32.
-__device__ __forceinline__ void pc_knn_lane_scan(const float4 *__restrict__ pts, uint32_t cnt, float qx, float qy, float qz,
-                                                 const pc_knn_dev &K, double *__restrict__ Ld, uint32_t *__restrict__ Li,
-                                                 double &kd, uint32_t &ki, float &thr)
+// The lane state of the packet walk: the list's column (entry j at Ld[32 j], Li[32 j]); the k-th entry and thr in registers.
+struct pc_knn_lane {
+    const pc_knn_dev &K;
+    double *Ld;
+    uint32_t *Li;
+    double kd;
+    uint32_t ki;
+    float thr;                          // < 0: this lane takes part in the votes only
+};
+
+__device__ __forceinline__ void pc_knn_lane_scan(const float4 *__restrict__ pts, uint32_t cnt, const float (&q)[3], pc_knn_lane &L)
 {
+    const float qx = q[0], qy = q[1], qz = q[2];
+    const pc_knn_dev &K = L.K;
 #pragma unroll
     for (int i = 0; i < PC_LEAF; i++) {
         if ((uint32_t)i >= cnt) break;
         const float4 p = __ldg(pts + i);
         const float dx = p.x - qx, dy = p.y - qy, dz = p.z - qz;
-        if (!(fmaf(dz, dz, fmaf(dy, dy, dx * dx)) <= thr)) continue;
+        if (!(fmaf(dz, dz, fmaf(dy, dy, dx * dx)) <= L.thr)) continue;
         const double e = pc_exact_d2(p.x, p.y, p.z, (double)qx, (double)qy, (double)qz);
         const uint32_t id = (uint32_t)__float_as_int(p.w);
-        if (!(e <= K.r2) || !pc_knn_less(e, id, kd, ki)) continue;
+        if (!(e <= K.r2) || !pc_knn_less(e, id, L.kd, L.ki)) continue;
         int j = K.k - 1;
         for (; j > 0; j--) {                             // insertion into the sorted column
-            const double dj = Ld[(j - 1) * 32];
-            const uint32_t ij = Li[(j - 1) * 32];
+            const double dj = L.Ld[(j - 1) * 32];
+            const uint32_t ij = L.Li[(j - 1) * 32];
             if (!pc_knn_less(e, id, dj, ij)) break;
-            Ld[j * 32] = dj; Li[j * 32] = ij;
+            L.Ld[j * 32] = dj; L.Li[j * 32] = ij;
         }
-        Ld[j * 32] = e; Li[j * 32] = id;
-        kd = Ld[(K.k - 1) * 32]; ki = Li[(K.k - 1) * 32];
-        thr = fminf(K.bound_thr, pc_thr_from(kd));
+        L.Ld[j * 32] = e; L.Li[j * 32] = id;
+        L.kd = L.Ld[(K.k - 1) * 32]; L.ki = L.Li[(K.k - 1) * 32];
+        L.thr = fminf(K.bound_thr, pc_thr_from(L.kd));
     }
+}
+
+// Leaf hook of pc_packet_traverse for pc_knn_lane: a lane scans the leaf over its own count when its query wants the leaf's box
+// (the root leaf: always); no vote, the lanes' lists are private.
+template <int WHICH>
+__device__ __forceinline__ void pc_packet_leaf(const pc_tree &T, uint32_t ref, uint32_t cnt, const float (&q)[1][3],
+                                               const float (&d)[1], pc_knn_lane (&L)[1])
+{
+    if (WHICH == PC_LEAF_ROOT || d[0] <= L[0].thr) pc_knn_lane_scan(T.points + (ref & ~PC_REF_LEAF), cnt, q[0], L[0]);
 }
 
 __global__ void __launch_bounds__(32 * PC_KNN_WARPS)
@@ -262,67 +278,12 @@ pc_knn_packet_kernel(pc_tree T, pc_knn_dev K, const float *__restrict__ q, int64
     for (int j = 0; j < K.k; j++) { Ld[j * 32] = INFINITY; Li[j * 32] = PC_KNN_NONE; }
     const bool valid = t < m_search;
     uint32_t slot = 0;
-    float qx = 0.f, qy = 0.f, qz = 0.f;
-    if (valid) pc_knn_fetch(q, qstride, perm, ordered, t, slot, qx, qy, qz);
-    double kd = INFINITY;
-    uint32_t ki = PC_KNN_NONE;
-    float thr = (valid && T.n_points > 0) ? K.bound_thr : -1.0f;     // thr < 0: this lane takes part in the votes only
-    if (K.packet_split > 0.f) {
-        // the incoherent-packet test of pc_query_packet_kernel: a packet with a query farther than packet_split (Chebyshev)
-        // from its first one is answered by pc_knn_coop_kernel, one warp per query
-        const float ax = __shfl_sync(PC_FULL_MASK, qx, 0), ay = __shfl_sync(PC_FULL_MASK, qy, 0), az = __shfl_sync(PC_FULL_MASK, qz, 0);
-        const bool far = thr >= 0.f && fmaxf(fmaxf(fabsf(qx - ax), fabsf(qy - ay)), fabsf(qz - az)) > K.packet_split;
-        if (__any_sync(PC_FULL_MASK, far)) {
-            if (lane == 0) K.defer_list[atomicAdd(K.defer_count, 1ull)] = (uint32_t)warp_id;
-            return;
-        }
-    }
-    // the walk of pc_packet_traverse<1>: ballot on wanted children, majority vote for the nearer one, one stack per warp in
-    // local memory at a warp-uniform index; leaves are scanned over their own counts
-    if (__ballot_sync(PC_FULL_MASK, thr >= 0.f)) {
-        if (T.root & PC_REF_LEAF) {
-            pc_knn_lane_scan(T.points + (T.root & ~PC_REF_LEAF), T.root_count, qx, qy, qz, K, Ld, Li, kd, ki, thr);
-        } else {
-            uint32_t stack[PC_STACK];
-            int sp = 0;
-            uint32_t ref = T.root;
-            for (;;) {
-                const pc_rec rec = pc_load_rec(T.rec + 4ull * ref);
-                const float2 dd = pc_rec_d2(rec, qx, qy, qz);
-                const float d0 = dd.x, d1 = dd.y;
-                const uint32_t w0 = __ballot_sync(PC_FULL_MASK, d0 <= thr), w1 = __ballot_sync(PC_FULL_MASK, d1 <= thr);
-                uint32_t next = PC_NO_NODE;
-                if (w0 | w1) {
-                    const bool both = w0 != 0 && w1 != 0;
-                    bool first0 = w1 == 0;
-                    if (both) {
-                        const uint32_t ia = __ballot_sync(PC_FULL_MASK, d0 <= thr || d1 <= thr);
-                        const uint32_t pa = __ballot_sync(PC_FULL_MASK, d0 <= d1) & ia;
-                        first0 = 2 * __popc(pa) >= __popc(ia);
-                    }
-                    const uint32_t r0 = pc_rec_ref(rec, 0), r1 = pc_rec_ref(rec, 1);
-                    const uint32_t rn = first0 ? r0 : r1, rf = first0 ? r1 : r0;
-                    const uint32_t cn = pc_rec_cnt(rec, first0 ? 0 : 1), cf = pc_rec_cnt(rec, first0 ? 1 : 0);
-                    if (rn & PC_REF_LEAF) {
-                        if ((first0 ? d0 : d1) <= thr) pc_knn_lane_scan(T.points + (rn & ~PC_REF_LEAF), cn, qx, qy, qz, K, Ld, Li, kd, ki, thr);
-                    } else next = rn;
-                    if (both) {
-                        if (rf & PC_REF_LEAF) {
-                            if ((first0 ? d1 : d0) <= thr) pc_knn_lane_scan(T.points + (rf & ~PC_REF_LEAF), cf, qx, qy, qz, K, Ld, Li, kd, ki, thr);
-                        } else if (next != PC_NO_NODE) {
-                            stack[sp] = rf;
-                            sp++;
-                        } else next = rf;
-                    }
-                }
-                __syncwarp();
-                if (next != PC_NO_NODE) { ref = next; continue; }
-                if (sp == 0) break;
-                sp--;
-                ref = stack[sp];
-            }
-        }
-    }
+    float qv[1][3] = { { 0.f, 0.f, 0.f } };
+    if (valid) pc_query_fetch(q, qstride, perm, ordered, t, slot, qv[0][0], qv[0][1], qv[0][2]);
+    pc_knn_lane L[1] = { { K, Ld, Li, INFINITY, PC_KNN_NONE, (valid && T.n_points > 0) ? K.bound_thr : -1.0f } };
+    // incoherent packets go to pc_knn_coop_kernel, one warp per query
+    if (K.packet_split > 0.f && pc_packet_defer(qv, L, K.packet_split, K.defer_count, K.defer_list, warp_id, lane)) return;
+    pc_packet_traverse(T, qv, L, lane);
     if (valid) {
         const size_t o = (size_t)slot * K.k;
         for (int j = 0; j < K.k; j++) {

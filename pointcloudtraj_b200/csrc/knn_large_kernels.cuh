@@ -131,7 +131,7 @@ pc_knn_large_kernel(pc_tree T, pc_knn_dev K, const float *__restrict__ q, int64_
     for (long long t = (long long)blockIdx.x * PC_KNN_LARGE_WARPS + w; t < m_search; t += n_warps) {
         uint32_t slot;
         pc_point_geo G;
-        pc_knn_fetch(q, qstride, perm, ordered, t, slot, G.qx, G.qy, G.qz);
+        pc_query_fetch(q, qstride, perm, ordered, t, slot, G.qx, G.qy, G.qz);
         W.n = W.qn = 0;
         W.kd = INFINITY; W.ki = PC_KNN_NONE; W.thr = K.bound_thr;
         if (T.n_points > 0) pc_warp_walk(T, K, F, lane, G, W);

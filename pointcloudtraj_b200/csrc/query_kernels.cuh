@@ -10,7 +10,8 @@
 //
 // Three walks, all returning identical results:
 //   pc_nearest_traverse     one thread per query, near-first descent with a per-thread stack (unordered large batches)
-//   pc_packet_traverse<NQ>  one WARP walks the tree once for 32 * NQ neighbouring queries of a curve-ordered batch
+//   pc_packet_traverse<NQ>  one WARP walks the tree once for 32 * NQ neighbouring queries of a curve-ordered batch (also
+//                           the walk of the kNN packets, knn_kernels.cuh, which share pc_packet_defer and pc_query_fetch too)
 //   pc_query_coop_kernel    a GROUP of 8 / 16 / 32 lanes per query (small batches, the planner's one-query calls)
 #pragma once
 #include "common.cuh"
@@ -322,21 +323,41 @@ pc_query_simple_kernel(pc_tree T, pc_radius_dev R, const float *__restrict__ q, 
 // Measured and dropped in round 1 (profiles/r1_sweep3/4/6/8*): rejecting stale stack entries with per-entry minimum
 // distances, a 32-wide sideways test of descendants against the packet's box, a 4-ary walk, letting both queries of a lane
 // vote, packed __reduce_add_sync votes, most-wanted-child-first ordering, far-child prefetch on push.
+// The walk is a template over the lane state S (pc_best here, pc_knn_lane in knn_kernels.cuh): it reads a query slot's
+// filter as b[j].thr and hands every leaf it meets to the overload of pc_packet_leaf for S.
 // Must be called by all 32 lanes of a warp, converged; lanes without a query pass thr < 0 and take part in the votes only.
-template <int NQ>
-__device__ __forceinline__ void pc_packet_traverse(const pc_tree &T, const float (&q)[NQ][3], pc_best (&b)[NQ], int lane)
+#define PC_LEAF_ROOT 0                  // the tree is one leaf
+#define PC_LEAF_NEAR 1                  // the child of a record the warp enters first
+#define PC_LEAF_FAR 2                   // the other child, after the near one may have tightened the bounds
+// Leaf hook of pc_best lanes: ref = the leaf (PC_REF_LEAF | first point), cnt = its own count (unused: these scans read
+// PC_LEAF points from any start), d = this lane's squared distances to the leaf's box.  The near leaf is scanned for the
+// whole warp, the far one only if a query still wants it.
+template <int WHICH, int NQ>
+__device__ __forceinline__ void pc_packet_leaf(const pc_tree &T, uint32_t ref, uint32_t, const float (&q)[NQ][3],
+                                               const float (&d)[NQ], pc_best (&b)[NQ])
+{
+    if constexpr (WHICH == PC_LEAF_FAR) {
+        bool again = false;
+#pragma unroll
+        for (int j = 0; j < NQ; j++) again = again || d[j] <= b[j].thr;
+        if (!__ballot_sync(PC_FULL_MASK, again)) return;
+    }
+    const float4 *pts = T.points + (ref & ~PC_REF_LEAF);
+    // NQ == 2: the lane's two queries packed per axis, negated (pc_scan_leaf_x2); the root leaf takes the plain scan
+    if constexpr (NQ == 2 && WHICH != PC_LEAF_ROOT) pc_scan_leaf_x2(pts, make_float2(-q[0][0], -q[1][0]), make_float2(-q[0][1], -q[1][1]), make_float2(-q[0][2], -q[1][2]), b);
+    else pc_scan_leaf<NQ>(pts, q, b);
+}
+
+template <int NQ, class S>
+__device__ __forceinline__ void pc_packet_traverse(const pc_tree &T, const float (&q)[NQ][3], S (&b)[NQ], int lane)
 {
     bool any = false;
 #pragma unroll
     for (int j = 0; j < NQ; j++) any = any || b[j].thr >= 0.f;
     if (__ballot_sync(PC_FULL_MASK, any) == 0) return;
-    if (T.root & PC_REF_LEAF) { pc_scan_leaf<NQ>(T.points + (T.root & ~PC_REF_LEAF), q, b); return; }
-    // NQ == 2: the lane's two queries packed per axis, negated, for the leaf scans (pc_scan_leaf_x2)
+    if (T.root & PC_REF_LEAF) { const float d[NQ] = {}; pc_packet_leaf<PC_LEAF_ROOT>(T, T.root, T.root_count, q, d, b); return; }
+    // NQ == 2: the lane's two queries packed per axis, negated, for the box tests below
     const float2 nqx = make_float2(-q[0][0], -q[NQ - 1][0]), nqy = make_float2(-q[0][1], -q[NQ - 1][1]), nqz = make_float2(-q[0][2], -q[NQ - 1][2]);
-    auto scan = [&](const float4 *pts) {
-        if constexpr (NQ == 2) pc_scan_leaf_x2(pts, nqx, nqy, nqz, b);
-        else pc_scan_leaf<NQ>(pts, q, b);
-    };
     // The warp's stack of postponed children lives in LOCAL memory, the same copy in every lane at a warp-uniform index: one
     // coalesced 128-byte STL per push, one LDL per pop (L1-resident), no registers, no shuffles.  Measured against three
     // registers per lane read back with __shfl_sync (which ptxas spilled at 48 registers anyway): 0.81 -> 0.77 ms; against
@@ -378,15 +399,12 @@ __device__ __forceinline__ void pc_packet_traverse(const pc_tree &T, const float
             }
             const uint32_t r0 = pc_rec_ref(rec, 0), r1 = pc_rec_ref(rec, 1);
             const uint32_t rn = first0 ? r0 : r1, rf = first0 ? r1 : r0;
-            if (rn & PC_REF_LEAF) scan(T.points + (rn & ~PC_REF_LEAF));
+            const uint32_t cn = pc_rec_cnt(rec, first0 ? 0 : 1), cf = pc_rec_cnt(rec, first0 ? 1 : 0);
+            if (rn & PC_REF_LEAF) pc_packet_leaf<PC_LEAF_NEAR>(T, rn, cn, q, first0 ? d0 : d1, b);
             else next = rn;
             if (both) {
-                if (rf & PC_REF_LEAF) {
-                    bool again = false;          // the near leaf may have tightened the bounds
-#pragma unroll
-                    for (int j = 0; j < NQ; j++) again = again || (first0 ? d1[j] : d0[j]) <= b[j].thr;
-                    if (__ballot_sync(PC_FULL_MASK, again)) scan(T.points + (rf & ~PC_REF_LEAF));
-                } else if (next != PC_NO_NODE) {
+                if (rf & PC_REF_LEAF) pc_packet_leaf<PC_LEAF_FAR>(T, rf, cf, q, first0 ? d1 : d0, b);
+                else if (next != PC_NO_NODE) {
                     stack[sp] = rf;
                     sp++;
                 } else next = rf;
@@ -397,6 +415,47 @@ __device__ __forceinline__ void pc_packet_traverse(const pc_tree &T, const float
         sp--;
         ref = stack[sp];
     }
+}
+
+// An UNBOUNDED walk is shared well only by queries that lie close together: a lane far from the others keeps an infinite (then
+// very loose) bound until the walk -- steered by the majority -- happens to come near it, and until then it wants every node.
+// Packets are cut from the curve order at fixed positions, so a few straddle a jump of the curve (the 3-D Hilbert order of a
+// flat map leaves and re-enters the slab of the map) or, in pc_batch_shard mode, two cells of the rank's share that are not
+// neighbours; one such packet can walk a large part of the tree, alone, for milliseconds (C5 split over 8 ranks: half of the
+// ranks took 12 ms instead of 6).  A packet with a live query (thr >= 0) farther than `split` (Chebyshev; some packet extents
+// at the batch's density) from its first one is not walked: it goes on the list, for a kernel that walks its queries alone.
+template <int NQ, class S>
+__device__ __forceinline__ bool pc_packet_defer(const float (&q)[NQ][3], const S (&b)[NQ], float split,
+                                                unsigned long long *count, uint32_t *list, long long packet, int lane)
+{
+    const float ax = __shfl_sync(PC_FULL_MASK, q[0][0], 0), ay = __shfl_sync(PC_FULL_MASK, q[0][1], 0), az = __shfl_sync(PC_FULL_MASK, q[0][2], 0);
+    bool far = false;
+#pragma unroll
+    for (int j = 0; j < NQ; j++)
+        far = far || (b[j].thr >= 0.f && fmaxf(fmaxf(fabsf(q[j][0] - ax), fabsf(q[j][1] - ay)), fabsf(q[j][2] - az)) > split);
+    if (!__any_sync(PC_FULL_MASK, far)) return false;
+    if (lane == 0) list[atomicAdd(count, 1ull)] = (uint32_t)packet;
+    return true;
+}
+
+// batch position of deferred work item e: query e % per_packet of the packet list[e / per_packet]
+__device__ __forceinline__ long long pc_deferred_query(const uint32_t *list, unsigned long long e, int per_packet)
+{
+    return (long long)list[e / (unsigned)per_packet] * per_packet + (long long)(e % (unsigned)per_packet);
+}
+
+// query t of a batch: slot t, perm[t] (radix-sorted order) or the gathered float4 of the cell-binned order
+__device__ __forceinline__ void pc_query_fetch(const float *__restrict__ q, int qstride, const uint32_t *__restrict__ perm,
+                                               const float4 *__restrict__ ordered, long long t, uint32_t &slot, float &qx, float &qy, float &qz)
+{
+    if (ordered) { const float4 v = ordered[t]; qx = v.x; qy = v.y; qz = v.z; slot = __float_as_uint(v.w); }
+    else { slot = perm ? perm[t] : (uint32_t)t; const float *qq = q + (size_t)slot * qstride; qx = qq[0]; qy = qq[1]; qz = qq[2]; }
+}
+
+// the slot alone, for batches whose rows are read from their own arrays (segments)
+__device__ __forceinline__ uint32_t pc_query_fetch(const uint32_t *__restrict__ perm, const float4 *__restrict__ ordered, long long t)
+{
+    return ordered ? __float_as_uint(ordered[t].w) : perm ? perm[t] : (uint32_t)t;
 }
 
 template <int KIND, int NQ>
@@ -435,26 +494,10 @@ pc_query_packet_kernel(pc_tree T, pc_radius_dev R, const float *__restrict__ q, 
             else { pc_write_trivial<KIND>(R, k[j], out_idx, out_f); valid[j] = false; }
         }
     }
-    if ((KIND == PC_KIND_NEAREST || !R.bounded) && R.packet_split > 0.f) {
-        // An UNBOUNDED walk is shared well only by queries that lie close together: a lane far from the others keeps an
-        // infinite (then very loose) bound until the walk -- steered by the majority -- happens to come near it, and until then
-        // it wants every node.  Packets are cut from the curve order at fixed positions, so a few straddle a jump of the curve
-        // (the 3-D Hilbert order of a flat map leaves and re-enters the slab of the map) or, in pc_batch_shard mode, two cells of
-        // the rank's share that are not neighbours; one such packet can walk a large part of the tree, alone, for milliseconds
-        // (C5 split over 8 ranks: half of the ranks took 12 ms instead of 6).  A packet with a query farther than packet_split
-        // (Chebyshev; some packet extents at the batch's density) from its first one is not walked here: it is queued for
-        // pc_query_deferred_kernel, where every query walks alone.
-        const float ax = __shfl_sync(PC_FULL_MASK, qv[0][0], 0), ay = __shfl_sync(PC_FULL_MASK, qv[0][1], 0), az = __shfl_sync(PC_FULL_MASK, qv[0][2], 0);
-        bool far = false;
-#pragma unroll
-        for (int j = 0; j < NQ; j++)
-            far = far || (b[j].thr >= 0.f && fmaxf(fmaxf(fabsf(qv[j][0] - ax), fabsf(qv[j][1] - ay)), fabsf(qv[j][2] - az)) > R.packet_split);
-        if (__any_sync(PC_FULL_MASK, far)) {
-            if (lane == 0) R.defer_list[atomicAdd(R.defer_count, 1ull)] = (uint32_t)warp_id;
-            return;
-        }
-    }
-    pc_packet_traverse<NQ>(T, qv, b, lane);
+    // incoherent packets go to pc_query_deferred_kernel (bounded radius walks prune early and cannot run away)
+    if ((KIND == PC_KIND_NEAREST || !R.bounded) && R.packet_split > 0.f &&
+        pc_packet_defer(qv, b, R.packet_split, R.defer_count, R.defer_list, warp_id, lane)) return;
+    pc_packet_traverse(T, qv, b, lane);
 #pragma unroll
     for (int j = 0; j < NQ; j++)
         if (valid[j]) pc_write_result<KIND>(R, b[j], k[j], out_idx, out_f);
@@ -477,12 +520,11 @@ pc_query_deferred_kernel(pc_tree T, pc_radius_dev R, const float *__restrict__ q
     const unsigned long long total = *R.defer_count * (unsigned long long)per_packet;
     const unsigned long long n_threads = (unsigned long long)gridDim.x * blockDim.x;
     for (unsigned long long e = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += n_threads) {
-        const long long t = (long long)R.defer_list[e / (unsigned)per_packet] * per_packet + (long long)(e % (unsigned)per_packet);
+        const long long t = pc_deferred_query(R.defer_list, e, per_packet);
         if (t >= m_search) continue;
         uint32_t k;
         float qx, qy, qz;
-        if (ordered) { const float4 v = ordered[t]; qx = v.x; qy = v.y; qz = v.z; k = __float_as_uint(v.w); }
-        else { k = perm ? perm[t] : (uint32_t)t; const float *qq = q + (size_t)k * qstride; qx = qq[0]; qy = qq[1]; qz = qq[2]; }
+        pc_query_fetch(q, qstride, perm, ordered, t, k, qx, qy, qz);
         pc_best b; b.d2 = INFINITY; b.idx = -1; b.thr = FLT_MAX;
         pc_nearest_traverse(T, qx, qy, qz, b);
         pc_write_result<KIND>(R, b, k, out_idx, out_f);

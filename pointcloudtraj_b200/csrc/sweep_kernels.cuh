@@ -68,17 +68,15 @@ pc_sphere_sweep_kernel(pc_tree T, pc_seg_dev S, float r_up, const float *__restr
 {
     __shared__ uint2 s_front[PC_SEG_WARPS][PC_KNN_FRONT];       // (inner node, float bits of its entry parameter)
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    pc_knn_dev K;
-    K.k = 1; K.r2 = S.r2; K.bound_thr = S.bound_thr; K.packet_split = 0.f; K.defer_count = nullptr; K.defer_list = nullptr;
+    const pc_knn_dev K = pc_knn_dev_k1(S.r2, S.bound_thr);
     const long long m_search = m_eff ? (long long)*m_eff : (long long)m;
     const long long n_warps = (long long)gridDim.x * PC_SEG_WARPS;
     for (long long t = (long long)blockIdx.x * PC_SEG_WARPS + w; t < m_search; t += n_warps) {
-        const uint32_t slot = ordered ? __float_as_uint(ordered[t].w) : perm ? perm[t] : (uint32_t)t;
+        const uint32_t slot = pc_query_fetch(perm, ordered, t);
         const float *a = a_xyz + (size_t)slot * stride, *b = b_xyz + (size_t)slot * stride;
         const float av[3] = { a[0], a[1], a[2] }, bv[3] = { b[0], b[1], b[2] };
         const bool finite = isfinite(av[0]) && isfinite(av[1]) && isfinite(av[2]) && isfinite(bv[0]) && isfinite(bv[1]) && isfinite(bv[2]);
-        pc_knn_wlist W;
-        W.ld = W.kd = INFINITY; W.li = W.ki = PC_KNN_NONE; W.thr = S.bound_thr;
+        pc_knn_wlist W = pc_knn_wlist_empty(S.bound_thr);
         if (finite && T.n_points > 0) {
             pc_sweep_geo G;
             const float len = pc_seg_setup(av, bv, G);

@@ -36,11 +36,9 @@ __device__ __noinline__ double pc_tnr_point_bound(const pc_tree &T, uint2 *__res
     P.qx = (float)bx; P.qy = (float)by; P.qz = (float)bz;
     const double eb = pc_exact_d2(P.qx, P.qy, P.qz, bx, by, bz);                 // |B - float(B)|^2
     const double Ur = fmin(U, PC_TNR_MAX_R);
-    pc_knn_dev K;
-    K.k = 1; K.r2 = __dmul_ru(Ur, Ur); K.bound_thr = pc_thr_from(K.r2);
-    K.packet_split = 0.f; K.defer_count = nullptr; K.defer_list = nullptr;
-    pc_knn_wlist V;
-    V.ld = V.kd = INFINITY; V.li = V.ki = PC_KNN_NONE; V.thr = K.bound_thr;
+    const double r2 = __dmul_ru(Ur, Ur);
+    const pc_knn_dev K = pc_knn_dev_k1(r2, pc_thr_from(r2));
+    pc_knn_wlist V = pc_knn_wlist_empty(K.bound_thr);
     pc_warp_walk(T, K, F, lane, P, V);
     qi = V.ki;
     return __dadd_ru(__dmul_ru(__dadd_ru(__dsqrt_ru(V.kd), __dsqrt_ru(eb)), PC_TNR_REL_UP), mu);

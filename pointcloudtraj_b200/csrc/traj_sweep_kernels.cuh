@@ -186,10 +186,9 @@ __device__ __forceinline__ pc_traj_chord pc_traj_piece(const double (*M)[PC_MAX_
 __device__ __forceinline__ void pc_traj_chord_walk(const pc_tree &T, uint2 *__restrict__ F, int lane, const pc_traj_chord &C,
                                                    double R, pc_knn_wlist &W)
 {
-    pc_knn_dev K;
-    K.k = 1; K.r2 = __dmul_ru(R, R); K.bound_thr = pc_thr_from(K.r2);
-    K.packet_split = 0.f; K.defer_count = nullptr; K.defer_list = nullptr;
-    W.ld = W.kd = INFINITY; W.li = W.ki = PC_KNN_NONE; W.thr = K.bound_thr;
+    const double r2 = __dmul_ru(R, R);
+    const pc_knn_dev K = pc_knn_dev_k1(r2, pc_thr_from(r2));
+    W = pc_knn_wlist_empty(K.bound_thr);
     if (T.n_points > 0) {
         const double ax = C.ax, ay = C.ay, az = C.az, bx = C.bx, by = C.by, bz = C.bz;
         const float af[3] = { (float)ax, (float)ay, (float)az }, bf[3] = { (float)bx, (float)by, (float)bz };
